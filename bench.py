@@ -6,11 +6,13 @@ pairs/s of banded forward-backward + posterior on `configs[1]`: 100 000 syntheti
 StateMachine5, library-default band and posterior threshold 0.01.  One "step" = one pass of the whole hot path
 (band builder -> forward -> backward -> totals -> posterior scan/compaction) over the batch.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--impl reference] [--dump-outputs DIR]
 
-value : inputs resident in HBM, CUDA-event time on the launching stream, max over ranks.
+value : inputs resident in HBM, CUDA-event time on the launching stream over K steps, max over ranks.
 e2e   : the same pass through the C-ABI with HOST buffers (pinned): cpb_batch_create (H2D) + cpb_batch_run +
-        cpb_batch_fetch_pairs (D2H) inside the timed region.
+        cpb_batch_fetch_pairs (D2H) inside the timed region, K steps.
+--dump-outputs DIR : after the timed steps, what the last one computed goes to DIR/*.npy (dump_outputs), so that two builds
+        can be compared output for output on the same seeded inputs.
 --impl reference : the reference's own CPU implementation (oracle/_ref when it was built, else the plain-C port)
         on all host cores over a bounded sample of the same workload.
 """
@@ -109,6 +111,22 @@ def make_inputs(n_pairs, rank, params):
 
     return synth.evolved_pairs(n_pairs, 1000, seed=0xC0FFEE + 7919 * rank, trim=int(params.constraintDiagonalTrim),
                                expansion=int(params.diagonalExpansion))
+
+
+def dump_outputs(batch, out_dir, n_sample=1024):
+    """The aligned pairs of the batch's last run, as cpb_batch_fetch_pairs hands them to a caller, in float64 (exact for these
+    integers).  All of them would be ~1.3 GB at 100 000 pairs, so: offsets.npy, where each pair's triples start (n + 1);
+    pint_sum.npy, the sum of pInt over each pair's triples (n); triples_sample.npy, the triples of a fixed, seeded sample of
+    n_sample pairs in the order they are returned, columns (pair, pInt, x, y) -- about 36 MB at 1 kb pairs."""
+    off, tri = batch.fetch_pairs(0)
+    n = len(off) - 1
+    csum = np.concatenate([[0], np.cumsum(tri[:, 0], dtype=np.int64)])
+    pick = np.sort(np.random.default_rng(0).choice(n, size=min(n, n_sample), replace=False))
+    sample = [np.column_stack([np.full(off[p + 1] - off[p], p), tri[off[p]:off[p + 1]]]) for p in pick]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "offsets.npy"), off.astype(np.float64))
+    np.save(os.path.join(out_dir, "pint_sum.npy"), (csum[off[1:]] - csum[off[:-1]]).astype(np.float64))
+    np.save(os.path.join(out_dir, "triples_sample.npy"), np.concatenate(sample or [np.zeros((0, 4))]).astype(np.float64))
 
 
 def cpu_arm(packed, n_sample, threads):
@@ -259,7 +277,12 @@ def main():
     ap.add_argument("--capi-pairs", type=int, default=20000, help="pairs of the workload sent through the reference-named C API (e2e_capi)")
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only: no end-to-end arm")
     ap.add_argument("--skip-cpu", action="store_true", help="profiling runs only: no CPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the aligned pairs of the last timed step to DIR/*.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the CUDA path computed: not with --impl reference")
 
     # Every timed pass plans its run anew (regions, bands, traceback schedule, chunks, work lists), as the first call on a new batch
     # does: the engine would otherwise keep the plan of a batch that is run again with the same parameters (what EM iterations do).
@@ -361,6 +384,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     st = batch.stats()
     cells, n_triples = int(st.cells), int(st.outputTriples)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(batch, args.dump_outputs)
     t = torch.tensor([ms, float(cells), float(args.pairs)], dtype=torch.float64, device="cuda")
     if dist is not None:
         tmax = t.clone()
@@ -382,7 +407,7 @@ def main():
     out_pinned = torch.empty((max(n_triples, 1) + 1024, 3), dtype=torch.int32).pin_memory()
     h2d = int(packed["xOff"][-1] + packed["yOff"][-1] + 12 * packed["aOff"][-1])
     d2h = int(n_triples * 12)
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
 
     def one_e2e():
         b = cp.Batch(ctx, None, None, packed=pinned)

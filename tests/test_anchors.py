@@ -1,11 +1,12 @@
 """Anchors without a subprocess (SURVEY.md section 8f, N3): host/anchors.c of libcpecan.so.
 
-filterToRemoveOverlap and the two-level scheme are the reference's own logic and are compared with the reference build
-(oracle/_ref) on fuzzed lists; getBlastPairs replaces the LASTZ subprocess by an in-process seed-and-chain aligner, whose anchors are
-checked for what anchors must be: strictly increasing after the filter, inside the matrix, and ON the true alignment of
+filterToRemoveOverlap and the two-level scheme are the reference's own logic; the filter is compared with the reference build
+(oracle/_ref) on fuzzed lists where that build exists, and with its recorded outputs (tests/golden/anchor_lists.json);
+getBlastPairs replaces the LASTZ subprocess by an in-process seed-and-chain aligner, whose anchors are checked for what anchors must be: strictly increasing after the filter, inside the matrix, and ON the true alignment of
 synthetic evolved pairs.  (What the DP makes of them is checked on the GPU in tests/test_gpu_anchors.py.)
 """
 import ctypes as C
+import json
 import os
 
 import numpy as np
@@ -15,6 +16,7 @@ import helpers
 from cpecan_b200 import synth
 
 LIB = os.environ.get("CPECAN_HOST_LIB") or os.path.join(helpers.ROOT, "cpecan_b200", "lib", "libcpecan.so")
+GOLDEN = os.path.join(helpers.ROOT, "tests", "golden", "anchor_lists.json")
 
 
 class Lists:
@@ -62,10 +64,8 @@ def ours():
     return Lists(LIB)
 
 
-def test_filter_to_remove_overlap_matches_the_reference(ours):
-    if helpers.ref_oracle() is None:
-        pytest.skip("needs the reference build (oracle/_ref)")
-    ref = Lists(helpers.REF_SO)
+def overlap_cases():
+    """300 sorted, overlapping anchor lists (seeded), every fifth with an exact duplicate"""
     rng = np.random.default_rng(5)
     for rep in range(300):
         n = int(rng.integers(0, 60))
@@ -73,11 +73,36 @@ def test_filter_to_remove_overlap_matches_the_reference(ours):
         t = sorted({(int(rng.integers(0, span)), int(rng.integers(0, span)), int(rng.integers(0, 3))) for _ in range(n)})
         if rep % 5 == 0 and t:
             t = sorted(t + [t[int(rng.integers(0, len(t)))]])  # an exact duplicate
-        a, b = ours.make(t), ref.make(t)
-        got, want = ours.read(ours.L.filterToRemoveOverlap(a)), ref.read(ref.L.filterToRemoveOverlap(b))
-        ours.L.stList_destruct(a)
-        ref.L.stList_destruct(b)
-        assert got == want, t
+        yield t
+
+
+def filtered(lists, t):
+    a = lists.make(t)
+    out = lists.read(lists.L.filterToRemoveOverlap(a))
+    lists.L.stList_destruct(a)
+    return out
+
+
+def test_filter_to_remove_overlap_matches_the_reference(ours):
+    if helpers.ref_oracle() is None:
+        pytest.skip("needs the reference build (oracle/_ref)")
+    ref = Lists(helpers.REF_SO)
+    for t in overlap_cases():
+        got = filtered(ours, t)
+        assert got == filtered(ref, t), t
+        assert all(p[0] < q[0] and p[1] < q[1] for p, q in zip(got, got[1:]))
+
+
+def test_filter_to_remove_overlap_matches_the_recorded_lists(ours):
+    """the same lists against tests/golden/anchor_lists.json (tools/make_anchor_golden.py), so that the filter is checked where
+    the reference build is not"""
+    with open(GOLDEN) as f:
+        want = json.load(f)["filterToRemoveOverlap"]
+    cases = list(overlap_cases())
+    assert len(want) == len(cases)
+    for t, w in zip(cases, want):
+        got = filtered(ours, t)
+        assert [list(p) for p in got] == w, t
         assert all(p[0] < q[0] and p[1] < q[1] for p, q in zip(got, got[1:]))
 
 

@@ -3,7 +3,8 @@ gap reweighting, scores, the maximal-expected-accuracy alignment, left shift and
 
 Checked (i) live against the reference's own functions in oracle/_ref (impl/pairwiseAligner.c:979-1003, :1519-1792 compiled
 unmodified) where that build exists, (ii) against tests/golden/realign_cases.json, generated from the same reference build by
-tools/make_realign_golden.py, and (iii) the chain -- which the reference computes inside its multiple aligner with randomised
+tools/make_realign_golden.py, and for the anchors from cigars against this library's recorded outputs (tests/golden/anchor_lists.json,
+tools/make_anchor_golden.py), and (iii) the chain -- which the reference computes inside its multiple aligner with randomised
 weights -- against a quadratic dynamic programme.  No GPU involved.
 """
 import ctypes as C
@@ -259,11 +260,17 @@ def test_chain_of_nothing_and_of_one(host):
     assert host.chain(np.array([[8000000, 2, 1]]), "ACGT", "ACGT", 0.85).shape == (0, 3)
 
 
-def test_cigar_anchors_match_the_reference(host):
-    ref = helpers.ref_oracle()
-    if ref is None:
-        pytest.skip("oracle/_ref not built here")
-    ref = Ref(ref)
+def cigar_cases():
+    """30 seeded alignments as (operations, start1, start2, trim, expansion)"""
+    rng = np.random.default_rng(11)
+    for _ in range(30):
+        ops = np.array([(int(rng.integers(0, 3)), int(rng.integers(1, 12))) for _ in range(int(rng.integers(1, 9)))], dtype=np.int64)
+        s1, s2, trim, e = int(rng.integers(0, 50)), int(rng.integers(0, 50)), int(rng.integers(0, 4)), 2 * int(rng.integers(0, 6))
+        yield ops, s1, s2, trim, e
+
+
+def host_cigar_anchors(host, ops, s1, s2, trim, e):
+    """convertPairwiseForwardStrandAlignmentToAnchorPairs of libcpecan.so on one alignment"""
     L = host.L
     vp, i64 = C.c_void_p, C.c_int64
     L.constructEmptyList.restype = vp
@@ -276,19 +283,34 @@ def test_cigar_anchors_match_the_reference(host):
     L.destructPairwiseAlignment.argtypes = [vp]
     L.convertPairwiseForwardStrandAlignmentToAnchorPairs.restype = vp
     L.convertPairwiseForwardStrandAlignmentToAnchorPairs.argtypes = [vp, i64, i64]
-    rng = np.random.default_rng(11)
-    for _ in range(30):
-        ops = np.array([(int(rng.integers(0, 3)), int(rng.integers(1, 12))) for _ in range(int(rng.integers(1, 9)))], dtype=np.int64)
-        s1, s2, trim, e = int(rng.integers(0, 50)), int(rng.integers(0, 50)), int(rng.integers(0, 4)), 2 * int(rng.integers(0, 6))
-        opList = L.constructEmptyList(0, C.cast(L.destructAlignmentOperation, vp))
-        for t, n in ops:
-            L.listAppend(opList, L.constructAlignmentOperation(int(t), int(n), 0.0))  # 0 match, 1 indel X, 2 indel Y (cpecan/pairwiseAlignment.h)
-        e1 = s1 + int(ops[ops[:, 0] != 2, 1].sum())
-        e2 = s2 + int(ops[ops[:, 0] != 1, 1].sum())
-        pA = L.constructPairwiseAlignment(b"a", s1, e1, 1, b"b", s2, e2, 1, 0.0, opList)
-        got = host.from_list(L.convertPairwiseForwardStrandAlignmentToAnchorPairs(pA, trim, e))
-        L.destructPairwiseAlignment(pA)
-        assert got.tolist() == ref.cigar_anchors(ops, s1, s2, trim, e).tolist()
+    opList = L.constructEmptyList(0, C.cast(L.destructAlignmentOperation, vp))
+    for t, n in ops:
+        L.listAppend(opList, L.constructAlignmentOperation(int(t), int(n), 0.0))  # 0 match, 1 indel X, 2 indel Y (cpecan/pairwiseAlignment.h)
+    e1 = s1 + int(ops[ops[:, 0] != 2, 1].sum())
+    e2 = s2 + int(ops[ops[:, 0] != 1, 1].sum())
+    pA = L.constructPairwiseAlignment(b"a", s1, e1, 1, b"b", s2, e2, 1, 0.0, opList)
+    got = host.from_list(L.convertPairwiseForwardStrandAlignmentToAnchorPairs(pA, trim, e))
+    L.destructPairwiseAlignment(pA)
+    return got
+
+
+def test_cigar_anchors_match_the_reference(host):
+    ref = helpers.ref_oracle()
+    if ref is None:
+        pytest.skip("oracle/_ref not built here")
+    ref = Ref(ref)
+    for case in cigar_cases():
+        assert host_cigar_anchors(host, *case).tolist() == ref.cigar_anchors(*case).tolist()
+
+
+def test_cigar_anchors_match_the_recorded_lists(host):
+    """the same alignments against tests/golden/anchor_lists.json (tools/make_anchor_golden.py), so that the conversion is checked
+    where the reference build is not"""
+    want = json.load(open(os.path.join(ROOT, "tests", "golden", "anchor_lists.json")))["cigarAnchors"]
+    cases = list(cigar_cases())
+    assert len(want) == len(cases)
+    for case, w in zip(cases, want):
+        assert host_cigar_anchors(host, *case).tolist() == w
 
 
 CIGARS = """cigar: b 0 10 + a 5 16 + 57.500000 M 4 D 1 M 6
