@@ -30,6 +30,9 @@ from .binding import (  # noqa: F401
     hmm_getStateMachine,
     getSplitPoints,
     default_context,
+    getAlignedPairs,
+    getAlignedPairsWithIndels,
+    getExpectations,
     getAlignedPairsUsingAnchors,
     getAlignedPairsWithIndelsUsingAnchors,
     getExpectationsUsingAnchors,

@@ -114,6 +114,11 @@ def _load():
     L.cpb_band.argtypes = [C.c_void_p, P(C.c_int64), C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int, P(C.c_int64)]
     L.cpb_batch_create.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, P(C.c_void_p)]
+    L.cpb_batch_create_anchored.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            P(CpbParams), P(C.c_void_p)]
+    L.cpb_batch_anchor_count.restype = C.c_int64
+    L.cpb_batch_anchor_count.argtypes = [C.c_void_p]
+    L.cpb_batch_fetch_anchors.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.cpb_batch_destroy.argtypes = [C.c_void_p]
     L.cpb_batch_run.argtypes = [C.c_void_p, P(CpbModel), P(CpbParams), C.c_int]
     L.cpb_batch_stats.argtypes = [C.c_void_p, P(CpbRunStats)]
@@ -249,6 +254,22 @@ def _as_bytes(s):
     return s.encode() if isinstance(s, str) else bytes(s)
 
 
+def _pack_sequences(seqs):
+    """-> (concatenated uint8 bytes, int64 offsets[n+1])"""
+    s = [_as_bytes(q) for q in seqs]
+    off = np.zeros(len(s) + 1, dtype=np.int64)
+    np.cumsum([len(q) for q in s], out=off[1:])
+    return np.frombuffer(b"".join(s) + b"\0", dtype=np.uint8), off
+
+
+def _ragged(flags):
+    return np.ascontiguousarray(flags, dtype=np.uint8) if flags is not None else None
+
+
+def _ptr(a):
+    return C.c_void_p(a.ctypes.data) if a is not None else None
+
+
 class Batch:
     """n independent (seqX, seqY, anchors, ragged flags) problems resident on the device."""
 
@@ -262,29 +283,40 @@ class Batch:
             rl, rr = packed.get("rl"), packed.get("rr")
         else:
             self.n = len(seqsX)
-            sx = [_as_bytes(s) for s in seqsX]
-            sy = [_as_bytes(s) for s in seqsY]
-            bx = np.frombuffer(b"".join(sx) + b"\0", dtype=np.uint8)
-            by = np.frombuffer(b"".join(sy) + b"\0", dtype=np.uint8)
-            xo = np.zeros(self.n + 1, dtype=np.int64)
-            yo = np.zeros(self.n + 1, dtype=np.int64)
-            np.cumsum([len(s) for s in sx], out=xo[1:])
-            np.cumsum([len(s) for s in sy], out=yo[1:])
+            bx, xo = _pack_sequences(seqsX)
+            by, yo = _pack_sequences(seqsY)
             alist = [_anchor_array(a) for a in (anchors if anchors is not None else [[]] * self.n)]
             ao = np.zeros(self.n + 1, dtype=np.int64)
             np.cumsum([a.size // 3 for a in alist], out=ao[1:])
             an = np.concatenate(alist) if alist and ao[-1] > 0 else np.zeros(3, dtype=np.int64)
-            rl = np.ascontiguousarray(raggedLeft, dtype=np.uint8) if raggedLeft is not None else None
-            rr = np.ascontiguousarray(raggedRight, dtype=np.uint8) if raggedRight is not None else None
+            rl, rr = _ragged(raggedLeft), _ragged(raggedRight)
         self._keep = (bx, xo, by, yo, an, ao, rl, rr)
         h = C.c_void_p()
-
-        def ptr(a):
-            return C.c_void_p(a.ctypes.data) if a is not None else None
-
-        _check(lib.cpb_batch_create(ctx.h, self.n, ptr(bx), ptr(xo), ptr(by), ptr(yo), ptr(an), ptr(ao), ptr(rl), ptr(rr), C.byref(h)))
+        _check(lib.cpb_batch_create(ctx.h, self.n, _ptr(bx), _ptr(xo), _ptr(by), _ptr(yo), _ptr(an), _ptr(ao), _ptr(rl), _ptr(rr), C.byref(h)))
         self.h = h
         self.S = None
+
+    @classmethod
+    def anchored(cls, ctx, seqsX, seqsY, params, raggedLeft=None, raggedRight=None):
+        """A batch whose anchors the device finds from the raw sequences: per pair the triples libcpecan.so's
+        getBlastPairsForPairwiseAlignmentParameters returns for `params` (lower case is the soft mask)."""
+        self = cls.__new__(cls)
+        self.ctx, self.n, self.S, self.h = ctx, len(seqsX), None, None
+        bx, xo = _pack_sequences(seqsX)
+        by, yo = _pack_sequences(seqsY)
+        rl, rr = _ragged(raggedLeft), _ragged(raggedRight)
+        h = C.c_void_p()
+        _check(lib.cpb_batch_create_anchored(ctx.h, self.n, _ptr(bx), _ptr(xo), _ptr(by), _ptr(yo), _ptr(rl), _ptr(rr), C.byref(params), C.byref(h)))
+        self.h = h
+        return self
+
+    def fetch_anchors(self):
+        """-> (offsets[n+1] int64, triples[m, 3] int64 (x, y, expansion)): the anchors the batch holds, the caller's or the device's"""
+        m = int(lib.cpb_batch_anchor_count(self.h))
+        off = np.zeros(self.n + 1, dtype=np.int64)
+        tri = np.zeros((max(m, 1), 3), dtype=np.int64)
+        _check(lib.cpb_batch_fetch_anchors(self.h, C.c_void_p(off.ctypes.data), C.c_void_p(tri.ctypes.data)))
+        return off, tri[:m]
 
     def run(self, model, params, mode):
         self.S = model.stateNumber
@@ -386,6 +418,41 @@ def getAlignedPairsWithIndelsUsingAnchors(sM, sX, sY, anchorPairs, p, alignmentH
 def getExpectationsUsingAnchors(sM, hmmExpectations, sX, sY, anchorPairs, p, alignmentHasRaggedLeftEnd=False, alignmentHasRaggedRightEnd=False, ctx=None):
     """Accumulates into hmmExpectations (a float64 array of hmm_len(S): transitions, emissions, likelihood) (inc/pairwiseAligner.h:105)."""
     b = _one(sM, sX, sY, anchorPairs, p, alignmentHasRaggedLeftEnd, alignmentHasRaggedRightEnd, MODE_EXPECTATIONS, ctx)
+    _, tot = b.fetch_expectations(per_pair=False)
+    b.close()
+    hmmExpectations += tot
+    return hmmExpectations
+
+
+# ---- the same from raw sequences, anchored on the device as the reference's getAlignedPairs anchors them ----
+def _one_anchored(sM, sX, sY, p, raggedLeft, raggedRight, mode, ctx):
+    b = Batch.anchored(ctx or default_context(), [sX], [sY], p, [int(raggedLeft)], [int(raggedRight)])
+    b.run(sM, p, mode)
+    return b
+
+
+def getAlignedPairs(sM, sX, sY, p, alignmentHasRaggedLeftEnd=False, alignmentHasRaggedRightEnd=False, ctx=None):
+    """-> list of (pInt, x, y) (inc/pairwiseAligner.h:58)"""
+    b = _one_anchored(sM, sX, sY, p, alignmentHasRaggedLeftEnd, alignmentHasRaggedRightEnd, MODE_ALIGNED_PAIRS, ctx)
+    _, tri = b.fetch_pairs(0)
+    b.close()
+    return [tuple(int(v) for v in t) for t in tri]
+
+
+def getAlignedPairsWithIndels(sM, sX, sY, p, alignmentHasRaggedLeftEnd=False, alignmentHasRaggedRightEnd=False, ctx=None):
+    """-> (alignedPairs, gapXPairs, gapYPairs) (inc/pairwiseAligner.h:60)"""
+    b = _one_anchored(sM, sX, sY, p, alignmentHasRaggedLeftEnd, alignmentHasRaggedRightEnd, MODE_ALIGNED_PAIRS_INDELS, ctx)
+    out = []
+    for which in range(3):
+        _, tri = b.fetch_pairs(which)
+        out.append([tuple(int(v) for v in t) for t in tri])
+    b.close()
+    return tuple(out)
+
+
+def getExpectations(sM, hmmExpectations, sX, sY, p, alignmentHasRaggedLeftEnd=False, alignmentHasRaggedRightEnd=False, ctx=None):
+    """Accumulates into hmmExpectations, as getExpectationsUsingAnchors (inc/pairwiseAligner.h:74)."""
+    b = _one_anchored(sM, sX, sY, p, alignmentHasRaggedLeftEnd, alignmentHasRaggedRightEnd, MODE_EXPECTATIONS, ctx)
     _, tot = b.fetch_expectations(per_pair=False)
     b.close()
     hmmExpectations += tot

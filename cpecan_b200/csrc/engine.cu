@@ -26,6 +26,7 @@
 #include "kernels.cuh"
 #include "strip_kernels.cuh"
 #include "narrow_kernels.cuh"
+#include "anchor_kernels.cuh"
 
 using namespace cpb;
 
@@ -394,9 +395,13 @@ struct cpb_batch {
     CpbRunStats planStats;
 };
 
-extern "C" int cpb_batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY, const int64_t *yOff,
-                                const int64_t *anchors, const int64_t *anchorOff, const uint8_t *raggedLeft, const uint8_t *raggedRight,
-                                cpb_batch **out) {
+static int find_anchors(cpb_batch *b, const CpbParams *p);
+
+/* cpb_batch_create and cpb_batch_create_anchored: the caller's anchors, or (anchorParams != nullptr) those find_anchors makes on the
+ * device from the raw sequences before they are encoded */
+static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY, const int64_t *yOff,
+                        const int64_t *anchors, const int64_t *anchorOff, const CpbParams *anchorParams, const uint8_t *raggedLeft,
+                        const uint8_t *raggedRight, cpb_batch **out) {
     if (ctx == nullptr || out == nullptr || nPairs < 0 || xOff == nullptr || yOff == nullptr) {
         cpb_set_error("cpb_batch_create: bad argument");
         return CPB_ERR_ARGUMENT;
@@ -453,21 +458,20 @@ extern "C" int cpb_batch_create(cpb_context *ctx, int64_t nPairs, const char *se
     const int64_t nx = xOff[nPairs], ny = yOff[nPairs];
     int rc = CPB_OK;
     /* the strip kernels index symbols up to 32 positions outside a region without bounds tests: pad both ends with 'n' */
-    if ((rc = b->symX.reserve(nx + 2 * kSymPad)) != CPB_OK || (rc = b->symY.reserve(ny + 2 * kSymPad)) != CPB_OK ||
-        (rc = b->dAnchors.reserve(std::max<int64_t>(nA, 1) * 3 * sizeof(int32_t))) != CPB_OK)
-        return rc;
+    if ((rc = b->symX.reserve(nx + 2 * kSymPad)) != CPB_OK || (rc = b->symY.reserve(ny + 2 * kSymPad)) != CPB_OK) return rc;
     cudaStream_t st = ctx->stream;
     CUDA_TRY(cudaMemsetAsync(b->symX.p, 4, nx + 2 * kSymPad, st));
     CUDA_TRY(cudaMemsetAsync(b->symY.p, 4, ny + 2 * kSymPad, st));
-    if (nx > 0) {
-        CUDA_TRY(cudaMemcpyAsync(b->symX.as<uint8_t>() + kSymPad, seqX, nx, cudaMemcpyHostToDevice, st));
-        k_encode<<<(unsigned) ((nx + 255) / 256), 256, 0, st>>>(b->symX.as<uint8_t>() + kSymPad, nx);
+    if (nx > 0) CUDA_TRY(cudaMemcpyAsync(b->symX.as<uint8_t>() + kSymPad, seqX, nx, cudaMemcpyHostToDevice, st));
+    if (ny > 0) CUDA_TRY(cudaMemcpyAsync(b->symY.as<uint8_t>() + kSymPad, seqY, ny, cudaMemcpyHostToDevice, st));
+    if (anchorParams != nullptr) {
+        if ((rc = find_anchors(b, anchorParams)) != CPB_OK) return rc; /* reads the raw bytes: the soft mask is their case */
+    } else if ((rc = b->dAnchors.reserve(std::max<int64_t>(nA, 1) * 3 * sizeof(int32_t))) != CPB_OK) {
+        return rc;
     }
-    if (ny > 0) {
-        CUDA_TRY(cudaMemcpyAsync(b->symY.as<uint8_t>() + kSymPad, seqY, ny, cudaMemcpyHostToDevice, st));
-        k_encode<<<(unsigned) ((ny + 255) / 256), 256, 0, st>>>(b->symY.as<uint8_t>() + kSymPad, ny);
-    }
-    if (nA > 0) {
+    if (nx > 0) k_encode<<<(unsigned) ((nx + 255) / 256), 256, 0, st>>>(b->symX.as<uint8_t>() + kSymPad, nx);
+    if (ny > 0) k_encode<<<(unsigned) ((ny + 255) / 256), 256, 0, st>>>(b->symY.as<uint8_t>() + kSymPad, ny);
+    if (anchorParams == nullptr && nA > 0) {
         /* int64 triples of the caller -> int32 triples, straight into a page-locked buffer that serves both the copy to the device
          * and the host-side region construction of every run; a few host threads share the conversion */
         const size_t bytes = (size_t) (3 * nA) * sizeof(int32_t);
@@ -539,6 +543,34 @@ extern "C" int cpb_batch_create(cpb_context *ctx, int64_t nPairs, const char *se
     return CPB_OK;
 }
 
+extern "C" int cpb_batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY, const int64_t *yOff,
+                                const int64_t *anchors, const int64_t *anchorOff, const uint8_t *raggedLeft, const uint8_t *raggedRight,
+                                cpb_batch **out) {
+    return batch_create(ctx, nPairs, seqX, xOff, seqY, yOff, anchors, anchorOff, nullptr, raggedLeft, raggedRight, out);
+}
+
+extern "C" int cpb_batch_create_anchored(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY,
+                                         const int64_t *yOff, const uint8_t *raggedLeft, const uint8_t *raggedRight, const CpbParams *p,
+                                         cpb_batch **out) {
+    if (p == nullptr || p->constraintDiagonalTrim < 0 || p->diagonalExpansion < 0 || p->diagonalExpansion > 0x7FFFFFFF) {
+        cpb_set_error("cpb_batch_create_anchored: %s", p == nullptr ? "no parameters" : "constraintDiagonalTrim and diagonalExpansion must be in [0, 2^31)");
+        return CPB_ERR_ARGUMENT;
+    }
+    return batch_create(ctx, nPairs, seqX, xOff, seqY, yOff, nullptr, nullptr, p, raggedLeft, raggedRight, out);
+}
+
+extern "C" int64_t cpb_batch_anchor_count(const cpb_batch *b) { return b != nullptr ? b->aOff[b->n] : 0; }
+
+extern "C" int cpb_batch_fetch_anchors(const cpb_batch *b, int64_t *offsets, int64_t *triples) {
+    if (b == nullptr || offsets == nullptr || (triples == nullptr && b->aOff[b->n] > 0)) {
+        cpb_set_error("cpb_batch_fetch_anchors: bad argument");
+        return CPB_ERR_ARGUMENT;
+    }
+    memcpy(offsets, b->aOff.data(), (size_t) (b->n + 1) * sizeof(int64_t));
+    for (int64_t k = 0; k < 3 * b->aOff[b->n]; k++) triples[k] = b->anchors[k];
+    return CPB_OK;
+}
+
 extern "C" void cpb_batch_destroy(cpb_batch *b) {
     if (b == nullptr) return;
     cudaSetDevice(b->ctx->device);
@@ -548,6 +580,254 @@ extern "C" void cpb_batch_destroy(cpb_batch *b) {
     for (DevBuf *d : bufs) d->release();
     if (b->anchors != nullptr && b->anchorsOwn.empty()) b->ctx->pinned.give(b->anchors);
     delete b;
+}
+
+/* ------------------------------------------------------------------------------------------------
+ * anchors on the device (anchor_kernels.cuh): getBlastPairsForPairwiseAlignmentParameters of host/anchors.c for every pair at once
+ * ---------------------------------------------------------------------------------------------- */
+/* word_length of anchors.c: the smallest k in 11..24 with 4^k >= 64 max(lX, lY) */
+static int anchor_word_length(int64_t lX, int64_t lY) {
+    int k = 11;
+    double space = 4194304.0; /* 4^11 */
+    while (k < 24 && space < 64.0 * (double) (lX < lY ? lY : lX)) {
+        k++;
+        space *= 4.0;
+    }
+    return k;
+}
+
+/* exclusive scan of n int32 counts into offsets[0..n], offsets[n] = startAt + the sum (tiles: (n + SCAN_TILE - 1) / SCAN_TILE entries) */
+static void scan_counts(cudaStream_t st, const int32_t *counts, int64_t n, int64_t startAt, int64_t *tiles, int64_t *offsets) {
+    const int64_t nTiles = (n + SCAN_TILE - 1) / SCAN_TILE;
+    if (nTiles > 0) k_scan_tiles<<<(unsigned) nTiles, 256, 0, st>>>(counts, n, tiles);
+    k_scan_sums<<<1, 1, 0, st>>>(tiles, nTiles, startAt, offsets + n);
+    if (nTiles > 0) k_scan_apply<<<(unsigned) nTiles, 256, 0, st>>>(counts, n, tiles, offsets);
+}
+
+static unsigned grid_of(int64_t n, int threads) { return (unsigned) std::max<int64_t>(1, (n + threads - 1) / threads); }
+
+/* Scratch bytes of one problem: its k-mer table, 40 bytes per X position (hit, seed flag, seed offset, seed, chain arrays), 8 per Y
+ * position (the Fenwick tree) and its records. */
+static size_t anchor_problem_bytes(int64_t lX, int64_t lY, int64_t tableEntries) {
+    return (size_t) (16 * tableEntries + 40 * lX + 8 * (lY + 2) + sizeof(AnchorProblem) + 64);
+}
+
+/* Every problem's anchors: triples into tri (capacity: the problems' lX summed), problem p's at [off[p], off[p + 1]).  probs holds the
+ * problems' x, y, lX, lY, mask, dx, dy; the rest is filled in here.  The problems go through the kernels in chunks whose scratch fits the
+ * context's budget. */
+static int anchor_problems(cpb_batch *b, std::vector<AnchorProblem> &probs, const CpbParams *p, DevBuf &tri, DevBuf &off, int64_t *total) {
+    cpb_context *ctx = b->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t nP = (int64_t) probs.size();
+    int64_t bound = 0;
+    for (AnchorProblem &P : probs) bound += P.lX;
+    int rc;
+    if ((rc = tri.reserve((size_t) std::max<int64_t>(bound, 1) * 3 * sizeof(int32_t))) != CPB_OK ||
+        (rc = off.reserve((size_t) (nP + 1) * sizeof(int64_t))) != CPB_OK)
+        return rc;
+    size_t budget = ctx->scratchBudget;
+    if (budget == 0) {
+        size_t freeB = 0, totalB = 0;
+        CUDA_TRY(cudaMemGetInfo(&freeB, &totalB));
+        budget = (size_t) ((double) (freeB + ctx->scratch.cap) * 0.70);
+    }
+    const size_t fixed = 16 * 256; /* alignment of the chunk's arrays */
+    int64_t running = 0;
+    for (int64_t p0 = 0; p0 < nP;) {
+        int64_t p1 = p0, X = 0, Y = 0, E = 0;
+        size_t bytes = fixed;
+        while (p1 < nP) {
+            AnchorProblem &P = probs[(size_t) p1];
+            int64_t cap = 16;
+            while (cap < 2 * (int64_t) P.lY) cap <<= 1;
+            const size_t need = anchor_problem_bytes(P.lX, P.lY, cap);
+            if (fixed + need > budget) {
+                cpb_set_error("anchoring a %d x %d problem needs %zu bytes of scratch, more than the budget of %zu", P.lX, P.lY, fixed + need, budget);
+                return CPB_ERR_MEMORY;
+            }
+            if (bytes + need > budget || p1 - p0 >= (1 << 30)) break;
+            bytes += need;
+            P.k = anchor_word_length(P.lX, P.lY);
+            P.capMask = (int32_t) (cap - 1);
+            P.xPos = X;
+            P.yPos = Y;
+            P.tab = E;
+            X += P.lX;
+            Y += P.lY + 2;
+            E += cap;
+            p1++;
+        }
+        const int nC = (int) (p1 - p0);
+        /* the chunk's arrays, 256-byte aligned, in ctx->scratch */
+        size_t at = 0;
+        auto carve = [&](size_t n) {
+            const size_t here = at;
+            at += (n + 255) & ~(size_t) 255;
+            return here;
+        };
+        const size_t oDesc = carve(nC * sizeof(AnchorProblem)), oTab = carve(E * sizeof(KmerEntry)), oHit = carve(X * 4), oFlag = carve(X * 4),
+                     oSeedOff = carve((X + 1) * 8), oSeeds = carve(X * sizeof(int3)), oScore = carve(X * 4), oPrev = carve(X * 4), oOrder = carve(X * 4),
+                     oFenS = carve(Y * 4), oFenW = carve(Y * 4), oChain = carve(nC * 4), oCount = carve(nC * 4),
+                     oTiles = carve(((std::max(X, (int64_t) nC) + SCAN_TILE - 1) / SCAN_TILE + 1) * 8);
+        if ((rc = ctx->scratch.reserve(std::max<size_t>(at, 256))) != CPB_OK) return rc;
+        char *s = ctx->scratch.as<char>();
+        AnchorProblem *dP = reinterpret_cast<AnchorProblem *>(s + oDesc);
+        KmerEntry *dTab = reinterpret_cast<KmerEntry *>(s + oTab);
+        int32_t *dHit = reinterpret_cast<int32_t *>(s + oHit), *dFlag = reinterpret_cast<int32_t *>(s + oFlag);
+        int64_t *dSeedOff = reinterpret_cast<int64_t *>(s + oSeedOff), *dTiles = reinterpret_cast<int64_t *>(s + oTiles);
+        int3 *dSeeds = reinterpret_cast<int3 *>(s + oSeeds);
+        int32_t *dScore = reinterpret_cast<int32_t *>(s + oScore), *dPrev = reinterpret_cast<int32_t *>(s + oPrev), *dOrder = reinterpret_cast<int32_t *>(s + oOrder);
+        int32_t *dFenS = reinterpret_cast<int32_t *>(s + oFenS), *dFenW = reinterpret_cast<int32_t *>(s + oFenW);
+        int32_t *dChain = reinterpret_cast<int32_t *>(s + oChain), *dCount = reinterpret_cast<int32_t *>(s + oCount);
+        const uint8_t *sx = b->symX.as<uint8_t>(), *sy = b->symY.as<uint8_t>();
+        int64_t *dOff = off.as<int64_t>() + p0;
+        CUDA_TRY(cudaMemcpyAsync(dP, probs.data() + p0, nC * sizeof(AnchorProblem), cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemsetAsync(dTab, 0xFF, E * sizeof(KmerEntry), st));
+        CUDA_TRY(cudaMemsetAsync(dFenS, 0, Y * 4, st));
+        CUDA_TRY(cudaMemsetAsync(dFenW, 0, Y * 4, st));
+        k_anchor_index<<<grid_of(Y, 256), 256, 0, st>>>(dP, nC, Y, sy, dTab);
+        k_anchor_hits<<<grid_of(X, 256), 256, 0, st>>>(dP, nC, X, sx, dTab, dHit);
+        k_anchor_seed_flags<<<grid_of(X, 256), 256, 0, st>>>(dP, nC, X, dHit, dFlag);
+        scan_counts(st, dFlag, X, 0, dTiles, dSeedOff);
+        k_anchor_seeds<<<grid_of(X, 256), 256, 0, st>>>(dP, nC, X, dHit, dFlag, dSeedOff, dSeeds);
+        k_anchor_chain<<<grid_of(nC, 64), 64, 0, st>>>(dP, nC, sx, sy, dSeedOff, dSeeds, dScore, dPrev, dOrder, dFenS, dFenW, p->constraintDiagonalTrim,
+                                                       dChain, dCount);
+        scan_counts(st, dCount, nC, running, dTiles, dOff);
+        k_anchor_runs<<<grid_of(nC, 64), 64, 0, st>>>(dP, nC, sx, sy, dSeedOff, dSeeds, dOrder, dChain, p->constraintDiagonalTrim,
+                                                      (int32_t) p->diagonalExpansion, dOff, tri.as<int32_t>());
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemcpyAsync(&running, dOff + nC, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st)); /* the next chunk's scan starts from this total, and reuses the scratch */
+        p0 = p1;
+    }
+    if (nP == 0) CUDA_TRY(cudaMemsetAsync(off.p, 0, sizeof(int64_t), st));
+    *total = running;
+    return CPB_OK;
+}
+
+/* getBlastPairsForPairwiseAlignmentParameters (anchors.c:361-381) of every pair: level 1 on every matrix bigger than
+ * anchorMatrixBiggerThanThis, level 2 on every gap of those lists that is still that big, merged per pair.  The lists need no sort and
+ * no overlap filter: a chain's triples ascend strictly in x and y, and a gap's lie strictly inside it.  Fills b->aOff, b->anchors (one
+ * copy back), b->dAnchors and b->oddExpansionPair.  The per-position arrays come out of the scratch budget; the lists and the per-gap
+ * tables, which grow with the anchors, are batch buffers like the anchors themselves. */
+static int find_anchors(cpb_batch *b, const CpbParams *p) {
+    cpb_context *ctx = b->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = b->n;
+    std::vector<AnchorProblem> l1;
+    std::vector<int32_t> problemOf((size_t) std::max<int64_t>(n, 1), -1), pairOf, lX1, lY1;
+    for (int64_t i = 0; i < n; i++) {
+        const int64_t lX = b->xOff[i + 1] - b->xOff[i], lY = b->yOff[i + 1] - b->yOff[i];
+        if (lX * lY <= p->anchorMatrixBiggerThanThis) continue;
+        AnchorProblem P;
+        memset(&P, 0, sizeof(P));
+        P.x = kSymPad + b->xOff[i];
+        P.y = kSymPad + b->yOff[i];
+        P.lX = (int32_t) lX;
+        P.lY = (int32_t) lY;
+        P.mask = 1;
+        problemOf[(size_t) i] = (int32_t) l1.size();
+        pairOf.push_back((int32_t) i);
+        lX1.push_back(P.lX);
+        lY1.push_back(P.lY);
+        l1.push_back(P);
+    }
+    const int64_t nP = (int64_t) l1.size();
+    DevBuf tri1, off1, tri2, off2, tab, flags, gapIdx, gaps, sizes, slotPos, tiles, counts, aOffDev;
+    DevBuf *all[] = { &tri1, &off1, &tri2, &off2, &tab, &flags, &gapIdx, &gaps, &sizes, &slotPos, &tiles, &counts, &aOffDev };
+    for (DevBuf *d : all) d->pool = &ctx->pool;
+    int rc;
+    int64_t n1 = 0, n2 = 0;
+    if ((rc = anchor_problems(b, l1, p, tri1, off1, &n1)) != CPB_OK) return rc;
+    /* level 2: gap slot off1[q] + q + g is gap g of problem q */
+    const int64_t nSlots = n1 + nP;
+    const size_t tabBytes = (size_t) (3 * nP + n + 3) * sizeof(int32_t);
+    if ((rc = tab.reserve(tabBytes)) != CPB_OK || (rc = flags.reserve((size_t) (nSlots + 1) * 4)) != CPB_OK ||
+        (rc = gapIdx.reserve((size_t) (nSlots + 1) * 8)) != CPB_OK || (rc = sizes.reserve((size_t) (nSlots + 1) * 4)) != CPB_OK ||
+        (rc = slotPos.reserve((size_t) (nSlots + 1) * 8)) != CPB_OK ||
+        (rc = tiles.reserve((size_t) ((std::max(nSlots, n) + SCAN_TILE - 1) / SCAN_TILE + 1) * 8)) != CPB_OK ||
+        (rc = counts.reserve((size_t) (n + 1) * 4)) != CPB_OK)
+        return rc;
+    int32_t *dLX = tab.as<int32_t>(), *dLY = dLX + nP, *dPairOf = dLY + nP, *dProblemOf = dPairOf + nP;
+    if (nP > 0) {
+        CUDA_TRY(cudaMemcpyAsync(dLX, lX1.data(), nP * 4, cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(dLY, lY1.data(), nP * 4, cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(dPairOf, pairOf.data(), nP * 4, cudaMemcpyHostToDevice, st));
+    }
+    if (n > 0) CUDA_TRY(cudaMemcpyAsync(dProblemOf, problemOf.data(), n * 4, cudaMemcpyHostToDevice, st));
+    const int64_t *dOff1 = off1.as<int64_t>();
+    const int32_t *dTri1 = tri1.as<int32_t>();
+    int64_t nGaps = 0;
+    if (nSlots > 0) {
+        k_anchor_gap_flags<<<grid_of(nSlots, 256), 256, 0, st>>>((int) nP, dOff1, dTri1, dLX, dLY, nSlots, (long long) p->anchorMatrixBiggerThanThis,
+                                                               flags.as<int32_t>());
+        scan_counts(st, flags.as<int32_t>(), nSlots, 0, tiles.as<int64_t>(), gapIdx.as<int64_t>());
+        CUDA_TRY(cudaMemcpyAsync(&nGaps, gapIdx.as<int64_t>() + nSlots, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    if (nGaps > 0) {
+        if ((rc = gaps.reserve((size_t) nGaps * sizeof(AnchorGap))) != CPB_OK) return rc;
+        k_anchor_gap_list<<<grid_of(nSlots, 256), 256, 0, st>>>((int) nP, dOff1, dTri1, dLX, dLY, dPairOf, nSlots, (long long) p->repeatMaskMatrixBiggerThanThis,
+                                                              flags.as<int32_t>(), gapIdx.as<int64_t>(), gaps.as<AnchorGap>());
+        std::vector<AnchorGap> hGaps((size_t) nGaps);
+        CUDA_TRY(cudaMemcpyAsync(hGaps.data(), gaps.p, (size_t) nGaps * sizeof(AnchorGap), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        std::vector<AnchorProblem> l2((size_t) nGaps);
+        for (int64_t q = 0; q < nGaps; q++) {
+            const AnchorGap &G = hGaps[(size_t) q];
+            AnchorProblem &P = l2[(size_t) q];
+            memset(&P, 0, sizeof(P));
+            P.x = kSymPad + b->xOff[G.pair] + G.x;
+            P.y = kSymPad + b->yOff[G.pair] + G.y;
+            P.lX = G.lX;
+            P.lY = G.lY;
+            P.mask = G.mask;
+            P.dx = G.x;
+            P.dy = G.y;
+        }
+        if ((rc = anchor_problems(b, l2, p, tri2, off2, &n2)) != CPB_OK) return rc;
+    }
+    /* merge: every gap slot's position in the final lists, then both levels' triples to their places */
+    const int64_t nA = n1 + n2;
+    if ((rc = b->dAnchors.reserve((size_t) std::max<int64_t>(nA, 1) * 3 * sizeof(int32_t))) != CPB_OK) return rc;
+    int32_t *dOut = b->dAnchors.as<int32_t>();
+    if (nSlots > 0) {
+        k_anchor_slot_sizes<<<grid_of(nSlots, 256), 256, 0, st>>>((int) nP, dOff1, nSlots, flags.as<int32_t>(), gapIdx.as<int64_t>(), off2.as<int64_t>(),
+                                                                sizes.as<int32_t>());
+        scan_counts(st, sizes.as<int32_t>(), nSlots, 0, tiles.as<int64_t>(), slotPos.as<int64_t>());
+        k_anchor_merge_level1<<<grid_of(nSlots, 256), 256, 0, st>>>((int) nP, dOff1, dTri1, nSlots, flags.as<int32_t>(), gapIdx.as<int64_t>(),
+                                                                  off2.as<int64_t>(), slotPos.as<int64_t>(), dOut);
+        if (n2 > 0)
+            k_anchor_merge_level2<<<grid_of(n2, 256), 256, 0, st>>>((int) nGaps, gaps.as<AnchorGap>(), off2.as<int64_t>(), tri2.as<int32_t>(),
+                                                                  slotPos.as<int64_t>(), dOut);
+    }
+    b->aOff.assign((size_t) n + 1, 0);
+    if (n > 0) {
+        if (nP > 0) {
+            k_anchor_pair_counts<<<grid_of(n, 256), 256, 0, st>>>((int) n, dProblemOf, dOff1, slotPos.as<int64_t>(), counts.as<int32_t>());
+        } else {
+            CUDA_TRY(cudaMemsetAsync(counts.p, 0, (size_t) n * 4, st));
+        }
+        if ((rc = aOffDev.reserve((size_t) (n + 1) * 8)) != CPB_OK) return rc;
+        scan_counts(st, counts.as<int32_t>(), n, 0, tiles.as<int64_t>(), aOffDev.as<int64_t>());
+        CUDA_TRY(cudaMemcpyAsync(b->aOff.data(), aOffDev.p, (size_t) (n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    }
+    if (nA > 0) {
+        const size_t bytes = (size_t) (3 * nA) * sizeof(int32_t);
+        b->anchors = static_cast<int32_t *>(ctx->pinned.take(bytes));
+        if (b->anchors == nullptr) {
+            b->anchorsOwn.resize((size_t) (3 * nA));
+            b->anchors = b->anchorsOwn.data();
+        }
+        CUDA_TRY(cudaMemcpyAsync(b->anchors, dOut, bytes, cudaMemcpyDeviceToHost, st));
+    }
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (p->diagonalExpansion & 1) {
+        for (int64_t i = 0; i < n && b->oddExpansionPair < 0; i++)
+            if (b->aOff[(size_t) i + 1] > b->aOff[(size_t) i]) b->oddExpansionPair = i;
+    }
+    return CPB_OK;
 }
 
 /* ------------------------------------------------------------------------------------------------

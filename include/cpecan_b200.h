@@ -126,6 +126,18 @@ int cpb_band(cpb_context *ctx, const int64_t *anchors, int64_t nAnchors, int64_t
 int cpb_batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY, const int64_t *yOff,
                      const int64_t *anchors, const int64_t *anchorOff, const uint8_t *raggedLeft, const uint8_t *raggedRight,
                      cpb_batch **out);
+/* As cpb_batch_create, with every pair's anchors found on the device: the triples, in order, that libcpecan.so's
+ * getBlastPairsForPairwiseAlignmentParameters returns on the host.  Reads p->constraintDiagonalTrim, diagonalExpansion,
+ * anchorMatrixBiggerThanThis, repeatMaskMatrixBiggerThanThis; cpb_batch_run takes its parameters as before.  Lower case is the soft
+ * mask, as there.  The per-position work arrays are processed in chunks that fit the scratch budget; a single problem (a pair's
+ * matrix, or a gap between its anchors) that does not fit returns CPB_ERR_MEMORY.  A negative trim or expansion, or an expansion of
+ * 2^31 or more, returns CPB_ERR_ARGUMENT. */
+int cpb_batch_create_anchored(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY,
+                              const int64_t *yOff, const uint8_t *raggedLeft, const uint8_t *raggedRight, const CpbParams *p,
+                              cpb_batch **out);
+/* the anchors a batch holds, whoever made them: n+1 offsets (in triples), int64 (x, y, expansion) triples */
+int64_t cpb_batch_anchor_count(const cpb_batch *b);
+int cpb_batch_fetch_anchors(const cpb_batch *b, int64_t *offsets, int64_t *triples);
 void cpb_batch_destroy(cpb_batch *b);
 
 /* Runs the whole hot path on the device for the batch; results stay in HBM until fetched.
