@@ -17,6 +17,10 @@ from .binding import (  # noqa: F401
     MODE_ALIGNED_PAIRS_INDELS,
     MODE_EXPECTATIONS,
     MODE_FORWARD,
+    SCORE_IDENTITY,
+    SCORE_IDENTITY_IGNORING_GAPS,
+    SCORE_POSTERIOR,
+    SCORE_POSTERIOR_IGNORING_GAPS,
     fiveState,
     fiveStateAsymmetric,
     threeState,
@@ -37,4 +41,5 @@ from .binding import (  # noqa: F401
     getAlignedPairsWithIndelsUsingAnchors,
     getExpectationsUsingAnchors,
     computeForwardProbability,
+    getShiftedMEAAlignment,
 )

@@ -16,6 +16,7 @@ LIB_PATH = os.environ.get("CPB_LIB") or os.path.join(_HERE, "lib", "libcpecan_b2
 PAIR_ALIGNMENT_PROB_1 = 10000000
 fiveState, fiveStateAsymmetric, threeState, threeStateAsymmetric = 0, 1, 2, 3
 MODE_ALIGNED_PAIRS, MODE_ALIGNED_PAIRS_INDELS, MODE_EXPECTATIONS, MODE_FORWARD = 0, 1, 2, 3
+SCORE_IDENTITY, SCORE_IDENTITY_IGNORING_GAPS, SCORE_POSTERIOR, SCORE_POSTERIOR_IGNORING_GAPS = 0, 1, 2, 3
 
 
 class CpbError(RuntimeError):
@@ -129,6 +130,12 @@ def _load():
     L.cpb_batch_fetch_pairs_reference_order.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     L.cpb_batch_reweight_pairs.argtypes = [C.c_void_p, C.c_double]
     L.cpb_batch_alignment_scores.argtypes = [C.c_void_p, C.c_void_p]
+    L.cpb_batch_ordered_chain.argtypes = [C.c_void_p, C.c_float]
+    L.cpb_batch_mea.argtypes = [C.c_void_p, C.c_float, C.c_int, C.c_void_p]
+    L.cpb_batch_alignments_count.restype = C.c_int64
+    L.cpb_batch_alignments_count.argtypes = [C.c_void_p]
+    L.cpb_batch_fetch_alignments.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    L.cpb_batch_score_alignments.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
     L.cpb_batch_device_triples.restype = C.c_void_p
     L.cpb_batch_device_triples.argtypes = [C.c_void_p, C.c_int]
     L.cpb_batch_fetch_expectations.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
@@ -360,6 +367,33 @@ class Batch:
         _check(lib.cpb_batch_alignment_scores(self.h, C.c_void_p(out.ctypes.data)))
         return out
 
+    def ordered_chain(self, match_gamma):
+        """filterPairwiseAlignmentToMakePairsOrdered (impl/multipleAligner.c:945-972) of every pair's list 0, on the device, into the
+        batch's alignment list (fetch_alignments)"""
+        _check(lib.cpb_batch_ordered_chain(self.h, float(match_gamma)))
+
+    def mea(self, gap_gamma, left_shift=True):
+        """getMaximalExpectedAccuracyPairwiseAlignment (impl/pairwiseAligner.c:1603-1724), and with left_shift leftShiftAlignment
+        (:1726-1767), of every pair of an ALIGNED_PAIRS_INDELS run, on the device, into the alignment list -> alignmentScore float64[n]"""
+        out = np.zeros(max(self.n, 1), dtype=np.float64)
+        _check(lib.cpb_batch_mea(self.h, float(gap_gamma), int(bool(left_shift)), C.c_void_p(out.ctypes.data)))
+        return out[: self.n]
+
+    def fetch_alignments(self):
+        """-> (offsets[n+1] int64, triples[count, 3] int32 (pInt, x, y)): the alignment list of the last decode call"""
+        m = int(lib.cpb_batch_alignments_count(self.h))
+        off = np.zeros(self.n + 1, dtype=np.int64)
+        tri = np.zeros((max(m, 1), 3), dtype=np.int32)
+        _check(lib.cpb_batch_fetch_alignments(self.h, C.c_void_p(off.ctypes.data), C.c_void_p(tri.ctypes.data)))
+        return off, tri[:m]
+
+    def score_alignments(self, kind):
+        """scoreByIdentity / ...IgnoringGaps / scoreByPosteriorProbability / ...IgnoringGaps (kind = SCORE_*, impl/pairwiseAligner.c:1562-1597)
+        of every pair's alignment -> float64[n]"""
+        out = np.zeros(max(self.n, 1), dtype=np.float64)
+        _check(lib.cpb_batch_score_alignments(self.h, int(kind), C.c_void_p(out.ctypes.data)))
+        return out[: self.n]
+
     def fetch_expectations(self, per_pair=True):
         L = hmm_len(self.S)
         pp = np.zeros((self.n, L), dtype=np.float64) if per_pair else None
@@ -457,6 +491,18 @@ def getExpectations(sM, hmmExpectations, sX, sY, p, alignmentHasRaggedLeftEnd=Fa
     b.close()
     hmmExpectations += tot
     return hmmExpectations
+
+
+def getShiftedMEAAlignment(seqX, seqY, anchorPairs, p, sM, alignmentHasRaggedLeftEnd=False, alignmentHasRaggedRightEnd=False, ctx=None):
+    """-> (list of (pInt, x, y), alignmentScore) (impl/pairwiseAligner.c:1769-1792): one ALIGNED_PAIRS_INDELS run, then the maximal expected
+    accuracy alignment with p.gapGamma and its left shift, on the device"""
+    b = _one(sM, seqX, seqY, anchorPairs, p, alignmentHasRaggedLeftEnd, alignmentHasRaggedRightEnd, MODE_ALIGNED_PAIRS_INDELS, ctx)
+    try:
+        score = float(b.mea(p.gapGamma, left_shift=True)[0])
+        _, tri = b.fetch_alignments()
+    finally:
+        b.close()
+    return [tuple(int(v) for v in t) for t in tri], score
 
 
 def computeForwardProbability(seqX, seqY, anchorPairs, p, sM, alignmentHasRaggedLeftEnd=False, alignmentHasRaggedRightEnd=False, ctx=None):

@@ -10,6 +10,7 @@
  * There is no CPU fallback anywhere in this file: without a CUDA device every entry point fails.
  */
 #include <algorithm>
+#include <cfloat>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -27,6 +28,7 @@
 #include "strip_kernels.cuh"
 #include "narrow_kernels.cuh"
 #include "anchor_kernels.cuh"
+#include "decode_kernels.cuh"
 
 using namespace cpb;
 
@@ -374,6 +376,7 @@ struct cpb_batch {
     bool reweighted = false;         /* cpb_batch_reweight_pairs has rewritten list 0 of the last run in place */
     int64_t oddExpansionPair = -1;   /* first pair with an odd anchor expansion: only an error for runs with dynamicAnchorExpansion (:166) */
     DevBuf symX, symY, dAnchors;
+    DevBuf keptX, keptY; /* the sequence bytes upper-cased (toupper): the decoders compare bytes, which the 0..4 symbols cannot */
     DevBuf dPairTab;   /* aOff, xOff, yOff as the device needs them for k_split_flags: 3 x (n + 1) int64 */
     DevBuf splitFlags; /* one bit per gap between anchors: 1 = getSplitPoints cuts the pair there; word 0 of the buffer counts the pairs with a cut */
     /* run state */
@@ -383,6 +386,10 @@ struct cpb_batch {
     DevBuf out[3];
     int64_t outCount[3] = { 0, 0, 0 };
     std::vector<int64_t> pairOff[3]; /* n+1 */
+    /* the alignment list: one alignment per pair from the last decode call (cpb_batch_ordered_chain, cpb_batch_mea), cleared by every run */
+    DevBuf aln;
+    std::vector<int64_t> alnOff; /* n+1 */
+    bool alnValid = false;
     int lastMode = -1, lastS = 0;
     CpbRunStats stats;
     HostArray<RegionDev> hRegions;
@@ -440,7 +447,7 @@ static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, cons
     {
         DevBuf *all[] = { &b->strips, &b->symX, &b->symY, &b->dAnchors, &b->dPairTab, &b->splitFlags, &b->regions, &b->diags, &b->blocks, &b->totals, &b->lists, &b->counts, &b->offsets,
                           &b->masks, &b->tileSums, &b->pairCounts, &b->partials, &b->pairBlockOff, &b->perPair, &b->hmmTotal, &b->forwardOut, &b->out[0],
-                          &b->out[1], &b->out[2], &b->ckRegions, &b->ckDiags, &b->ckSizes, &b->ckpt };
+                          &b->out[1], &b->out[2], &b->ckRegions, &b->ckDiags, &b->ckSizes, &b->ckpt, &b->keptX, &b->keptY, &b->aln };
         for (DevBuf *d : all) d->pool = &ctx->pool;
     }
     b->n = nPairs;
@@ -458,7 +465,9 @@ static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, cons
     const int64_t nx = xOff[nPairs], ny = yOff[nPairs];
     int rc = CPB_OK;
     /* the strip kernels index symbols up to 32 positions outside a region without bounds tests: pad both ends with 'n' */
-    if ((rc = b->symX.reserve(nx + 2 * kSymPad)) != CPB_OK || (rc = b->symY.reserve(ny + 2 * kSymPad)) != CPB_OK) return rc;
+    if ((rc = b->symX.reserve(nx + 2 * kSymPad)) != CPB_OK || (rc = b->symY.reserve(ny + 2 * kSymPad)) != CPB_OK ||
+        (rc = b->keptX.reserve(std::max<int64_t>(nx, 1))) != CPB_OK || (rc = b->keptY.reserve(std::max<int64_t>(ny, 1))) != CPB_OK)
+        return rc;
     cudaStream_t st = ctx->stream;
     CUDA_TRY(cudaMemsetAsync(b->symX.p, 4, nx + 2 * kSymPad, st));
     CUDA_TRY(cudaMemsetAsync(b->symY.p, 4, ny + 2 * kSymPad, st));
@@ -469,8 +478,8 @@ static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, cons
     } else if ((rc = b->dAnchors.reserve(std::max<int64_t>(nA, 1) * 3 * sizeof(int32_t))) != CPB_OK) {
         return rc;
     }
-    if (nx > 0) k_encode<<<(unsigned) ((nx + 255) / 256), 256, 0, st>>>(b->symX.as<uint8_t>() + kSymPad, nx);
-    if (ny > 0) k_encode<<<(unsigned) ((ny + 255) / 256), 256, 0, st>>>(b->symY.as<uint8_t>() + kSymPad, ny);
+    if (nx > 0) k_encode<<<(unsigned) ((nx + 255) / 256), 256, 0, st>>>(b->symX.as<uint8_t>() + kSymPad, b->keptX.as<uint8_t>(), nx);
+    if (ny > 0) k_encode<<<(unsigned) ((ny + 255) / 256), 256, 0, st>>>(b->symY.as<uint8_t>() + kSymPad, b->keptY.as<uint8_t>(), ny);
     if (anchorParams == nullptr && nA > 0) {
         /* int64 triples of the caller -> int32 triples, straight into a page-locked buffer that serves both the copy to the device
          * and the host-side region construction of every run; a few host threads share the conversion */
@@ -576,7 +585,7 @@ extern "C" void cpb_batch_destroy(cpb_batch *b) {
     cudaSetDevice(b->ctx->device);
     DevBuf *bufs[] = { &b->strips, &b->symX, &b->symY, &b->dAnchors, &b->dPairTab, &b->splitFlags, &b->regions, &b->diags, &b->blocks, &b->totals, &b->lists, &b->counts,
                        &b->offsets, &b->masks, &b->tileSums, &b->pairCounts, &b->partials, &b->pairBlockOff, &b->perPair, &b->hmmTotal, &b->forwardOut, &b->out[0], &b->out[1],
-                       &b->out[2], &b->ckRegions, &b->ckDiags, &b->ckSizes, &b->ckpt };
+                       &b->out[2], &b->ckRegions, &b->ckDiags, &b->ckSizes, &b->ckpt, &b->keptX, &b->keptY, &b->aln };
     for (DevBuf *d : bufs) d->release();
     if (b->anchors != nullptr && b->anchorsOwn.empty()) b->ctx->pinned.give(b->anchors);
     delete b;
@@ -1916,6 +1925,7 @@ extern "C" int cpb_batch_run(cpb_batch *b, const CpbModel *m, const CpbParams *p
         cpb_set_error("cpb_batch_run: bad argument");
         return CPB_ERR_ARGUMENT;
     }
+    b->alnValid = false; /* the alignment list belongs to the lists of the run before */
     int rc = check_params(p);
     if (rc != CPB_OK) return rc;
     if (p->dynamicAnchorExpansion && mode != CPB_MODE_FORWARD && b->oddExpansionPair >= 0) {
@@ -2047,13 +2057,13 @@ extern "C" int cpb_batch_fetch_pairs_reference_order(cpb_batch *b, int list, int
     return CPB_OK;
 }
 
-/* device copies of the per-pair offsets the post-posterior kernels need */
-static int upload_pair_tables(cpb_batch *b, int list, DevBuf &dOff, DevBuf &dX, DevBuf &dY) {
+/* device copies of the per-pair offsets the post-posterior kernels need: `off` (n+1 triple offsets of a list), xOff, yOff */
+static int upload_pair_tables(cpb_batch *b, const std::vector<int64_t> &off, DevBuf &dOff, DevBuf &dX, DevBuf &dY) {
     int rc;
     const size_t bytes = (size_t) (b->n + 1) * sizeof(int64_t);
     if ((rc = dOff.reserve(bytes)) != CPB_OK || (rc = dX.reserve(bytes)) != CPB_OK || (rc = dY.reserve(bytes)) != CPB_OK) return rc;
     cudaStream_t st = b->ctx->stream;
-    CUDA_TRY(cudaMemcpyAsync(dOff.p, b->pairOff[list].data(), bytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(dOff.p, off.data(), bytes, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(dX.p, b->xOff.data(), bytes, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(dY.p, b->yOff.data(), bytes, cudaMemcpyHostToDevice, st));
     return CPB_OK;
@@ -2073,7 +2083,7 @@ extern "C" int cpb_batch_reweight_pairs(cpb_batch *b, double gapGamma) {
     cudaStream_t st = b->ctx->stream;
     DevBuf dOff, dX, dY, gX, gY;
     for (DevBuf *d : { &dOff, &dX, &dY, &gX, &gY }) d->pool = &b->ctx->pool;
-    int rc = upload_pair_tables(b, 0, dOff, dX, dY);
+    int rc = upload_pair_tables(b, b->pairOff[0], dOff, dX, dY);
     const int64_t lenX = b->xOff[b->n], lenY = b->yOff[b->n];
     if (rc == CPB_OK) rc = gX.reserve(std::max<int64_t>(lenX, 1) * sizeof(long long));
     if (rc == CPB_OK) rc = gY.reserve(std::max<int64_t>(lenY, 1) * sizeof(long long));
@@ -2112,7 +2122,7 @@ extern "C" int cpb_batch_alignment_scores(cpb_batch *b, int64_t *scores) {
     cudaStream_t st = b->ctx->stream;
     DevBuf dOff, dX, dY, dS;
     for (DevBuf *d : { &dOff, &dX, &dY, &dS }) d->pool = &b->ctx->pool;
-    int rc = upload_pair_tables(b, 0, dOff, dX, dY);
+    int rc = upload_pair_tables(b, b->pairOff[0], dOff, dX, dY);
     if (rc == CPB_OK) rc = dS.reserve((size_t) b->n * sizeof(int64_t));
     if (rc == CPB_OK) {
         k_alignment_scores<<<(unsigned) ((b->n * 32 + 255) / 256), 256, 0, st>>>(b->out[0].as<int32_t>(), dOff.as<int64_t>(), (int) b->n, dX.as<int64_t>(),
@@ -2127,6 +2137,317 @@ extern "C" int cpb_batch_alignment_scores(cpb_batch *b, int64_t *scores) {
     }
     for (DevBuf *d : { &dOff, &dX, &dY, &dS }) d->release();
     return rc;
+}
+
+/* ------------------------------------------------------------------------------------------------
+ * decoders on the device (decode_kernels.cuh): one alignment per pair from the lists of the last run, into the batch's alignment list.
+ * The host functions of host/realign.c are the definition; libcpecan.so and cPecanRealign still decode on the host.
+ * ---------------------------------------------------------------------------------------------- */
+/* the pair descriptors of every pair (work offsets are filled in per chunk); false if a pair's list 0 is too long for the kernels' int32
+ * indices */
+static bool decode_pairs(const cpb_batch *b, bool withGaps, std::vector<DecodePair> &P) {
+    P.assign((size_t) b->n, DecodePair());
+    for (int64_t i = 0; i < b->n; i++) {
+        DecodePair &D = P[(size_t) i];
+        memset(&D, 0, sizeof(D));
+        const int64_t n0 = b->pairOff[0][i + 1] - b->pairOff[0][i];
+        if (n0 >= INT32_MAX) return false;
+        D.list0 = b->pairOff[0][i];
+        D.n0 = (int32_t) n0;
+        if (withGaps) {
+            D.gap1 = b->pairOff[1][i];
+            D.n1 = (int32_t) (b->pairOff[1][i + 1] - b->pairOff[1][i]);
+            D.gap2 = b->pairOff[2][i];
+            D.n2 = (int32_t) (b->pairOff[2][i + 1] - b->pairOff[2][i]);
+        }
+        D.seqX = b->xOff[i];
+        D.seqY = b->yOff[i];
+        D.lX = (int32_t) (b->xOff[i + 1] - b->xOff[i]);
+        D.lY = (int32_t) (b->yOff[i + 1] - b->yOff[i]);
+    }
+    return true;
+}
+
+/* Runs body(p0, p1, chunk) over chunks of pairs whose work arrays (workBytes(pair) each) and per-pair tables fit the scratch budget, and
+ * gathers the alignment list: body launches the chunk's kernels and leaves every pair's length in chunk.lens, or (count == false) writes
+ * the pairs' alignments at chunk.off (the chunk's n+1 offsets into b->aln) itself once the lengths are scanned -- decode_chunks scans
+ * chunk.lens and then calls emit(chunk).  A single pair that does not fit returns CPB_ERR_MEMORY. */
+struct DecodeChunk {
+    int64_t p0, p1;
+    int nC;
+    DecodePair *desc;
+    char *work;
+    int32_t *lens, *aux;
+    double *scores;
+    int64_t *off;
+};
+
+template <class WorkBytes, class Body, class Emit>
+static int decode_chunks(cpb_batch *b, const char *call, std::vector<DecodePair> &P, WorkBytes workBytes, Body body, Emit emit, double *scoresOut,
+                         int64_t minCap = 0) {
+    cpb_context *ctx = b->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = b->n;
+    int rc;
+    int64_t cap = 0; /* every alignment is strictly increasing in x and y */
+    for (int64_t i = 0; i < n; i++) cap += std::min(b->xOff[i + 1] - b->xOff[i], b->yOff[i + 1] - b->yOff[i]);
+    cap = std::max(cap, minCap);
+    DevBuf dOff;
+    dOff.pool = &ctx->pool;
+    if ((rc = b->aln.reserve((size_t) std::max<int64_t>(cap, 1) * 3 * sizeof(int32_t))) != CPB_OK || (rc = dOff.reserve((size_t) (n + 1) * sizeof(int64_t))) != CPB_OK)
+        return rc;
+    size_t budget = ctx->scratchBudget;
+    if (budget == 0) {
+        size_t freeB = 0, totalB = 0;
+        CUDA_TRY(cudaMemGetInfo(&freeB, &totalB));
+        budget = (size_t) ((double) (freeB + ctx->scratch.cap) * 0.70);
+    }
+    const size_t fixed = 16 * 256, perPair = sizeof(DecodePair) + 4 + 4 + 8 + 16;
+    int64_t running = 0;
+    if (n == 0) CUDA_TRY(cudaMemsetAsync(dOff.p, 0, sizeof(int64_t), st));
+    for (int64_t p0 = 0; p0 < n;) {
+        int64_t p1 = p0, W = 0;
+        size_t bytes = fixed;
+        while (p1 < n) {
+            DecodePair &D = P[(size_t) p1];
+            const size_t need = (size_t) workBytes(D) + perPair;
+            if (fixed + need > budget) {
+                cpb_set_error("%s: pair %lld (%d x %d, %d pairs in list 0) needs %zu bytes of scratch, more than the budget of %zu", call, (long long) p1, D.lX,
+                              D.lY, D.n0, fixed + need, budget);
+                return CPB_ERR_MEMORY;
+            }
+            if (bytes + need > budget || p1 - p0 >= (1 << 24)) break;
+            bytes += need;
+            D.work = W;
+            W += (int64_t) workBytes(D);
+            p1++;
+        }
+        DecodeChunk c;
+        c.p0 = p0;
+        c.p1 = p1;
+        c.nC = (int) (p1 - p0);
+        size_t at = 0;
+        auto carve = [&](size_t nb) {
+            const size_t here = at;
+            at += (nb + 255) & ~(size_t) 255;
+            return here;
+        };
+        const size_t oDesc = carve(c.nC * sizeof(DecodePair)), oLens = carve(c.nC * 4), oAux = carve(c.nC * 4), oScores = carve(c.nC * 8),
+                     oTiles = carve(((c.nC + SCAN_TILE - 1) / SCAN_TILE + 1) * 8), oWork = carve((size_t) W);
+        if ((rc = ctx->scratch.reserve(std::max<size_t>(at, 256))) != CPB_OK) return rc;
+        char *s = ctx->scratch.as<char>();
+        c.desc = reinterpret_cast<DecodePair *>(s + oDesc);
+        c.lens = reinterpret_cast<int32_t *>(s + oLens);
+        c.aux = reinterpret_cast<int32_t *>(s + oAux);
+        c.scores = reinterpret_cast<double *>(s + oScores);
+        c.work = s + oWork;
+        c.off = dOff.as<int64_t>() + p0;
+        int64_t *dTiles = reinterpret_cast<int64_t *>(s + oTiles);
+        CUDA_TRY(cudaMemcpyAsync(c.desc, P.data() + p0, c.nC * sizeof(DecodePair), cudaMemcpyHostToDevice, st));
+        /* body and emit return the number of kernels they launched */
+        b->stats.kernelLaunches += body(c);
+        scan_counts(st, c.lens, c.nC, running, dTiles, c.off);
+        b->stats.kernelLaunches += 3;
+        b->stats.kernelLaunches += emit(c);
+        CUDA_TRY(cudaGetLastError());
+        if (scoresOut != nullptr) CUDA_TRY(cudaMemcpyAsync(scoresOut + p0, c.scores, c.nC * sizeof(double), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaMemcpyAsync(&running, c.off + c.nC, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(cudaStreamSynchronize(st)); /* the next chunk's scan starts from this total, and reuses the scratch */
+        p0 = p1;
+    }
+    b->alnOff.assign((size_t) n + 1, 0);
+    CUDA_TRY(cudaMemcpyAsync(b->alnOff.data(), dOff.p, (size_t) (n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    b->alnValid = true;
+    return CPB_OK;
+}
+
+extern "C" int cpb_batch_ordered_chain(cpb_batch *b, float matchGamma) {
+    if (b != nullptr) b->alnValid = false; /* a decode call replaces the list, also when it is refused */
+    if (b == nullptr || (b->lastMode != CPB_MODE_ALIGNED_PAIRS && b->lastMode != CPB_MODE_ALIGNED_PAIRS_INDELS)) {
+        cpb_set_error("cpb_batch_ordered_chain: no aligned-pair results in this batch");
+        return CPB_ERR_ARGUMENT;
+    }
+    if (!(matchGamma >= 0.0f && matchGamma <= 1.0f)) {
+        cpb_set_error("cpb_batch_ordered_chain: matchGamma must be in [0, 1] (a fraction of PAIR_ALIGNMENT_PROB_1), not %g", (double) matchGamma);
+        return CPB_ERR_ARGUMENT;
+    }
+    std::vector<DecodePair> P;
+    if (!decode_pairs(b, false, P)) {
+        cpb_set_error("cpb_batch_ordered_chain: a pair has 2^31 or more aligned pairs");
+        return CPB_ERR_ARGUMENT;
+    }
+    CUDA_TRY(cudaSetDevice(b->ctx->device));
+    cudaStream_t st = b->ctx->stream;
+    const int32_t *list0 = b->out[0].as<int32_t>();
+    return decode_chunks(
+        b, "cpb_batch_ordered_chain", P, [](const DecodePair &D) { return chain_work_bytes(D.n0, D.lX, D.lY); },
+        [&](DecodeChunk &c) {
+            k_chain_sort<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, list0, c.work, (double) matchGamma);
+            k_chain_sweep<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, c.work, c.lens, c.aux);
+            return 2;
+        },
+        [&](DecodeChunk &c) {
+            k_chain_write<<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, c.work, c.lens, c.aux, c.off, b->aln.as<int32_t>());
+            return 1;
+        },
+        nullptr);
+}
+
+/* The run's region and block tables, which put list 0 into the reference's order (what cpb_batch_fetch_pairs_reference_order does on the
+ * host), on the device; every pair's range of regions into P. */
+struct RefOrderTables {
+    DevBuf tab;
+    int64_t *shift = nullptr, *block0 = nullptr;
+    int32_t *blocks = nullptr, *from = nullptr;
+};
+
+static int ref_order_tables(cpb_batch *b, std::vector<DecodePair> &P, RefOrderTables &T) {
+    cudaStream_t st = b->ctx->stream;
+    const int64_t nR = (int64_t) b->hRegions.size();
+    std::vector<int64_t> regShift((size_t) std::max<int64_t>(nR, 1)), regBlock0((size_t) std::max<int64_t>(nR, 1));
+    std::vector<int32_t> regBlocks((size_t) std::max<int64_t>(nR, 1)), blockFrom;
+    int64_t nB = 0;
+    for (int64_t r = 0; r < nR; r++) {
+        const RegionDev &R = b->hRegions[(size_t) r];
+        regShift[(size_t) r] = (int64_t) R.ox + R.oy - 2;
+        regBlock0[(size_t) r] = nB;
+        regBlocks[(size_t) r] = R.nBlocks;
+        nB += R.nBlocks;
+    }
+    blockFrom.resize((size_t) std::max<int64_t>(nB, 1));
+    for (int64_t k = 0; k < nB; k++) blockFrom[(size_t) k] = b->hBlocks[(size_t) k].from;
+    for (int64_t r = nR; r-- > 0;) {
+        DecodePair &D = P[(size_t) b->hRegions[(size_t) r].pair];
+        if (D.region1 == 0) D.region1 = r + 1;
+        D.region0 = r;
+    }
+    T.tab.pool = &b->ctx->pool;
+    const size_t nRs = (size_t) std::max<int64_t>(nR, 1);
+    const int rc = T.tab.reserve(nRs * 20 + blockFrom.size() * 4 + 64);
+    if (rc != CPB_OK) return rc;
+    T.shift = T.tab.as<int64_t>();
+    T.block0 = T.shift + nRs;
+    T.blocks = reinterpret_cast<int32_t *>(T.block0 + nRs);
+    T.from = T.blocks + nRs;
+    CUDA_TRY(cudaMemcpyAsync(T.shift, regShift.data(), nRs * 8, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(T.block0, regBlock0.data(), nRs * 8, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(T.blocks, regBlocks.data(), nRs * 4, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(T.from, blockFrom.data(), blockFrom.size() * 4, cudaMemcpyHostToDevice, st));
+    return CPB_OK;
+}
+
+extern "C" int cpb_batch_mea(cpb_batch *b, float gapGamma, int leftShift, double *scores) {
+    if (b != nullptr) b->alnValid = false; /* a decode call replaces the list, also when it is refused */
+    if (b == nullptr || b->lastMode != CPB_MODE_ALIGNED_PAIRS_INDELS) {
+        cpb_set_error("cpb_batch_mea: needs the gap lists of an ALIGNED_PAIRS_INDELS run");
+        return CPB_ERR_ARGUMENT;
+    }
+    if (!(gapGamma >= 0.0f && gapGamma <= FLT_MAX)) {
+        cpb_set_error("cpb_batch_mea: gapGamma must be finite and >= 0, not %g", (double) gapGamma);
+        return CPB_ERR_ARGUMENT;
+    }
+    std::vector<DecodePair> P;
+    if (!decode_pairs(b, true, P)) {
+        cpb_set_error("cpb_batch_mea: a pair has 2^31 or more aligned pairs");
+        return CPB_ERR_ARGUMENT;
+    }
+    CUDA_TRY(cudaSetDevice(b->ctx->device));
+    cudaStream_t st = b->ctx->stream;
+    RefOrderTables T;
+    int rc = ref_order_tables(b, P, T);
+    if (rc != CPB_OK) return rc;
+    const int32_t *l0 = b->out[0].as<int32_t>(), *l1 = b->out[1].as<int32_t>(), *l2 = b->out[2].as<int32_t>();
+    const uint8_t *kx = b->keptX.as<uint8_t>(), *ky = b->keptY.as<uint8_t>();
+    return decode_chunks(
+        b, "cpb_batch_mea", P, [](const DecodePair &D) { return mea_work_bytes(D.n0, D.lX, D.lY); },
+        [&](DecodeChunk &c) {
+            k_ref_order<<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, l0, T.shift, T.block0, T.blocks, T.from, c.work);
+            k_mea_gaps<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, l1, l2, c.work);
+            k_mea<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, c.work, gapGamma, c.scores, c.lens);
+            if (leftShift) k_decode_emit<true><<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, c.work, kx, ky, c.lens, nullptr, nullptr);
+            return leftShift ? 4 : 3;
+        },
+        [&](DecodeChunk &c) {
+            if (leftShift) k_decode_emit<true><<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, c.work, kx, ky, c.lens, c.off, b->aln.as<int32_t>());
+            else k_decode_emit<false><<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, c.work, kx, ky, c.lens, c.off, b->aln.as<int32_t>());
+            return 1;
+        },
+        scores);
+}
+
+/* Test support, not part of the ABI header: the alignment list becomes list 0 of the last run in the reference's order as cpb_batch_mea
+ * builds it on the device (k_ref_order), so that this permutation can be compared with cpb_batch_fetch_pairs_reference_order. */
+extern "C" int cpb_debug_reference_order(cpb_batch *b) {
+    if (b != nullptr) b->alnValid = false;
+    if (b == nullptr || (b->lastMode != CPB_MODE_ALIGNED_PAIRS && b->lastMode != CPB_MODE_ALIGNED_PAIRS_INDELS)) {
+        cpb_set_error("cpb_debug_reference_order: no aligned-pair results in this batch");
+        return CPB_ERR_ARGUMENT;
+    }
+    std::vector<DecodePair> P;
+    if (!decode_pairs(b, false, P)) {
+        cpb_set_error("cpb_debug_reference_order: a pair has 2^31 or more aligned pairs");
+        return CPB_ERR_ARGUMENT;
+    }
+    CUDA_TRY(cudaSetDevice(b->ctx->device));
+    cudaStream_t st = b->ctx->stream;
+    RefOrderTables T;
+    int rc = ref_order_tables(b, P, T);
+    if (rc != CPB_OK) return rc;
+    const int32_t *l0 = b->out[0].as<int32_t>();
+    return decode_chunks(
+        b, "cpb_debug_reference_order", P, [](const DecodePair &D) { return mea_work_bytes(D.n0, D.lX, D.lY); },
+        [&](DecodeChunk &c) {
+            k_ref_order<<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, l0, T.shift, T.block0, T.blocks, T.from, c.work);
+            k_ref_emit<<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, c.work, c.lens, nullptr, nullptr);
+            return 2;
+        },
+        [&](DecodeChunk &c) {
+            k_ref_emit<<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, c.work, c.lens, c.off, b->aln.as<int32_t>());
+            return 1;
+        },
+        nullptr, b->outCount[0]);
+}
+
+extern "C" int64_t cpb_batch_alignments_count(const cpb_batch *b) { return b != nullptr && b->alnValid ? b->alnOff[(size_t) b->n] : 0; }
+
+extern "C" int cpb_batch_fetch_alignments(const cpb_batch *b, int64_t *offsets, int32_t *triples) {
+    if (b == nullptr || !b->alnValid || offsets == nullptr || (triples == nullptr && b->alnOff[(size_t) b->n] > 0)) {
+        cpb_set_error("cpb_batch_fetch_alignments: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain or cpb_batch_mea after the run"
+                                                                                     : "bad argument");
+        return CPB_ERR_ARGUMENT;
+    }
+    CUDA_TRY(cudaSetDevice(b->ctx->device));
+    memcpy(offsets, b->alnOff.data(), (size_t) (b->n + 1) * sizeof(int64_t));
+    const int64_t count = b->alnOff[(size_t) b->n];
+    if (count > 0) {
+        CUDA_TRY(cudaMemcpyAsync(triples, b->aln.p, (size_t) count * 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, b->ctx->stream));
+        CUDA_TRY(cudaStreamSynchronize(b->ctx->stream));
+    }
+    return CPB_OK;
+}
+
+extern "C" int cpb_batch_score_alignments(cpb_batch *b, int kind, double *scores) {
+    if (b == nullptr || !b->alnValid || kind < CPB_SCORE_IDENTITY || kind > CPB_SCORE_POSTERIOR_IGNORING_GAPS || (scores == nullptr && b->n > 0)) {
+        cpb_set_error("cpb_batch_score_alignments: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain or cpb_batch_mea after the run"
+                                                                                     : "bad argument (kind is one of CPB_SCORE_*)");
+        return CPB_ERR_ARGUMENT;
+    }
+    if (b->n == 0) return CPB_OK;
+    CUDA_TRY(cudaSetDevice(b->ctx->device));
+    cudaStream_t st = b->ctx->stream;
+    DevBuf dOff, dX, dY, dS;
+    for (DevBuf *d : { &dOff, &dX, &dY, &dS }) d->pool = &b->ctx->pool;
+    int rc = upload_pair_tables(b, b->alnOff, dOff, dX, dY);
+    if (rc != CPB_OK || (rc = dS.reserve((size_t) b->n * sizeof(double))) != CPB_OK) return rc;
+    k_decode_scores<<<grid_of(b->n * 32, 256), 256, 0, st>>>(b->aln.as<int32_t>(), dOff.as<int64_t>(), (int) b->n, dX.as<int64_t>(), dY.as<int64_t>(),
+                                                            b->keptX.as<uint8_t>(), b->keptY.as<uint8_t>(), kind, dS.as<double>());
+    b->stats.kernelLaunches++;
+    CUDA_TRY(cudaMemcpyAsync(scores, dS.p, (size_t) b->n * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    return CPB_OK;
 }
 
 extern "C" int cpb_batch_fetch_expectations(cpb_batch *b, double *perPair, double *total) {

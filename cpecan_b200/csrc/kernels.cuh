@@ -938,12 +938,15 @@ __global__ void __launch_bounds__(256) k_reduce_total(const double *perPair, int
 }
 
 /* ---------------------------------------------------------------------------------------------
- * k_encode : chars -> symbols a,c,g,t,n = 0..4 (symbol_convertCharToSymbol, impl/pairwiseAligner.c:317-334)
+ * k_encode : chars -> symbols a,c,g,t,n = 0..4 (symbol_convertCharToSymbol, impl/pairwiseAligner.c:317-334), in place; the bytes
+ * themselves, upper-cased as C's toupper does (only a-z change), go to `kept` for the decoders (left shift and identity compare bytes)
  * ------------------------------------------------------------------------------------------- */
-__global__ void k_encode(uint8_t *s, int64_t n) {
+__global__ void k_encode(uint8_t *s, uint8_t *kept, int64_t n) {
     const int64_t i = (int64_t) blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const uint8_t c = s[i] & 0xDF; /* fold case */
+    const uint8_t raw = s[i];
+    kept[i] = raw >= 'a' && raw <= 'z' ? (uint8_t) (raw - ('a' - 'A')) : raw;
+    const uint8_t c = raw & 0xDF; /* fold case */
     s[i] = c == 'A' ? 0 : (c == 'C' ? 1 : (c == 'G' ? 2 : (c == 'T' ? 3 : 4)));
 }
 

@@ -185,6 +185,35 @@ int cpb_batch_fetch_pairs_reference_order(cpb_batch *b, int list, int64_t *offse
  * cpb_batch_alignment_scores: per pair, getAlignmentScore of impl/multipleAligner.c:604-619 (n int64 values to the host). */
 int cpb_batch_reweight_pairs(cpb_batch *b, double gapGamma);
 int cpb_batch_alignment_scores(cpb_batch *b, int64_t *scores);
+/*
+ * Decoders: one alignment per pair from the lists of the last run, on the device, into the batch's alignment list -- n+1 offsets and
+ * int32 (pInt, x, y) triples, 0-based, like the result lists; per pair the pairs of the alignment, x and y strictly increasing.  Each
+ * returns, at tolerance 0 (same triples, same order, same double bits), what the host function of libcpecan.so (host/realign.c) returns on
+ * the lists libcpecan.so would hand it.  Each decode call replaces the alignment list; cpb_batch_run clears it; cpb_batch_reweight_pairs
+ * does not touch it.  Work arrays are processed in chunks that fit the scratch budget; a single pair that does not fit returns
+ * CPB_ERR_MEMORY.  libcpecan.so and cPecanRealign still decode on the host.
+ *
+ * cpb_batch_ordered_chain: filterPairwiseAlignmentToMakePairsOrdered (impl/multipleAligner.c:945-972; realign.c:150-247) of list 0 as it
+ *   stands (reweighted if cpb_batch_reweight_pairs was called, as cPecanRealign does): the heaviest chain, strictly increasing in x and y,
+ *   of the pairs with weight / PAIR_ALIGNMENT_PROB_1 >= matchGamma and > 0.  matchGamma in [0, 1].  Needs an ALIGNED_PAIRS or
+ *   ALIGNED_PAIRS_INDELS run.
+ * cpb_batch_mea: getMaximalExpectedAccuracyPairwiseAlignment (impl/pairwiseAligner.c:1603-1724; realign.c:249-326) of list 0 in the order
+ *   cpb_batch_fetch_pairs_reference_order gives, with lists 1 and 2 as the gap weights and gapGamma >= 0 as p->gapGamma; with leftShift
+ *   set, followed by leftShiftAlignment (:1726-1767; realign.c:330-356), which is getShiftedMEAAlignment (:1769-1792).  scores (n doubles,
+ *   or NULL) receives every pair's alignmentScore.  Needs an ALIGNED_PAIRS_INDELS run.
+ * cpb_batch_score_alignments: per pair, scoreByIdentity, scoreByIdentityIgnoringGaps, scoreByPosteriorProbability or
+ *   scoreByPosteriorProbabilityIgnoringGaps (impl/pairwiseAligner.c:1562-1597; realign.c:113-148) of its alignment; the two "ignoring
+ *   gaps" forms are NaN for an empty alignment, as on the host.  Letters compare case-blind, N never matches.
+ * Fetching or scoring before a decode call, a decode after an EXPECTATIONS or FORWARD run, and gammas or kind out of range return
+ * CPB_ERR_ARGUMENT.  A decode call that returns an error, for whatever reason, leaves no alignment list (the previous one is gone too).
+ * cpb_batch_alignments_count is 0 while there is no alignment list.
+ */
+enum { CPB_SCORE_IDENTITY = 0, CPB_SCORE_IDENTITY_IGNORING_GAPS = 1, CPB_SCORE_POSTERIOR = 2, CPB_SCORE_POSTERIOR_IGNORING_GAPS = 3 };
+int cpb_batch_ordered_chain(cpb_batch *b, float matchGamma);
+int cpb_batch_mea(cpb_batch *b, float gapGamma, int leftShift, double *scores);
+int64_t cpb_batch_alignments_count(const cpb_batch *b);
+int cpb_batch_fetch_alignments(const cpb_batch *b, int64_t *offsets, int32_t *triples);
+int cpb_batch_score_alignments(cpb_batch *b, int kind, double *scores);
 /* device pointers of the same (valid until the next run / destroy) */
 const int32_t *cpb_batch_device_triples(const cpb_batch *b, int list);
 /* EXPECTATIONS mode: perPair (may be NULL) receives n * CPB_HMM_LEN(S) doubles, total receives CPB_HMM_LEN(S) doubles
