@@ -136,6 +136,7 @@ def _load():
     L.cpb_batch_alignments_count.argtypes = [C.c_void_p]
     L.cpb_batch_fetch_alignments.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.cpb_batch_score_alignments.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+    L.cpb_batch_anchors_from_alignments.argtypes = [C.c_void_p, P(CpbParams)]
     L.cpb_batch_device_triples.restype = C.c_void_p
     L.cpb_batch_device_triples.argtypes = [C.c_void_p, C.c_int]
     L.cpb_batch_fetch_expectations.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
@@ -394,6 +395,11 @@ class Batch:
         _check(lib.cpb_batch_score_alignments(self.h, int(kind), C.c_void_p(out.ctypes.data)))
         return out[: self.n]
 
+    def anchors_from_alignments(self, params):
+        """replaces every pair's anchors with those its alignment gives (params.constraintDiagonalTrim, params.diagonalExpansion): the
+        anchors cPecanRealign's job_prepare builds from the cigar of that alignment; the next run plans anew with them"""
+        _check(lib.cpb_batch_anchors_from_alignments(self.h, C.byref(params) if params is not None else None))
+
     def fetch_expectations(self, per_pair=True):
         L = hmm_len(self.S)
         pp = np.zeros((self.n, L), dtype=np.float64) if per_pair else None
@@ -412,7 +418,10 @@ class Batch:
 
     def close(self):
         if self.h:
-            lib.cpb_batch_destroy(self.h)
+            # cpb_batch_destroy reads the batch's context (device, buffer pools): after the context is closed it must not run; the batch's
+            # device memory then goes back with the process
+            if self.ctx.h:
+                lib.cpb_batch_destroy(self.h)
             self.h = None
 
     def __del__(self):

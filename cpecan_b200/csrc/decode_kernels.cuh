@@ -8,6 +8,8 @@
  *   k_mea_gaps / k_mea                             getMaximalExpectedAccuracyPairwiseAlignment realign.c:249-326
  *   k_decode_emit<SHIFT>                           its traceback, and leftShiftAlignment        realign.c:313-318, :330-356
  *   k_decode_scores                                scoreByIdentity ... IgnoringGaps             realign.c:113-148
+ *   k_reanchor_count / k_reanchor_write            the anchors job_prepare builds from the cigar of an alignment (realignJobs.h:149-173,
+ *                                                  realign.c:32-72, cPecanRealign.c:98-123)
  *
  * Pairs are processed in chunks whose work arrays fit the context's scratch budget (engine.cu); DecodePair says where a pair's inputs
  * and work arrays are.  Alignments are int32 (pInt, x, y) triples, 0-based, like the result lists.
@@ -509,6 +511,76 @@ __global__ void k_decode_scores(const int32_t *aln, const int64_t *off, int nPai
         break;
     }
     scores[pair] = s;
+}
+
+/* ---- anchors from the alignment list (cpb_batch_anchors_from_alignments) ----
+ * The anchors job_prepare (host/realignJobs.h) builds from the cigar cPecanRealign writes for an alignment (pairs_to_alignment): the cigar's
+ * match operations are the alignment's maximal diagonal runs (each next pair at (x + 1, y + 1)); convertPairwiseForwardStrandAlignmentToAnchorPairs
+ * (realign.c:32-72) takes the columns at positions l in [trim, L - trim) of a run of length L, i.e. those with at least trim pairs of their
+ * run before and after them; columns_match keeps those whose two bytes are equal and not N.  DecodePair.list0 / n0 say where a pair's
+ * alignment is.  Work array of a pair of m triples: per triple the number of its run's triples before it, then its keep flag. */
+__host__ __device__ __forceinline__ int64_t reanchor_work_bytes(int64_t m) { return dec_round(4 * m); }
+
+/* One warp per pair, O(1) per triple: a forward sweep finds every triple's run start (the last start at or before it: the chunk's ballot,
+ * or the run carried in from the chunks before), a backward sweep its run end likewise; lens[pi] receives the number of kept columns. */
+__global__ void k_reanchor_count(const DecodePair *P, int nP, const int32_t *aln, const uint8_t *X, const uint8_t *Y, char *scratch, int32_t trim,
+                                 int32_t *lens) {
+    const int pi = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (pi >= nP) return;
+    const DecodePair D = P[pi];
+    const int32_t *t = aln + 3 * D.list0;
+    int32_t *w = reinterpret_cast<int32_t *>(scratch + D.work);
+    const int m = D.n0;
+    auto diagonal = [&](int k) { return t[3 * k + 1] == t[3 * k - 2] + 1 && t[3 * k + 2] == t[3 * k - 1] + 1; }; /* triple k follows k - 1 */
+    int carry = 0;
+    for (int k0 = 0; k0 < m; k0 += 32) {
+        const int k = k0 + lane;
+        const unsigned starts = __ballot_sync(0xFFFFFFFFu, k < m && (k == 0 || !diagonal(k)));
+        const unsigned upTo = starts & (0xFFFFFFFFu >> (31 - lane));
+        if (k < m) w[k] = k - (upTo != 0 ? k0 + 31 - __clz(upTo) : carry);
+        if (starts != 0) carry = k0 + 31 - __clz(starts);
+    }
+    __syncwarp();
+    const uint8_t *sx = X + D.seqX, *sy = Y + D.seqY;
+    int kept = 0;
+    carry = m - 1;
+    for (int k0 = (m - 1) & ~31; k0 >= 0; k0 -= 32) {
+        const int k = k0 + lane;
+        const unsigned ends = __ballot_sync(0xFFFFFFFFu, k < m && (k == m - 1 || !diagonal(k + 1)));
+        const unsigned from = ends & (0xFFFFFFFFu << lane);
+        bool keep = false;
+        if (k < m) {
+            const int end = from != 0 ? k0 + __ffs(from) - 1 : carry;
+            const uint8_t cx = sx[t[3 * k + 1]], cy = sy[t[3 * k + 2]];
+            keep = w[k] >= trim && end - k >= trim && cx == cy && cx != 'N';
+            w[k] = keep;
+        }
+        kept += __popc(__ballot_sync(0xFFFFFFFFu, keep));
+        if (ends != 0) carry = k0 + __ffs(ends) - 1;
+    }
+    if (lane == 0) lens[pi] = kept;
+}
+
+/* One warp per pair, after the scan of lens: the kept columns as (x, y, expansion) at out[off[pi]...], x ascending */
+__global__ void k_reanchor_write(const DecodePair *P, int nP, const int32_t *aln, const char *scratch, int32_t expansion, const int64_t *off, int32_t *out) {
+    const int pi = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (pi >= nP) return;
+    const DecodePair D = P[pi];
+    const int32_t *t = aln + 3 * D.list0;
+    const int32_t *w = reinterpret_cast<const int32_t *>(scratch + D.work);
+    int64_t at = off[pi];
+    for (int k0 = 0; k0 < D.n0; k0 += 32) {
+        const int k = k0 + lane;
+        const bool keep = k < D.n0 && w[k] != 0;
+        const unsigned keeps = __ballot_sync(0xFFFFFFFFu, keep);
+        if (keep) {
+            const int64_t o = at + __popc(keeps & ((1u << lane) - 1));
+            out[3 * o] = t[3 * k + 1];
+            out[3 * o + 1] = t[3 * k + 2];
+            out[3 * o + 2] = expansion;
+        }
+        at += __popc(keeps);
+    }
 }
 
 } // namespace cpb

@@ -2168,10 +2168,10 @@ static bool decode_pairs(const cpb_batch *b, bool withGaps, std::vector<DecodePa
     return true;
 }
 
-/* Runs body(p0, p1, chunk) over chunks of pairs whose work arrays (workBytes(pair) each) and per-pair tables fit the scratch budget, and
- * gathers the alignment list: body launches the chunk's kernels and leaves every pair's length in chunk.lens, or (count == false) writes
- * the pairs' alignments at chunk.off (the chunk's n+1 offsets into b->aln) itself once the lengths are scanned -- decode_chunks scans
- * chunk.lens and then calls emit(chunk).  A single pair that does not fit returns CPB_ERR_MEMORY. */
+/* Runs body(chunk) over chunks of pairs whose work arrays (workBytes(pair) each) and per-pair tables fit the scratch budget, and gathers
+ * a per-pair list of triples: body launches the chunk's kernels and leaves every pair's length in chunk.lens; pair_chunks scans them into
+ * chunk.off (the chunk's part of dOff, the n+1 device offsets of the list) and then calls emit(chunk), which writes the pairs' triples at
+ * those offsets.  hostOff receives the offsets.  A single pair that does not fit returns CPB_ERR_MEMORY. */
 struct DecodeChunk {
     int64_t p0, p1;
     int nC;
@@ -2183,19 +2183,12 @@ struct DecodeChunk {
 };
 
 template <class WorkBytes, class Body, class Emit>
-static int decode_chunks(cpb_batch *b, const char *call, std::vector<DecodePair> &P, WorkBytes workBytes, Body body, Emit emit, double *scoresOut,
-                         int64_t minCap = 0) {
+static int pair_chunks(cpb_batch *b, const char *call, std::vector<DecodePair> &P, WorkBytes workBytes, Body body, Emit emit, double *scoresOut,
+                       int64_t *dOff, std::vector<int64_t> &hostOff) {
     cpb_context *ctx = b->ctx;
     cudaStream_t st = ctx->stream;
     const int64_t n = b->n;
     int rc;
-    int64_t cap = 0; /* every alignment is strictly increasing in x and y */
-    for (int64_t i = 0; i < n; i++) cap += std::min(b->xOff[i + 1] - b->xOff[i], b->yOff[i + 1] - b->yOff[i]);
-    cap = std::max(cap, minCap);
-    DevBuf dOff;
-    dOff.pool = &ctx->pool;
-    if ((rc = b->aln.reserve((size_t) std::max<int64_t>(cap, 1) * 3 * sizeof(int32_t))) != CPB_OK || (rc = dOff.reserve((size_t) (n + 1) * sizeof(int64_t))) != CPB_OK)
-        return rc;
     size_t budget = ctx->scratchBudget;
     if (budget == 0) {
         size_t freeB = 0, totalB = 0;
@@ -2204,7 +2197,7 @@ static int decode_chunks(cpb_batch *b, const char *call, std::vector<DecodePair>
     }
     const size_t fixed = 16 * 256, perPair = sizeof(DecodePair) + 4 + 4 + 8 + 16;
     int64_t running = 0;
-    if (n == 0) CUDA_TRY(cudaMemsetAsync(dOff.p, 0, sizeof(int64_t), st));
+    if (n == 0) CUDA_TRY(cudaMemsetAsync(dOff, 0, sizeof(int64_t), st));
     for (int64_t p0 = 0; p0 < n;) {
         int64_t p1 = p0, W = 0;
         size_t bytes = fixed;
@@ -2241,7 +2234,7 @@ static int decode_chunks(cpb_batch *b, const char *call, std::vector<DecodePair>
         c.aux = reinterpret_cast<int32_t *>(s + oAux);
         c.scores = reinterpret_cast<double *>(s + oScores);
         c.work = s + oWork;
-        c.off = dOff.as<int64_t>() + p0;
+        c.off = dOff + p0;
         int64_t *dTiles = reinterpret_cast<int64_t *>(s + oTiles);
         CUDA_TRY(cudaMemcpyAsync(c.desc, P.data() + p0, c.nC * sizeof(DecodePair), cudaMemcpyHostToDevice, st));
         /* body and emit return the number of kernels they launched */
@@ -2255,10 +2248,27 @@ static int decode_chunks(cpb_batch *b, const char *call, std::vector<DecodePair>
         CUDA_TRY(cudaStreamSynchronize(st)); /* the next chunk's scan starts from this total, and reuses the scratch */
         p0 = p1;
     }
-    b->alnOff.assign((size_t) n + 1, 0);
-    CUDA_TRY(cudaMemcpyAsync(b->alnOff.data(), dOff.p, (size_t) (n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    hostOff.assign((size_t) n + 1, 0);
+    CUDA_TRY(cudaMemcpyAsync(hostOff.data(), dOff, (size_t) (n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
+    return CPB_OK;
+}
+
+/* pair_chunks into the batch's alignment list */
+template <class WorkBytes, class Body, class Emit>
+static int decode_chunks(cpb_batch *b, const char *call, std::vector<DecodePair> &P, WorkBytes workBytes, Body body, Emit emit, double *scoresOut,
+                         int64_t minCap = 0) {
+    const int64_t n = b->n;
+    int rc;
+    int64_t cap = 0; /* every alignment is strictly increasing in x and y */
+    for (int64_t i = 0; i < n; i++) cap += std::min(b->xOff[i + 1] - b->xOff[i], b->yOff[i + 1] - b->yOff[i]);
+    cap = std::max(cap, minCap);
+    DevBuf dOff;
+    dOff.pool = &b->ctx->pool;
+    if ((rc = b->aln.reserve((size_t) std::max<int64_t>(cap, 1) * 3 * sizeof(int32_t))) != CPB_OK || (rc = dOff.reserve((size_t) (n + 1) * sizeof(int64_t))) != CPB_OK)
+        return rc;
+    if ((rc = pair_chunks(b, call, P, workBytes, body, emit, scoresOut, dOff.as<int64_t>(), b->alnOff)) != CPB_OK) return rc;
     b->alnValid = true;
     return CPB_OK;
 }
@@ -2447,6 +2457,95 @@ extern "C" int cpb_batch_score_alignments(cpb_batch *b, int kind, double *scores
     CUDA_TRY(cudaMemcpyAsync(scores, dS.p, (size_t) b->n * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
+    return CPB_OK;
+}
+
+/* The anchors job_prepare builds from the cigar of every pair's alignment (k_reanchor_count / k_reanchor_write), built into new buffers --
+ * device triples, the device pair table, the page-locked host copy that build_regions reads -- which replace the batch's only once all of
+ * them are there.  Only planning reads the anchors (k_split_flags, build_regions, k_band), so the lists, the alignment list and everything
+ * else of the last run stay as they are; the kept plan goes. */
+extern "C" int cpb_batch_anchors_from_alignments(cpb_batch *b, const CpbParams *p) {
+    if (b == nullptr || p == nullptr || p->constraintDiagonalTrim < 0 || p->constraintDiagonalTrim > 0x7FFFFFFF || p->diagonalExpansion < 0 ||
+        p->diagonalExpansion > 0x7FFFFFFF) {
+        cpb_set_error("cpb_batch_anchors_from_alignments: %s", b == nullptr ? "bad argument"
+                                                                            : (p == nullptr ? "no parameters" : "constraintDiagonalTrim and diagonalExpansion must be in [0, 2^31)"));
+        return CPB_ERR_ARGUMENT;
+    }
+    if (!b->alnValid) {
+        cpb_set_error("cpb_batch_anchors_from_alignments: no alignments: call cpb_batch_ordered_chain or cpb_batch_mea after the run");
+        return CPB_ERR_ARGUMENT;
+    }
+    const int64_t n = b->n;
+    std::vector<DecodePair> P((size_t) n);
+    for (int64_t i = 0; i < n; i++) {
+        DecodePair &D = P[(size_t) i];
+        memset(&D, 0, sizeof(D));
+        D.list0 = b->alnOff[(size_t) i];
+        D.n0 = (int32_t) (b->alnOff[(size_t) i + 1] - b->alnOff[(size_t) i]); /* at most min(lX, lY) */
+        D.seqX = b->xOff[(size_t) i];
+        D.seqY = b->yOff[(size_t) i];
+        D.lX = (int32_t) (b->xOff[(size_t) i + 1] - b->xOff[(size_t) i]);
+        D.lY = (int32_t) (b->yOff[(size_t) i + 1] - b->yOff[(size_t) i]);
+    }
+    cpb_context *ctx = b->ctx;
+    CUDA_TRY(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    DevBuf tri, tab; /* the new device triples; the new pair table (aOff, xOff, yOff), whose first n + 1 entries the chunks fill */
+    tri.pool = tab.pool = &ctx->pool;
+    const size_t tabBytes = (size_t) (n + 1) * sizeof(int64_t);
+    int rc;
+    if ((rc = tri.reserve((size_t) std::max<int64_t>(b->alnOff[(size_t) n], 1) * 3 * sizeof(int32_t))) != CPB_OK || (rc = tab.reserve(3 * tabBytes)) != CPB_OK)
+        return rc;
+    const int32_t *aln = b->aln.as<int32_t>();
+    const uint8_t *kx = b->keptX.as<uint8_t>(), *ky = b->keptY.as<uint8_t>();
+    const int32_t trim = (int32_t) p->constraintDiagonalTrim, expansion = (int32_t) p->diagonalExpansion;
+    std::vector<int64_t> aOff;
+    rc = pair_chunks(
+        b, "cpb_batch_anchors_from_alignments", P, [](const DecodePair &D) { return reanchor_work_bytes(D.n0); },
+        [&](DecodeChunk &c) {
+            k_reanchor_count<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, aln, kx, ky, c.work, trim, c.lens);
+            return 1;
+        },
+        [&](DecodeChunk &c) {
+            k_reanchor_write<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, aln, c.work, expansion, c.off, tri.as<int32_t>());
+            return 1;
+        },
+        nullptr, tab.as<int64_t>(), aOff);
+    if (rc != CPB_OK) return rc;
+    if (n > 0) CUDA_TRY(cudaMemcpyAsync(tab.as<char>() + tabBytes, b->dPairTab.as<char>() + tabBytes, 2 * tabBytes, cudaMemcpyDeviceToDevice, st));
+    const int64_t nA = aOff[(size_t) n];
+    const size_t bytes = (size_t) (3 * nA) * sizeof(int32_t);
+    int32_t *host = nA > 0 ? static_cast<int32_t *>(ctx->pinned.take(bytes)) : nullptr;
+    std::vector<int32_t> own;
+    if (nA > 0 && host == nullptr) {
+        own.resize((size_t) (3 * nA));
+        host = own.data();
+    }
+    cudaError_t e = nA > 0 ? cudaMemcpyAsync(host, tri.p, bytes, cudaMemcpyDeviceToHost, st) : cudaSuccess;
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        if (host != nullptr && own.empty()) ctx->pinned.give(host);
+        cpb_set_error("cpb_batch_anchors_from_alignments: %s", cudaGetErrorString(e));
+        return CPB_ERR_CUDA;
+    }
+    /* everything is built: swap */
+    if (b->anchors != nullptr && b->anchorsOwn.empty()) ctx->pinned.give(b->anchors);
+    b->anchors = host;
+    b->anchorsOwn.swap(own);
+    b->aOff.swap(aOff);
+    b->dAnchors.release();
+    b->dAnchors.adopt(tri);
+    if (n > 0) {
+        b->dPairTab.release();
+        b->dPairTab.adopt(tab);
+    }
+    b->oddExpansionPair = -1;
+    if (expansion & 1) {
+        for (int64_t i = 0; i < n && b->oddExpansionPair < 0; i++)
+            if (b->aOff[(size_t) i + 1] > b->aOff[(size_t) i]) b->oddExpansionPair = i;
+    }
+    b->planValid = false;
     return CPB_OK;
 }
 

@@ -10,7 +10,15 @@
  *     normalise -> [keep the old emissions unless --trainEmissions; --tieEmissions] -> next model.
  * Same options where they make sense in one process; the model file is written in cPecanEm.py's format (:31-35): line 1 type,
  * transitions, likelihood; line 2 emissions; line 3 the likelihood of every iteration.
- * Not carried over: --updateTheBand (re-anchoring between iterations), the XML summary and the LASTZ scoring-matrix export.
+ * --updateTheBand: after the maximisation step of every iteration but the last, every alignment is realigned under the model that step
+ * produced and re-anchored from the result, so that the next expectation pass runs in a band that follows the model rather than the
+ * input cigars.  The order is train, then re-anchor under the new model; the band is never derived from the untrained starting model
+ * (under all-equal or random values a realignment says nothing).  One update is what cPecanRealign --loadHmm <model>
+ * --diagonalExpansion 10 --splitMatrixBiggerThanThis 3000 --constraintDiagonalTrim t (matchGamma 0.85, its default) writes for the
+ * current alignments, read back by cPecanEm -- but under the model in full doubles rather than through the model file's 12 digits, and on
+ * the device (cpecanResidentBatch_updateAnchors): no list, alignment or cigar crosses to the host.  Every --randomStart trial starts from
+ * the input alignments' anchors.
+ * Not carried over: the XML summary and the LASTZ scoring-matrix export.
  * Several GPUs: tools/em_multi_gpu.py runs the same loop with one NCCL all-reduce of the expectation vector per iteration.
  */
 #include <getopt.h>
@@ -37,6 +45,8 @@ static void usage(void) {
     fprintf(stderr, "--maxAlignmentLengthToSample N : use at most N bases of alignment, sampled without replacement (default 50000000)\n");
     fprintf(stderr, "--seed N : seed of the random start and of the sampling (default: time)\n");
     fprintf(stderr, "--gpus N : spread the alignments over the first N GPUs; the expectations are summed with one NCCL all-reduce per iteration (default 1)\n");
+    fprintf(stderr, "--updateTheBand : after every iteration but the last, realign the alignments under the new model (as cPecanRealign, matchGamma 0.85)\n");
+    fprintf(stderr, "    and take the next iteration's anchors from the realigned alignments\n");
     fprintf(stderr, "--diagonalExpansion N, --constraintDiagonalTrim N, --splitMatrixBiggerThanThis N : band options, as cPecanRealign\n");
     fprintf(stderr, "    (defaults: cPecanEm.py's --optionsToRealign, diagonalExpansion 10 and splitMatrixBiggerThanThis 3000)\n");
 }
@@ -92,11 +102,14 @@ static void tie_emissions(Hmm *hmm) { /* cPecanEm.py:95-105 */
     }
 }
 
+/* the matchGamma of cPecanRealign's default realignment (cPecanRealign.c, o.matchGamma) with which --updateTheBand realigns */
+#define UPDATE_BAND_MATCH_GAMMA 0.85f
+
 typedef struct {
     const char *inputModel;
     StateMachineType type;
     int64_t iterations;
-    bool randomStart, useDefaultModelAsStart, trainEmissions, tieEmissions;
+    bool randomStart, useDefaultModelAsStart, trainEmissions, tieEmissions, updateTheBand;
     double jukesCantor; /* < 0: not set */
 } EmOptions;
 
@@ -136,9 +149,24 @@ static Hmm *expectation_maximisation(CpecanResidentBatch *batch, PairwiseAlignme
         hmm_destruct(hmm);
         hmm = expectations;
         write_model(hmm, outputModel, NULL, 0);
+        if (o->updateTheBand && it + 1 < o->iterations) { /* the next iteration's band, from the alignments under the model just trained */
+            sM = hmm_getStateMachine(hmm);
+            cpecanResidentBatch_updateAnchors(batch, sM, p, UPDATE_BAND_MATCH_GAMMA);
+            stateMachine_destruct(sM);
+            log_info("Updated the band under the model of iteration %" PRIi64 "\n", it);
+        }
     }
     write_model(hmm, outputModel, likelihoods, o->iterations);
     return hmm;
+}
+
+static void release_jobs(Job *jobs, int64_t n, const char **sX, const char **sY, stList **anchors, bool *ragged) {
+    for (int64_t i = 0; i < n; i++) job_release(&jobs[i]);
+    free(jobs);
+    free(sX);
+    free(sY);
+    free(anchors);
+    free(ragged);
 }
 
 int main(int argc, char *argv[]) {
@@ -175,6 +203,7 @@ int main(int argc, char *argv[]) {
                                            { "constraintDiagonalTrim", required_argument, 0, 't' },
                                            { "splitMatrixBiggerThanThis", required_argument, 0, 'o' },
                                            { "gpus", required_argument, 0, 'G' },
+                                           { "updateTheBand", no_argument, 0, 'U' },
                                            { 0, 0, 0, 0 } };
     for (;;) {
         int index = 0;
@@ -212,6 +241,7 @@ int main(int argc, char *argv[]) {
             cpecan_setDevices((int) gpus);
             break;
         }
+        case 'U': o.updateTheBand = true; break;
         default: usage(); return 1;
         }
     }
@@ -263,13 +293,8 @@ int main(int argc, char *argv[]) {
         ragged[i] = 1;
     }
     CpecanResidentBatch *batch = cpecanResidentBatch_construct(used, sX, sY, anchors, p, ragged, ragged);
-    for (int64_t i = 0; i < used; i++) job_release(&jobs[i]);
-    free(jobs);
-    free(sX);
-    free(sY);
-    free(anchors);
-    free(ragged);
-    free_sequences();
+    free_sequences(); /* the jobs hold their own sub-sequences */
+    if (!o.updateTheBand) release_jobs(jobs, used, sX, sY, anchors, ragged); /* else kept: every trial starts from the input alignments' anchors */
 
     double *likelihoods = xmalloc((size_t) (o.iterations + 1) * sizeof(double));
     if (o.inputModel != NULL || !o.randomStart) { /* one run (cPecanEm.py:218-219) */
@@ -283,6 +308,10 @@ int main(int argc, char *argv[]) {
         char *trialFile = xmalloc(strlen(outputModel) + 32);
         for (int64_t t = 0; t < trials; t++) {
             sprintf(trialFile, "%s_%" PRIi64, outputModel, t);
+            if (o.updateTheBand && t > 0) { /* the previous trial moved the band */
+                cpecanResidentBatch_destruct(batch);
+                batch = cpecanResidentBatch_construct(used, sX, sY, anchors, p, ragged, ragged);
+            }
             Hmm *hmm = expectation_maximisation(batch, p, &o, trialFile, likelihoods);
             if (!outputTrialHmms) remove(trialFile);
             if (best == NULL || hmm->likelihood > best->likelihood) {
@@ -303,6 +332,7 @@ int main(int argc, char *argv[]) {
     }
     free(likelihoods);
     cpecanResidentBatch_destruct(batch);
+    if (o.updateTheBand) release_jobs(jobs, used, sX, sY, anchors, ragged);
     pairwiseAlignmentBandingParameters_destruct(p);
     cpecan_shutdown();
     return 0;

@@ -695,27 +695,38 @@ typedef struct {
     cpb_batch *b;
     const CpbModel *model;
     const CpbParams *q;
+    int updateAnchors; /* 0: an expectation run; 1: realign and re-anchor (cpecanResidentBatch_updateAnchors) */
+    float matchGamma;
 } ResidentRun;
-static void *resident_run(void *v) {
-    ResidentRun *r = v;
-    const int rc = cpb_batch_run(r->b, r->model, r->q, CPB_MODE_EXPECTATIONS);
+static void resident_check(int rc) {
     if (rc == CPB_ERR_BAND) st_errAbort("%s: %s", PAIRWISE_ALIGNMENT_EXCEPTION_ID, cpb_last_error());
     if (rc != CPB_OK) st_errAbort("cpecan: %s", cpb_last_error());
+}
+static void *resident_run(void *v) {
+    ResidentRun *r = v;
+    if (!r->updateAnchors) {
+        resident_check(cpb_batch_run(r->b, r->model, r->q, CPB_MODE_EXPECTATIONS));
+        return NULL;
+    }
+    /* cPecanRealign's default steps for every alignment (job_finish: reweight, ordered chain), then the anchors job_prepare makes from the
+     * cigar it would write; no list leaves the device */
+    resident_check(cpb_batch_run(r->b, r->model, r->q, CPB_MODE_ALIGNED_PAIRS));
+    resident_check(cpb_batch_reweight_pairs(r->b, r->q->gapGamma));
+    resident_check(cpb_batch_ordered_chain(r->b, r->matchGamma));
+    resident_check(cpb_batch_anchors_from_alignments(r->b, r->q));
     return NULL;
 }
 
-void cpecanResidentBatch_getExpectations(CpecanResidentBatch *r, StateMachine *sM, Hmm *hmmExpectations, PairwiseAlignmentParameters *p) {
-    if (hmmExpectations->stateNumber != sM->stateNumber)
-        st_errAbort("getExpectations: the Hmm has %lld states, the state machine %lld", (long long) hmmExpectations->stateNumber,
-                    (long long) sM->stateNumber);
-    CpbParams q;
-    to_engine_params(p, &q);
+/* one host thread per device */
+static void resident_each(CpecanResidentBatch *r, StateMachine *sM, const CpbParams *q, int updateAnchors, float matchGamma) {
     ResidentRun runs[CPECAN_MAX_DEVICES];
     pthread_t ids[CPECAN_MAX_DEVICES];
     for (int d = 0; d < r->nDev; d++) {
         runs[d].b = r->b[d];
         runs[d].model = cpecan_model_of(sM);
-        runs[d].q = &q;
+        runs[d].q = q;
+        runs[d].updateAnchors = updateAnchors;
+        runs[d].matchGamma = matchGamma;
     }
     if (r->nDev == 1) {
         resident_run(&runs[0]);
@@ -724,7 +735,23 @@ void cpecanResidentBatch_getExpectations(CpecanResidentBatch *r, StateMachine *s
             if (pthread_create(&ids[d], NULL, resident_run, &runs[d]) != 0) st_errAbort("cpecan: cannot start a host thread");
         for (int d = 0; d < r->nDev; d++) pthread_join(ids[d], NULL);
     }
+}
+
+void cpecanResidentBatch_getExpectations(CpecanResidentBatch *r, StateMachine *sM, Hmm *hmmExpectations, PairwiseAlignmentParameters *p) {
+    if (hmmExpectations->stateNumber != sM->stateNumber)
+        st_errAbort("getExpectations: the Hmm has %lld states, the state machine %lld", (long long) hmmExpectations->stateNumber,
+                    (long long) sM->stateNumber);
+    CpbParams q;
+    to_engine_params(p, &q);
+    resident_each(r, sM, &q, 0, 0.0f);
     add_expectations(hmmExpectations, sM->stateNumber, r->b, r->nDev);
+}
+
+void cpecanResidentBatch_updateAnchors(CpecanResidentBatch *r, StateMachine *sM, PairwiseAlignmentParameters *p, float matchGamma) {
+    if (!(matchGamma >= 0.0f && matchGamma <= 1.0f)) st_errAbort("cpecanResidentBatch_updateAnchors: matchGamma must be in [0, 1], not %g", (double) matchGamma);
+    CpbParams q;
+    to_engine_params(p, &q);
+    resident_each(r, sM, &q, 1, matchGamma);
 }
 
 void computeForwardProbabilityBatch(StateMachine *sM, int64_t n, const char *const *sX, const char *const *sY, stList *const *anchorPairs,

@@ -239,6 +239,12 @@ CpecanResidentBatch *cpecanResidentBatch_construct(int64_t n, const char *const 
 void cpecanResidentBatch_destruct(CpecanResidentBatch *batch);
 /* += into hmmExpectations, as getExpectationsUsingAnchorsBatch */
 void cpecanResidentBatch_getExpectations(CpecanResidentBatch *batch, StateMachine *sM, Hmm *hmmExpectations, PairwiseAlignmentParameters *p);
+/* Re-anchors every alignment of the batch under sM, on every device (one host thread each), with no list leaving the device: an
+ * ALIGNED_PAIRS run with p, reweighting by p->gapGamma, the heaviest ordered chain at matchGamma, then the anchors of that chain as
+ * cPecanRealign's cigar would give them (p->constraintDiagonalTrim, p->diagonalExpansion; cpb_batch_anchors_from_alignments).  These are
+ * cPecanRealign's default steps; the next expectation pass runs in the new band.  An invalid band aborts with
+ * PAIRWISE_ALIGNMENT_EXCEPTION, any other engine error as cpecanResidentBatch_getExpectations does. */
+void cpecanResidentBatch_updateAnchors(CpecanResidentBatch *batch, StateMachine *sM, PairwiseAlignmentParameters *p, float matchGamma);
 
 #ifdef __cplusplus
 }

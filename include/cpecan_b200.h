@@ -214,6 +214,19 @@ int cpb_batch_mea(cpb_batch *b, float gapGamma, int leftShift, double *scores);
 int64_t cpb_batch_alignments_count(const cpb_batch *b);
 int cpb_batch_fetch_alignments(const cpb_batch *b, int64_t *offsets, int32_t *triples);
 int cpb_batch_score_alignments(cpb_batch *b, int kind, double *scores);
+/*
+ * Re-anchoring from the alignment list, for the next run of the same batch (cPecanEm --updateTheBand): replaces every pair's anchors with
+ * those its alignment gives (p->constraintDiagonalTrim, p->diagonalExpansion) -- exactly the triples cPecanRealign's job_prepare
+ * (host/realignJobs.h) builds from the cigar cPecanRealign writes for that alignment.  The alignment's maximal diagonal runs are the cigar's
+ * match operations; a run of length L gives its columns at positions [trim, L - trim) (convertPairwiseForwardStrandAlignmentToAnchorPairs,
+ * mismatched columns counted); each becomes (x, y, diagonalExpansion) and is kept iff its two bytes are equal after toupper and not N.
+ * Per pair x ascending.  Needs an alignment list (cpb_batch_ordered_chain or cpb_batch_mea); without one, with p NULL, or with a trim or
+ * expansion outside [0, 2^31) it returns CPB_ERR_ARGUMENT.  All or nothing: on any error, CPB_ERR_MEMORY for a pair whose work array does
+ * not fit the scratch budget included, the batch keeps its anchors.  On success cpb_batch_anchor_count / cpb_batch_fetch_anchors return the
+ * new anchors and the next cpb_batch_run plans anew (planReused 0); the lists of the last run, the alignment list and its scores stay as
+ * they were.  The batch then runs as one cpb_batch_create makes from the fetched anchors.
+ */
+int cpb_batch_anchors_from_alignments(cpb_batch *b, const CpbParams *p);
 /* device pointers of the same (valid until the next run / destroy) */
 const int32_t *cpb_batch_device_triples(const cpb_batch *b, int list);
 /* EXPECTATIONS mode: perPair (may be NULL) receives n * CPB_HMM_LEN(S) doubles, total receives CPB_HMM_LEN(S) doubles
