@@ -21,6 +21,9 @@ from .binding import (  # noqa: F401
     SCORE_IDENTITY_IGNORING_GAPS,
     SCORE_POSTERIOR,
     SCORE_POSTERIOR_IGNORING_GAPS,
+    OP_MATCH,
+    OP_INDEL_X,
+    OP_INDEL_Y,
     fiveState,
     fiveStateAsymmetric,
     threeState,

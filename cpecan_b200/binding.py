@@ -17,6 +17,7 @@ PAIR_ALIGNMENT_PROB_1 = 10000000
 fiveState, fiveStateAsymmetric, threeState, threeStateAsymmetric = 0, 1, 2, 3
 MODE_ALIGNED_PAIRS, MODE_ALIGNED_PAIRS_INDELS, MODE_EXPECTATIONS, MODE_FORWARD = 0, 1, 2, 3
 SCORE_IDENTITY, SCORE_IDENTITY_IGNORING_GAPS, SCORE_POSTERIOR, SCORE_POSTERIOR_IGNORING_GAPS = 0, 1, 2, 3
+OP_MATCH, OP_INDEL_X, OP_INDEL_Y = 0, 1, 2  # cigar operation types (CPB_OP_*)
 
 
 class CpbError(RuntimeError):
@@ -137,6 +138,8 @@ def _load():
     L.cpb_batch_fetch_alignments.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.cpb_batch_score_alignments.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
     L.cpb_batch_anchors_from_alignments.argtypes = [C.c_void_p, P(CpbParams)]
+    L.cpb_batch_alignment_cigars.argtypes = [C.c_void_p, C.c_void_p]
+    L.cpb_batch_fetch_cigars.argtypes = [C.c_void_p, C.c_void_p]
     L.cpb_batch_device_triples.restype = C.c_void_p
     L.cpb_batch_device_triples.argtypes = [C.c_void_p, C.c_int]
     L.cpb_batch_fetch_expectations.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
@@ -394,6 +397,16 @@ class Batch:
         out = np.zeros(max(self.n, 1), dtype=np.float64)
         _check(lib.cpb_batch_score_alignments(self.h, int(kind), C.c_void_p(out.ctypes.data)))
         return out[: self.n]
+
+    def alignment_cigars(self):
+        """-> (offsets[n+1] int64, ops[count, 2] int32 (type OP_*, length)): the cigar operations cPecanRealign writes for every pair's
+        alignment, built on the device from the alignment list"""
+        off = np.zeros(self.n + 1, dtype=np.int64)
+        _check(lib.cpb_batch_alignment_cigars(self.h, C.c_void_p(off.ctypes.data)))
+        m = int(off[-1])
+        ops = np.zeros((max(m, 1), 2), dtype=np.int32)
+        _check(lib.cpb_batch_fetch_cigars(self.h, C.c_void_p(ops.ctypes.data)))
+        return off, ops[:m]
 
     def anchors_from_alignments(self, params):
         """replaces every pair's anchors with those its alignment gives (params.constraintDiagonalTrim, params.diagonalExpansion): the

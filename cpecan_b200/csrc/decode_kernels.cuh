@@ -10,6 +10,8 @@
  *   k_decode_scores                                scoreByIdentity ... IgnoringGaps             realign.c:113-148
  *   k_reanchor_count / k_reanchor_write            the anchors job_prepare builds from the cigar of an alignment (realignJobs.h:149-173,
  *                                                  realign.c:32-72, cPecanRealign.c:98-123)
+ *   k_cigar_count / k_cigar_write                  the cigar operations cPecanRealign writes for an alignment (pairs_to_alignment,
+ *                                                  cPecanRealign.c:98-123)
  *
  * Pairs are processed in chunks whose work arrays fit the context's scratch budget (engine.cu); DecodePair says where a pair's inputs
  * and work arrays are.  Alignments are int32 (pInt, x, y) triples, 0-based, like the result lists.
@@ -580,6 +582,91 @@ __global__ void k_reanchor_write(const DecodePair *P, int nP, const int32_t *aln
             out[3 * o + 2] = expansion;
         }
         at += __popc(keeps);
+    }
+}
+
+/* ---- cigar operations of the alignment list (cpb_batch_alignment_cigars) ----
+ * pairs_to_alignment of cPecanRealign.c:98-123 for every pair: before column k an INDEL_X of x_k - x_{k-1} - 1 and an INDEL_Y of
+ * y_k - y_{k-1} - 1 where positive, with (x_-1, y_-1) = (-1, -1); then the column, which starts a MATCH operation if it is the first or
+ * follows a gap; after the last column an INDEL_X and an INDEL_Y up to (lX, lY).  A MATCH runs from its start column to the next start.
+ * One warp per pair, 32 columns per step, no work array: every lane takes its predecessor by shuffle, lane 0 from memory. */
+__device__ __forceinline__ void cigar_column(const int32_t *t, int m, int k0, int lane, int32_t &gx, int32_t &gy, bool &start) {
+    const int k = k0 + lane;
+    int32_t x = 0, y = 0;
+    if (k < m) {
+        x = t[3 * k + 1];
+        y = t[3 * k + 2];
+    }
+    int32_t px = __shfl_up_sync(0xFFFFFFFFu, x, 1), py = __shfl_up_sync(0xFFFFFFFFu, y, 1);
+    if (lane == 0) {
+        px = k0 > 0 ? t[3 * k0 - 2] : -1;
+        py = k0 > 0 ? t[3 * k0 - 1] : -1;
+    }
+    gx = k < m ? x - px - 1 : 0;
+    gy = k < m ? y - py - 1 : 0;
+    start = k < m && (k == 0 || gx > 0 || gy > 0);
+}
+
+/* the trailing INDEL_X and INDEL_Y of a pair of m columns */
+__device__ __forceinline__ void cigar_tail(const int32_t *t, int m, int64_t lX, int64_t lY, int32_t &tx, int32_t &ty) {
+    tx = (int32_t) (lX - (m > 0 ? t[3 * m - 2] : -1) - 1);
+    ty = (int32_t) (lY - (m > 0 ? t[3 * m - 1] : -1) - 1);
+}
+
+/* lens[pair] = the number of operations of the pair's cigar (at most 3m + 2) */
+__global__ void k_cigar_count(const int32_t *aln, const int64_t *off, int nPairs, const int64_t *xOff, const int64_t *yOff, int32_t *lens) {
+    const int pair = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (pair >= nPairs) return;
+    const int32_t *t = aln + 3 * off[pair];
+    const int m = (int) (off[pair + 1] - off[pair]);
+    int32_t count = 0, gx, gy;
+    bool start;
+    for (int k0 = 0; k0 < m; k0 += 32) {
+        cigar_column(t, m, k0, lane, gx, gy, start);
+        count += (gx > 0) + (gy > 0) + start;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) count += __shfl_xor_sync(0xFFFFFFFFu, count, o);
+    if (lane != 0) return;
+    int32_t tx, ty;
+    cigar_tail(t, m, xOff[pair + 1] - xOff[pair], yOff[pair + 1] - yOff[pair], tx, ty);
+    lens[pair] = count + (tx > 0) + (ty > 0);
+}
+
+/* After the scan of lens: the pair's operations as int32 (type, length) at ops[2 * opOff[pair]...].  The steps run last to first, so the
+ * next MATCH start after a lane's is the next start bit of the step's ballot or, if there is none, the first start of the steps after it
+ * (m past the last run); each lane's first operation is the step's end minus the operations of the lanes from it to 31. */
+__global__ void k_cigar_write(const int32_t *aln, const int64_t *off, int nPairs, const int64_t *xOff, const int64_t *yOff, const int64_t *opOff,
+                              int32_t *ops) {
+    const int pair = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (pair >= nPairs) return;
+    const int32_t *t = aln + 3 * off[pair];
+    const int m = (int) (off[pair + 1] - off[pair]);
+    int2 *out = reinterpret_cast<int2 *>(ops);
+    int32_t tx, ty;
+    cigar_tail(t, m, xOff[pair + 1] - xOff[pair], yOff[pair + 1] - yOff[pair], tx, ty);
+    int64_t at = opOff[pair + 1] - (tx > 0) - (ty > 0); /* one past the operation of the last column */
+    if (lane == 0) {
+        if (tx > 0) out[at] = make_int2(CPB_OP_INDEL_X, tx);
+        if (ty > 0) out[at + (tx > 0)] = make_int2(CPB_OP_INDEL_Y, ty);
+    }
+    int32_t next = m, gx, gy;
+    bool start;
+    for (int k0 = (m - 1) & ~31; k0 >= 0; k0 -= 32) {
+        cigar_column(t, m, k0, lane, gx, gy, start);
+        int32_t s = (gx > 0) + (gy > 0) + start; /* then: the operations of lanes lane..31 */
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int32_t u = __shfl_down_sync(0xFFFFFFFFu, s, o);
+            if (lane + o < 32) s += u;
+        }
+        const unsigned starts = __ballot_sync(0xFFFFFFFFu, start), after = starts & (0xFFFFFFFEu << lane);
+        int64_t w = at - s;
+        if (gx > 0) out[w++] = make_int2(CPB_OP_INDEL_X, gx);
+        if (gy > 0) out[w++] = make_int2(CPB_OP_INDEL_Y, gy);
+        if (start) out[w] = make_int2(CPB_OP_MATCH, (after != 0 ? k0 + __ffs(after) - 1 : next) - (k0 + lane));
+        at -= __shfl_sync(0xFFFFFFFFu, s, 0);
+        if (starts != 0) next = k0 + __ffs(starts) - 1;
     }
 }
 

@@ -390,6 +390,10 @@ struct cpb_batch {
     DevBuf aln;
     std::vector<int64_t> alnOff; /* n+1 */
     bool alnValid = false;
+    /* its cigar operations (cpb_batch_alignment_cigars): int32 (type, length) per operation; they go whenever the alignment list goes */
+    DevBuf cig;
+    std::vector<int64_t> cigOff; /* n+1, in operations */
+    bool cigValid = false;
     int lastMode = -1, lastS = 0;
     CpbRunStats stats;
     HostArray<RegionDev> hRegions;
@@ -447,7 +451,7 @@ static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, cons
     {
         DevBuf *all[] = { &b->strips, &b->symX, &b->symY, &b->dAnchors, &b->dPairTab, &b->splitFlags, &b->regions, &b->diags, &b->blocks, &b->totals, &b->lists, &b->counts, &b->offsets,
                           &b->masks, &b->tileSums, &b->pairCounts, &b->partials, &b->pairBlockOff, &b->perPair, &b->hmmTotal, &b->forwardOut, &b->out[0],
-                          &b->out[1], &b->out[2], &b->ckRegions, &b->ckDiags, &b->ckSizes, &b->ckpt, &b->keptX, &b->keptY, &b->aln };
+                          &b->out[1], &b->out[2], &b->ckRegions, &b->ckDiags, &b->ckSizes, &b->ckpt, &b->keptX, &b->keptY, &b->aln, &b->cig };
         for (DevBuf *d : all) d->pool = &ctx->pool;
     }
     b->n = nPairs;
@@ -585,7 +589,7 @@ extern "C" void cpb_batch_destroy(cpb_batch *b) {
     cudaSetDevice(b->ctx->device);
     DevBuf *bufs[] = { &b->strips, &b->symX, &b->symY, &b->dAnchors, &b->dPairTab, &b->splitFlags, &b->regions, &b->diags, &b->blocks, &b->totals, &b->lists, &b->counts,
                        &b->offsets, &b->masks, &b->tileSums, &b->pairCounts, &b->partials, &b->pairBlockOff, &b->perPair, &b->hmmTotal, &b->forwardOut, &b->out[0], &b->out[1],
-                       &b->out[2], &b->ckRegions, &b->ckDiags, &b->ckSizes, &b->ckpt, &b->keptX, &b->keptY, &b->aln };
+                       &b->out[2], &b->ckRegions, &b->ckDiags, &b->ckSizes, &b->ckpt, &b->keptX, &b->keptY, &b->aln, &b->cig };
     for (DevBuf *d : bufs) d->release();
     if (b->anchors != nullptr && b->anchorsOwn.empty()) b->ctx->pinned.give(b->anchors);
     delete b;
@@ -1925,7 +1929,7 @@ extern "C" int cpb_batch_run(cpb_batch *b, const CpbModel *m, const CpbParams *p
         cpb_set_error("cpb_batch_run: bad argument");
         return CPB_ERR_ARGUMENT;
     }
-    b->alnValid = false; /* the alignment list belongs to the lists of the run before */
+    b->alnValid = b->cigValid = false; /* the alignment list belongs to the lists of the run before */
     int rc = check_params(p);
     if (rc != CPB_OK) return rc;
     if (p->dynamicAnchorExpansion && mode != CPB_MODE_FORWARD && b->oddExpansionPair >= 0) {
@@ -2274,7 +2278,7 @@ static int decode_chunks(cpb_batch *b, const char *call, std::vector<DecodePair>
 }
 
 extern "C" int cpb_batch_ordered_chain(cpb_batch *b, float matchGamma) {
-    if (b != nullptr) b->alnValid = false; /* a decode call replaces the list, also when it is refused */
+    if (b != nullptr) b->alnValid = b->cigValid = false; /* a decode call replaces the list, also when it is refused */
     if (b == nullptr || (b->lastMode != CPB_MODE_ALIGNED_PAIRS && b->lastMode != CPB_MODE_ALIGNED_PAIRS_INDELS)) {
         cpb_set_error("cpb_batch_ordered_chain: no aligned-pair results in this batch");
         return CPB_ERR_ARGUMENT;
@@ -2349,7 +2353,7 @@ static int ref_order_tables(cpb_batch *b, std::vector<DecodePair> &P, RefOrderTa
 }
 
 extern "C" int cpb_batch_mea(cpb_batch *b, float gapGamma, int leftShift, double *scores) {
-    if (b != nullptr) b->alnValid = false; /* a decode call replaces the list, also when it is refused */
+    if (b != nullptr) b->alnValid = b->cigValid = false; /* a decode call replaces the list, also when it is refused */
     if (b == nullptr || b->lastMode != CPB_MODE_ALIGNED_PAIRS_INDELS) {
         cpb_set_error("cpb_batch_mea: needs the gap lists of an ALIGNED_PAIRS_INDELS run");
         return CPB_ERR_ARGUMENT;
@@ -2390,7 +2394,7 @@ extern "C" int cpb_batch_mea(cpb_batch *b, float gapGamma, int leftShift, double
 /* Test support, not part of the ABI header: the alignment list becomes list 0 of the last run in the reference's order as cpb_batch_mea
  * builds it on the device (k_ref_order), so that this permutation can be compared with cpb_batch_fetch_pairs_reference_order. */
 extern "C" int cpb_debug_reference_order(cpb_batch *b) {
-    if (b != nullptr) b->alnValid = false;
+    if (b != nullptr) b->alnValid = b->cigValid = false;
     if (b == nullptr || (b->lastMode != CPB_MODE_ALIGNED_PAIRS && b->lastMode != CPB_MODE_ALIGNED_PAIRS_INDELS)) {
         cpb_set_error("cpb_debug_reference_order: no aligned-pair results in this batch");
         return CPB_ERR_ARGUMENT;
@@ -2457,6 +2461,64 @@ extern "C" int cpb_batch_score_alignments(cpb_batch *b, int kind, double *scores
     CUDA_TRY(cudaMemcpyAsync(scores, dS.p, (size_t) b->n * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     CUDA_TRY(cudaGetLastError());
+    return CPB_OK;
+}
+
+/* The cigar operations of every pair's alignment (k_cigar_count / k_cigar_write).  No work array: the counts are scanned over all pairs
+ * at once and the operation buffer is sized from the exact total. */
+extern "C" int cpb_batch_alignment_cigars(cpb_batch *b, int64_t *offsets) {
+    if (b != nullptr) b->cigValid = false; /* a build replaces the cigar list, also when it fails */
+    if (b == nullptr || !b->alnValid || offsets == nullptr) {
+        cpb_set_error("cpb_batch_alignment_cigars: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain or cpb_batch_mea after the run"
+                                                                                     : "bad argument");
+        return CPB_ERR_ARGUMENT;
+    }
+    const int64_t n = b->n;
+    for (int64_t i = 0; i < n; i++) {
+        if (3 * (b->alnOff[(size_t) i + 1] - b->alnOff[(size_t) i]) + 2 > INT32_MAX) {
+            cpb_set_error("cpb_batch_alignment_cigars: pair %lld has too long an alignment for 2^31 operations", (long long) i);
+            return CPB_ERR_ARGUMENT;
+        }
+    }
+    CUDA_TRY(cudaSetDevice(b->ctx->device));
+    cudaStream_t st = b->ctx->stream;
+    DevBuf dOff, dX, dY, dLens, dOpOff, dTiles;
+    for (DevBuf *d : { &dOff, &dX, &dY, &dLens, &dOpOff, &dTiles }) d->pool = &b->ctx->pool;
+    int rc = upload_pair_tables(b, b->alnOff, dOff, dX, dY);
+    if (rc != CPB_OK || (rc = dLens.reserve((size_t) std::max<int64_t>(n, 1) * sizeof(int32_t))) != CPB_OK ||
+        (rc = dOpOff.reserve((size_t) (n + 1) * sizeof(int64_t))) != CPB_OK || (rc = dTiles.reserve((size_t) ((n + SCAN_TILE - 1) / SCAN_TILE + 1) * 8)) != CPB_OK)
+        return rc;
+    const int32_t *aln = b->aln.as<int32_t>();
+    if (n > 0) k_cigar_count<<<grid_of(n * 32, 256), 256, 0, st>>>(aln, dOff.as<int64_t>(), (int) n, dX.as<int64_t>(), dY.as<int64_t>(), dLens.as<int32_t>());
+    scan_counts(st, dLens.as<int32_t>(), n, 0, dTiles.as<int64_t>(), dOpOff.as<int64_t>());
+    std::vector<int64_t> opOff((size_t) n + 1);
+    CUDA_TRY(cudaMemcpyAsync(opOff.data(), dOpOff.p, (size_t) (n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    if ((rc = b->cig.reserve((size_t) std::max<int64_t>(opOff[(size_t) n], 1) * 2 * sizeof(int32_t))) != CPB_OK) return rc;
+    if (n > 0)
+        k_cigar_write<<<grid_of(n * 32, 256), 256, 0, st>>>(aln, dOff.as<int64_t>(), (int) n, dX.as<int64_t>(), dY.as<int64_t>(), dOpOff.as<int64_t>(),
+                                                           b->cig.as<int32_t>());
+    b->stats.kernelLaunches += (n > 0 ? 2 : 0) + 3;
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    b->cigOff.swap(opOff);
+    b->cigValid = true;
+    memcpy(offsets, b->cigOff.data(), (size_t) (n + 1) * sizeof(int64_t));
+    return CPB_OK;
+}
+
+extern "C" int cpb_batch_fetch_cigars(const cpb_batch *b, int32_t *ops) {
+    if (b == nullptr || !b->cigValid || (ops == nullptr && b->cigOff[(size_t) b->n] > 0)) {
+        cpb_set_error("cpb_batch_fetch_cigars: %s", b != nullptr && !b->cigValid ? "no cigars: call cpb_batch_alignment_cigars after the decode" : "bad argument");
+        return CPB_ERR_ARGUMENT;
+    }
+    const int64_t count = b->cigOff[(size_t) b->n];
+    if (count > 0) {
+        CUDA_TRY(cudaSetDevice(b->ctx->device));
+        CUDA_TRY(cudaMemcpyAsync(ops, b->cig.p, (size_t) count * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, b->ctx->stream));
+        CUDA_TRY(cudaStreamSynchronize(b->ctx->stream));
+    }
     return CPB_OK;
 }
 

@@ -4,10 +4,12 @@
  * cPecanRealign.c (options :374-473, coordinate handling :509-523, post-processing :546-599, expectations :530-535 and :608-614).
  *
  * What is different is the shape of the loop.  The reference runs one alignment at a time through the CPU DP
- * (cPecanRealign.c:509-605).  Here the cigars are read in batches, every batch goes through ONE device pass
- * (getAlignedPairsUsingAnchorsBatch / getExpectationsUsingAnchorsBatch of libcpecan.so), and the host only does the list work
- * either side of it; output order is input order.  There is no host DP: without a CUDA device the program aborts with the
- * engine's message.
+ * (cPecanRealign.c:509-605).  Here the cigars are read in batches and every batch goes through ONE device pass of libcpecan.so:
+ * getRealignedCigarsUsingAnchorsBatch runs the pair-HMM, reweights, chains, scores and builds the output's cigar operations on the
+ * device, so only operations and scores (and, for the posterior files, triples) come back; --rescoreOriginalAlignment takes the
+ * posteriors (getAlignedPairsUsingAnchorsBatch) and --outputExpectations the expectations (getExpectationsUsingAnchorsBatch).  The
+ * host threads prepare the sub-sequences and anchors before the pass and write the cigars after it; output order is input order.
+ * There is no host DP: without a CUDA device the program aborts with the engine's message.
  */
 #include <getopt.h>
 #include <time.h>
@@ -43,15 +45,26 @@ static void usage(void) {
 
 static int64_t transform_coordinate(int64_t c, int64_t shift, bool flip, int64_t seqLength) { return shift + (flip ? seqLength - 1 - c : c); }
 
-static void write_posterior_probs(const char *file, stList *pairs, int64_t shift1, bool flip1, int64_t len1, int64_t shift2, bool flip2, int64_t len2) {
+/* n (pInt, x, y) triples, in original coordinates */
+static void write_posterior_probs(const char *file, const int32_t *pairs, int64_t n, const Job *j) {
+    const struct PairwiseAlignment *pA = j->pA;
     FILE *f = fopen(file, "w");
     if (f == NULL) st_errAbort("cPecanRealign: cannot write %s", file);
-    for (int64_t i = 0; i < stList_length(pairs); i++) {
-        stIntTuple *t = stList_get(pairs, i);
-        fprintf(f, "%" PRIi64 "\t%" PRIi64 "\t%f\n", transform_coordinate(stIntTuple_get(t, 1), shift1, flip1, len1),
-                transform_coordinate(stIntTuple_get(t, 2), shift2, flip2, len2), ((double) stIntTuple_get(t, 0)) / PAIR_ALIGNMENT_PROB_1);
+    for (int64_t i = 0; i < n; i++) {
+        fprintf(f, "%" PRIi64 "\t%" PRIi64 "\t%f\n", transform_coordinate(pairs[3 * i + 1], j->shift1, j->flip1, pA->end1 - pA->start1),
+                transform_coordinate(pairs[3 * i + 2], j->shift2, j->flip2, pA->end2 - pA->start2), ((double) pairs[3 * i]) / PAIR_ALIGNMENT_PROB_1);
     }
     fclose(f);
+}
+
+static void write_posterior_list(const char *file, stList *pairs, const Job *j) {
+    const int64_t n = stList_length(pairs);
+    int32_t *t = xmalloc((size_t) n * 3 * sizeof(int32_t));
+    for (int64_t i = 0; i < n; i++) {
+        for (int64_t k = 0; k < 3; k++) t[3 * i + k] = (int32_t) stIntTuple_get(stList_get(pairs, i), k);
+    }
+    write_posterior_probs(file, t, n, j);
+    free(t);
 }
 
 /* ---- the original alignment's columns with their posterior weights (cPecanRealign.c:322-353) ---- */
@@ -90,7 +103,7 @@ static stList *score_anchor_pairs(stList *anchorPairs, stList *alignedPairs) {
     return scored;
 }
 
-/* ---- aligned pairs -> cigar (cPecanRealign.c:50-92) ---- */
+/* ---- aligned pairs -> cigar (cPecanRealign.c:50-92), for --rescoreOriginalAlignment; the realignment's cigars come from the device ---- */
 
 static void add_op(struct List *ops, int64_t type, int64_t length) { listAppend(ops, constructAlignmentOperation(type, length, 0)); }
 
@@ -185,31 +198,63 @@ typedef struct {
         rescoreByPosteriorProbabilityIgnoringGaps;
     int64_t splitIndelsLongerThanThis; /* -1 = never */
     const char *posteriorProbsFile, *allPosteriorProbsFile;
-    bool reweightedOnDevice; /* the pairs arrive already reweighted by gapGamma (nobody asked for the raw posteriors) */
 } Options;
 
-/* everything after the device pass for one alignment (cPecanRealign.c:540-599); consumes alignedPairs */
-static void job_finish(Job *j, stList *alignedPairs, const Options *o, const PairwiseAlignmentParameters *p, FILE *out) {
+/* the score the options ask for (cPecanRealign.c:561-569: the first of these that is set), or -1 to keep the input's */
+static int score_kind(const Options *o) {
+    if (o->rescoreByPosteriorProbability) return CPECAN_SCORE_BY_POSTERIOR_PROBABILITY;
+    if (o->rescoreByPosteriorProbabilityIgnoringGaps) return CPECAN_SCORE_BY_POSTERIOR_PROBABILITY_IGNORING_GAPS;
+    if (o->rescoreByIdentity) return CPECAN_SCORE_BY_IDENTITY;
+    if (o->rescoreByIdentityIgnoringGaps) return CPECAN_SCORE_BY_IDENTITY_IGNORING_GAPS;
+    return -1;
+}
+
+/* the realigned alignment of a job, on the forward strands from 0, to its original strands and coordinates and out as cigars
+ * (cPecanRealign.c:570-599); consumes rPA */
+static void write_alignment(const Job *j, struct PairwiseAlignment *rPA, const Options *o, FILE *out) {
+    rebase(&rPA->start1, &rPA->end1, &rPA->strand1, j->shift1, j->flip1);
+    rebase(&rPA->start2, &rPA->end2, &rPA->strand2, j->shift2, j->flip2);
+    checkPairwiseAlignment(rPA);
+    if (o->splitIndelsLongerThanThis != -1) {
+        stList *pieces = split_alignment(rPA, o->splitIndelsLongerThanThis);
+        for (int64_t i = 0; i < stList_length(pieces); i++) cigarWrite(out, stList_get(pieces, i), 0);
+        stList_destruct(pieces);
+    } else {
+        cigarWrite(out, rPA, 0);
+    }
+    destructPairwiseAlignment(rPA);
+}
+
+/* everything after the device pass for alignment i of the batch (cPecanRealign.c:540-599): the device decoded it (r) */
+static void job_finish(Job *j, const CpecanRealignedCigars *r, int64_t i, const Options *o, FILE *out) {
+    struct PairwiseAlignment *pA = j->pA;
+    if (o->allPosteriorProbsFile != NULL) {
+        const int64_t *off = r->rawPairs.offsets;
+        write_posterior_probs(o->allPosteriorProbsFile, r->rawPairs.values + 3 * off[i], off[i + 1] - off[i], j);
+    }
+    if (r->scores != NULL) pA->score = r->scores[i];
+    if (o->posteriorProbsFile != NULL) {
+        const int64_t *off = r->alignments.offsets;
+        write_posterior_probs(o->posteriorProbsFile, r->alignments.values + 3 * off[i], off[i + 1] - off[i], j);
+    }
+    struct List *ops = constructEmptyList(0, (void (*)(void *)) destructAlignmentOperation);
+    for (int64_t k = r->ops.offsets[i]; k < r->ops.offsets[i + 1]; k++) add_op(ops, r->ops.values[2 * k], r->ops.values[2 * k + 1]);
+    write_alignment(j, constructPairwiseAlignment(pA->contig1, 0, pA->end1, 1, pA->contig2, 0, pA->end2, 1, pA->score, ops), o, out);
+}
+
+/* the same for --rescoreOriginalAlignment: the input columns scored against the posteriors (consumes alignedPairs) */
+static void job_finish_rescored(Job *j, stList *alignedPairs, const Options *o, FILE *out) {
     struct PairwiseAlignment *pA = j->pA;
     const int64_t lX = (int64_t) strlen(j->subX), lY = (int64_t) strlen(j->subY);
-    if (o->allPosteriorProbsFile != NULL) {
-        write_posterior_probs(o->allPosteriorProbsFile, alignedPairs, j->shift1, j->flip1, pA->end1 - pA->start1, j->shift2, j->flip2, pA->end2 - pA->start2);
-    }
-    if (o->rescoreOriginalAlignment) {
-        stList *rescored = score_anchor_pairs(j->anchors, alignedPairs);
-        stList_destruct(alignedPairs);
-        alignedPairs = rescored;
-    } else {
-        if (!o->reweightedOnDevice) alignedPairs = reweightAlignedPairs2(alignedPairs, lX, lY, p->gapGamma);
-        alignedPairs = filterPairwiseAlignmentToMakePairsOrdered(alignedPairs, j->subX, j->subY, o->matchGamma);
-    }
+    if (o->allPosteriorProbsFile != NULL) write_posterior_list(o->allPosteriorProbsFile, alignedPairs, j);
+    stList *rescored = score_anchor_pairs(j->anchors, alignedPairs);
+    stList_destruct(alignedPairs);
+    alignedPairs = rescored;
     if (o->rescoreByPosteriorProbability) pA->score = scoreByPosteriorProbability(lX, lY, alignedPairs);
     else if (o->rescoreByPosteriorProbabilityIgnoringGaps) pA->score = scoreByPosteriorProbabilityIgnoringGaps(alignedPairs);
     else if (o->rescoreByIdentity) pA->score = scoreByIdentity(j->subX, j->subY, lX, lY, alignedPairs);
     else if (o->rescoreByIdentityIgnoringGaps) pA->score = scoreByIdentityIgnoringGaps(j->subX, j->subY, alignedPairs);
-    if (o->posteriorProbsFile != NULL) {
-        write_posterior_probs(o->posteriorProbsFile, alignedPairs, j->shift1, j->flip1, pA->end1 - pA->start1, j->shift2, j->flip2, pA->end2 - pA->start2);
-    }
+    if (o->posteriorProbsFile != NULL) write_posterior_list(o->posteriorProbsFile, alignedPairs, j);
     /* (weight, x, y) -> (x, y), ascending */
     const int64_t nPairs = stList_length(alignedPairs);
     int64_t *xy = xmalloc((size_t) (nPairs > 0 ? nPairs : 1) * 2 * sizeof(int64_t));
@@ -224,27 +269,23 @@ static void job_finish(Job *j, stList *alignedPairs, const Options *o, const Pai
     if (!ascending) qsort(xy, (size_t) nPairs, 2 * sizeof(int64_t), by_x_then_y);
     struct PairwiseAlignment *rPA = pairs_to_alignment(pA->contig1, pA->contig2, pA->score, pA->end1, pA->end2, xy, nPairs);
     free(xy);
-    rebase(&rPA->start1, &rPA->end1, &rPA->strand1, j->shift1, j->flip1);
-    rebase(&rPA->start2, &rPA->end2, &rPA->strand2, j->shift2, j->flip2);
-    checkPairwiseAlignment(rPA);
-    if (o->splitIndelsLongerThanThis != -1) {
-        stList *pieces = split_alignment(rPA, o->splitIndelsLongerThanThis);
-        for (int64_t i = 0; i < stList_length(pieces); i++) cigarWrite(out, stList_get(pieces, i), 0);
-        stList_destruct(pieces);
-    } else {
-        cigarWrite(out, rPA, 0);
-    }
-    destructPairwiseAlignment(rPA);
+    write_alignment(j, rPA, o, out);
 }
 
 /* the host work on either side of a device pass, over a range of the batch's alignments (cpecan_parallel_for) */
 typedef struct {
     Job *jobs;
-    stList **pairs;
+    stList **pairs;                 /* --rescoreOriginalAlignment: the posteriors of every alignment */
+    const CpecanRealignedCigars *r; /* otherwise: the device's realignments */
     char **text;
     const PairwiseAlignmentParameters *p;
     const Options *o;
 } HostPass;
+
+static void finish_one(HostPass *h, int64_t i, FILE *out) {
+    if (h->pairs != NULL) job_finish_rescored(&h->jobs[i], h->pairs[i], h->o, out);
+    else job_finish(&h->jobs[i], h->r, i, h->o, out);
+}
 
 static void prepare_range(int64_t first, int64_t last, void *arg) {
     HostPass *h = arg;
@@ -257,7 +298,7 @@ static void finish_range(int64_t first, int64_t last, void *arg) {
         size_t size = 0;
         FILE *f = open_memstream(&h->text[i], &size);
         if (f == NULL) st_errAbort("cPecanRealign: out of memory");
-        job_finish(&h->jobs[i], h->pairs[i], h->o, h->p, f);
+        finish_one(h, i, f);
         fclose(f);
     }
 }
@@ -405,7 +446,7 @@ int main(int argc, char *argv[]) {
             work[i + 1] = work[i] + llabs((long long) (q->end1 - q->start1)) + llabs((long long) (q->end2 - q->start2)) + 1;
         }
         {
-            HostPass pass = { jobs, NULL, NULL, p, NULL };
+            HostPass pass = { jobs, NULL, NULL, NULL, p, NULL };
             cpecan_parallel_for(n, work, prepare_range, &pass);
         }
         const char **sX = xmalloc((size_t) n * sizeof(char *)), **sY = xmalloc((size_t) n * sizeof(char *));
@@ -422,18 +463,26 @@ int main(int argc, char *argv[]) {
         if (hmmExpectations != NULL) {
             getExpectationsUsingAnchorsBatch(sM, hmmExpectations, n, sX, sY, anchors, p, ragged, ragged);
         } else {
-            /* the gap reweighting (cPecanRealign.c:560) runs on the device unless the raw posteriors are wanted as well */
-            o.reweightedOnDevice = !o.rescoreOriginalAlignment && o.allPosteriorProbsFile == NULL;
-            stList **pairs = o.reweightedOnDevice ? getReweightedAlignedPairsUsingAnchorsBatch(sM, n, sX, sY, anchors, p, ragged, ragged, p->gapGamma)
-                                                  : getAlignedPairsUsingAnchorsBatch(sM, n, sX, sY, anchors, p, ragged, ragged);
-            stage("batch call (device pass + lists)");
+            /* the realignment (cPecanRealign.c:560-569: reweighting, ordered chain, score) and its cigar are built on the device; only
+             * --rescoreOriginalAlignment scores the input columns against the posteriors here */
+            stList **pairs = NULL;
+            CpecanRealignedCigars *r = NULL;
+            if (o.rescoreOriginalAlignment) {
+                pairs = getAlignedPairsUsingAnchorsBatch(sM, n, sX, sY, anchors, p, ragged, ragged);
+                stage("batch call (device pass + lists)");
+            } else {
+                r = getRealignedCigarsUsingAnchorsBatch(sM, n, sX, sY, anchors, p, ragged, ragged, o.matchGamma, score_kind(&o), o.posteriorProbsFile != NULL,
+                                                        o.allPosteriorProbsFile != NULL);
+                stage("batch call (device pass, decode, cigars)");
+            }
+            HostPass pass = { jobs, pairs, r, NULL, p, &o };
             if (o.posteriorProbsFile != NULL || o.allPosteriorProbsFile != NULL) {
-                for (int64_t i = 0; i < n; i++) job_finish(&jobs[i], pairs[i], &o, p, stdout); /* they append to one file, in input order */
+                for (int64_t i = 0; i < n; i++) finish_one(&pass, i, stdout); /* each rewrites the files, in input order */
             } else {
                 /* everything after the device pass is per alignment: on the host threads, each alignment's cigars into a buffer of
                  * its own, the buffers to the standard output in input order */
                 char **text = xmalloc((size_t) n * sizeof(char *));
-                HostPass pass = { jobs, pairs, text, p, &o };
+                pass.text = text;
                 cpecan_parallel_for(n, work, finish_range, &pass);
                 for (int64_t i = 0; i < n; i++) {
                     fputs(text[i], stdout);
@@ -442,7 +491,8 @@ int main(int argc, char *argv[]) {
                 free(text);
             }
             free(pairs);
-            stage("chains, cigars out (host threads)");
+            cpecanRealignedCigars_destruct(r);
+            stage("cigars out (host threads)");
         }
         for (int64_t i = 0; i < n; i++) job_release(&jobs[i]);
         free(work);

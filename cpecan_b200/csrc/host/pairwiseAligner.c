@@ -429,11 +429,109 @@ typedef struct {
     const char *const *sX, *const *sY;
     stList *const *anchorPairs;
     const bool *raggedLeft, *raggedRight;
+    /* getRealignedCigarsUsingAnchorsBatch */
+    int realign, scoreKind, wantAlignments, wantRawPairs;
+    float matchGamma;
     /* results, in the caller's indexing */
     stList **lists[3];
     double *logProbs;
-    cpb_batch *batch; /* expectation mode / keepBatch: left alive for the reduction */
+    cpb_batch *batch;             /* expectation mode / keepBatch: left alive for the reduction */
+    CpecanRealignedCigars cigars; /* realign: this device's problems, in the order of idx */
 } DeviceJob;
+
+static void engine_check(int rc) {
+    if (rc == CPB_ERR_BAND) st_errAbort("%s: %s", PAIRWISE_ALIGNMENT_EXCEPTION_ID, cpb_last_error());
+    if (rc != CPB_OK) st_errAbort("cpecan: %s", cpb_last_error());
+}
+
+/* cPecanRealign's default steps for every alignment of a batch (job_finish of host/cPecanRealign.c): an ALIGNED_PAIRS run, reweighting by
+ * q->gapGamma, the heaviest ordered chain into the alignment list.  raw, when not NULL, receives list 0 of the run (n pairs) before the
+ * reweighting, in the reference's order.  matchGamma above 1 admits no pair (weights are at most PAIR_ALIGNMENT_PROB_1): then no chain is
+ * built and the caller gives every alignment as empty. */
+static void realign_steps(cpb_batch *b, int64_t n, const CpbModel *model, const CpbParams *q, float matchGamma, CpecanFlatList *raw) {
+    engine_check(cpb_batch_run(b, model, q, CPB_MODE_ALIGNED_PAIRS));
+    if (raw != NULL) {
+        raw->offsets = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t));
+        raw->values = cpecan_malloc((size_t) (3 * cpb_batch_result_count(b, 0) + 3) * sizeof(int32_t));
+        engine_check(cpb_batch_fetch_pairs_reference_order(b, 0, raw->offsets, raw->values));
+    }
+    engine_check(cpb_batch_reweight_pairs(b, q->gapGamma));
+    if (matchGamma <= 1.0f) engine_check(cpb_batch_ordered_chain(b, matchGamma));
+}
+
+/* the score of an empty alignment, from the host function itself (the "ignoring gaps" forms divide 0 by 0, and the sign of that NaN is the
+ * host's) */
+static double empty_alignment_score(int kind, const char *sX, const char *sY) {
+    stList *none = stList_construct();
+    const int64_t lX = (int64_t) strlen(sX), lY = (int64_t) strlen(sY);
+    double s;
+    switch (kind) {
+    case CPECAN_SCORE_BY_IDENTITY: s = scoreByIdentity((char *) sX, (char *) sY, lX, lY, none); break;
+    case CPECAN_SCORE_BY_IDENTITY_IGNORING_GAPS: s = scoreByIdentityIgnoringGaps((char *) sX, (char *) sY, none); break;
+    case CPECAN_SCORE_BY_POSTERIOR_PROBABILITY: s = scoreByPosteriorProbability(lX, lY, none); break;
+    default: s = scoreByPosteriorProbabilityIgnoringGaps(none); break;
+    }
+    stList_destruct(none);
+    return s;
+}
+
+/* the realignment of this device's problems (realign_steps, then cigars, scores and triples off the device) into j->cigars */
+static void device_realign(DeviceJob *j, cpb_batch *b, const char *const *sX, const char *const *sY) {
+    const int64_t n = j->n;
+    CpecanRealignedCigars *r = &j->cigars;
+    memset(r, 0, sizeof(*r));
+    r->n = n;
+    CpbParams q;
+    to_engine_params(j->p, &q);
+    realign_steps(b, n, cpecan_model_of(j->sM), &q, j->matchGamma, j->wantRawPairs ? &r->rawPairs : NULL);
+    int64_t *opOff = r->ops.offsets = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t));
+    if (j->scoreKind >= 0) r->scores = cpecan_malloc((size_t) (n + 1) * sizeof(double));
+    if (j->matchGamma > 1.0f) { /* every alignment is empty: [INDEL_X lX][INDEL_Y lY] */
+        int32_t *ops = r->ops.values = cpecan_malloc((size_t) (4 * n + 1) * sizeof(int32_t));
+        opOff[0] = 0;
+        for (int64_t i = 0; i < n; i++) {
+            const int32_t len[2] = { (int32_t) strlen(sX[i]), (int32_t) strlen(sY[i]) };
+            int64_t at = opOff[i];
+            for (int s = 0; s < 2; s++) {
+                if (len[s] > 0) {
+                    ops[2 * at] = s == 0 ? CPB_OP_INDEL_X : CPB_OP_INDEL_Y;
+                    ops[2 * at + 1] = len[s];
+                    at++;
+                }
+            }
+            opOff[i + 1] = at;
+            if (r->scores != NULL) r->scores[i] = empty_alignment_score(j->scoreKind, sX[i], sY[i]);
+        }
+        if (j->wantAlignments) {
+            r->alignments.offsets = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t));
+            memset(r->alignments.offsets, 0, (size_t) (n + 1) * sizeof(int64_t));
+            r->alignments.values = cpecan_malloc(3 * sizeof(int32_t));
+        }
+        return;
+    }
+    engine_check(cpb_batch_alignment_cigars(b, opOff));
+    int32_t *ops = r->ops.values = cpecan_malloc((size_t) (2 * opOff[n] + 2) * sizeof(int32_t));
+    engine_check(cpb_batch_fetch_cigars(b, ops));
+    if (r->scores != NULL) {
+        engine_check(cpb_batch_score_alignments(b, j->scoreKind, r->scores));
+        for (int64_t i = 0; i < n; i++) { /* an alignment without a MATCH operation is empty */
+            bool empty = true;
+            for (int64_t k = opOff[i]; k < opOff[i + 1] && empty; k++) empty = ops[2 * k] != CPB_OP_MATCH;
+            if (empty) r->scores[i] = empty_alignment_score(j->scoreKind, sX[i], sY[i]);
+        }
+    }
+    if (j->wantAlignments) {
+        r->alignments.offsets = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t));
+        r->alignments.values = cpecan_malloc((size_t) (3 * cpb_batch_alignments_count(b) + 3) * sizeof(int32_t));
+        engine_check(cpb_batch_fetch_alignments(b, r->alignments.offsets, r->alignments.values));
+    }
+    if (getenv("CPECAN_HOST_TIMING") != NULL) {
+        const int64_t bytes = 8 * (n + 1) + 8 * opOff[n] + (r->scores != NULL ? 8 * n : 0) +
+                              (j->wantAlignments ? 8 * (n + 1) + 12 * r->alignments.offsets[n] : 0) +
+                              (j->wantRawPairs ? 8 * (n + 1) + 12 * r->rawPairs.offsets[n] : 0);
+        fprintf(stderr, "    device to host: %lld cigar operations, %lld bytes in all\n", (long long) opOff[n], (long long) bytes);
+    }
+}
 
 static void *device_job(void *v) {
     DeviceJob *j = v;
@@ -463,13 +561,15 @@ static void *device_job(void *v) {
     pack(&k, n, sX, sY, an, rl, rr, j->p->diagonalExpansion);
     STAGE("pack (tuples -> flat arrays)");
     cpb_batch *b = NULL;
-    if (j->mode < 0) { /* resident batch: inputs to the device, no run yet */
+    if (j->mode < 0 || j->realign) { /* resident batch: inputs to the device, no run yet; realign: runs in device_realign */
         if (cpb_batch_create(j->ctx, k.n, k.seqX, k.xOff, k.seqY, k.yOff, k.anchors, k.aOff, k.rl, k.rr, &b) != CPB_OK) st_errAbort("cpecan: %s", cpb_last_error());
+        if (j->realign) device_realign(j, b, sX, sY);
     } else {
         b = run(j->ctx, &k, j->sM, j->p, j->mode, j->reweight ? NULL : &sinks); /* (reweighting rewrites the list on the device after the run) */
     }
     STAGE("device pass (create + run)");
-    if (j->mode == CPB_MODE_ALIGNED_PAIRS || j->mode == CPB_MODE_ALIGNED_PAIRS_INDELS) {
+    if (j->realign) {
+    } else if (j->mode == CPB_MODE_ALIGNED_PAIRS || j->mode == CPB_MODE_ALIGNED_PAIRS_INDELS) {
         if (j->reweight && cpb_batch_reweight_pairs(b, j->gapGamma) != CPB_OK) st_errAbort("cpecan: %s", cpb_last_error());
         const int nLists = j->mode == CPB_MODE_ALIGNED_PAIRS ? 1 : 3;
         for (int l = 0; l < nLists; l++) {
@@ -626,6 +726,77 @@ void getAlignedPairsWithIndelsUsingAnchorsBatch(StateMachine *sM, int64_t n, con
     *gapYPairs = proto.lists[2];
 }
 
+/* per-device flat lists (entries of `width` int32; the problems of device d are idx[d], ascending) as one list in the problems' own order */
+static CpecanFlatList *flat_list(CpecanRealignedCigars *r, int which) { return which == 0 ? &r->ops : (which == 1 ? &r->alignments : &r->rawPairs); }
+
+/* flat list `which` (entries of `width` int32) of every device (the problems of device d are idx[d], ascending) as one list in the problems'
+ * own order; frees the devices' lists */
+static void gather_flat(CpecanRealignedCigars *r, int nDev, int64_t *const *idx, DeviceJob *jobs, int which, int width) {
+    const int64_t n = r->n;
+    CpecanFlatList *to = flat_list(r, which);
+    int64_t *off = to->offsets = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t));
+    off[0] = 0;
+    for (int d = 0; d < nDev; d++) {
+        const int64_t *o = flat_list(&jobs[d].cigars, which)->offsets;
+        for (int64_t i = 0; i < jobs[d].n; i++) off[idx[d][i] + 1] = o[i + 1] - o[i];
+    }
+    for (int64_t i = 0; i < n; i++) off[i + 1] += off[i];
+    to->values = cpecan_malloc((size_t) (width * off[n] + width) * sizeof(int32_t));
+    for (int d = 0; d < nDev; d++) {
+        CpecanFlatList *from = flat_list(&jobs[d].cigars, which);
+        for (int64_t i = 0; i < jobs[d].n; i++)
+            memcpy(to->values + width * off[idx[d][i]], from->values + width * from->offsets[i],
+                   (size_t) (width * (from->offsets[i + 1] - from->offsets[i])) * sizeof(int32_t));
+        free(from->offsets);
+        free(from->values);
+    }
+}
+
+CpecanRealignedCigars *getRealignedCigarsUsingAnchorsBatch(StateMachine *sM, int64_t n, const char *const *sX, const char *const *sY,
+                                                           stList *const *anchorPairs, PairwiseAlignmentParameters *p, const bool *raggedLeft,
+                                                           const bool *raggedRight, float matchGamma, int scoreKind, bool wantAlignments,
+                                                           bool wantRawPairs) {
+    if (!(matchGamma >= 0.0f) || scoreKind < -1 || scoreKind > CPECAN_SCORE_BY_POSTERIOR_PROBABILITY_IGNORING_GAPS)
+        st_errAbort("getRealignedCigarsUsingAnchorsBatch: matchGamma must be >= 0 (not %g) and scoreKind in [-1, 3] (not %d)", (double) matchGamma, scoreKind);
+    DeviceJob proto = job_of(sM, sX, sY, anchorPairs, p, raggedLeft, raggedRight, CPB_MODE_ALIGNED_PAIRS), jobs[CPECAN_MAX_DEVICES];
+    proto.realign = 1;
+    proto.matchGamma = matchGamma;
+    proto.scoreKind = scoreKind;
+    proto.wantAlignments = wantAlignments;
+    proto.wantRawPairs = wantRawPairs;
+    int64_t *idx[CPECAN_MAX_DEVICES];
+    const int nDev = run_on_devices(&proto, n, jobs, idx);
+    CpecanRealignedCigars *r = cpecan_malloc(sizeof(*r));
+    if (nDev == 1) {
+        *r = jobs[0].cigars;
+        return r;
+    }
+    memset(r, 0, sizeof(*r));
+    r->n = n;
+    gather_flat(r, nDev, idx, jobs, 0, 2);
+    if (wantAlignments) gather_flat(r, nDev, idx, jobs, 1, 3);
+    if (wantRawPairs) gather_flat(r, nDev, idx, jobs, 2, 3);
+    if (scoreKind >= 0) {
+        r->scores = cpecan_malloc((size_t) (n + 1) * sizeof(double));
+        for (int d = 0; d < nDev; d++) {
+            for (int64_t i = 0; i < jobs[d].n; i++) r->scores[idx[d][i]] = jobs[d].cigars.scores[i];
+            free(jobs[d].cigars.scores);
+        }
+    }
+    for (int d = 0; d < nDev; d++) free(idx[d]);
+    return r;
+}
+
+void cpecanRealignedCigars_destruct(CpecanRealignedCigars *r) {
+    if (r == NULL) return;
+    for (int which = 0; which < 3; which++) {
+        free(flat_list(r, which)->offsets);
+        free(flat_list(r, which)->values);
+    }
+    free(r->scores);
+    free(r);
+}
+
 /* the expectation totals of nDev finished expectation runs, summed: NCCL all-reduce across the devices when there are several (every
  * device then holds the sum; device 0's copy is read), else the one total as it is */
 static void add_expectations(Hmm *hmmExpectations, int64_t S, cpb_batch **batches, int nDev) {
@@ -698,22 +869,15 @@ typedef struct {
     int updateAnchors; /* 0: an expectation run; 1: realign and re-anchor (cpecanResidentBatch_updateAnchors) */
     float matchGamma;
 } ResidentRun;
-static void resident_check(int rc) {
-    if (rc == CPB_ERR_BAND) st_errAbort("%s: %s", PAIRWISE_ALIGNMENT_EXCEPTION_ID, cpb_last_error());
-    if (rc != CPB_OK) st_errAbort("cpecan: %s", cpb_last_error());
-}
 static void *resident_run(void *v) {
     ResidentRun *r = v;
     if (!r->updateAnchors) {
-        resident_check(cpb_batch_run(r->b, r->model, r->q, CPB_MODE_EXPECTATIONS));
+        engine_check(cpb_batch_run(r->b, r->model, r->q, CPB_MODE_EXPECTATIONS));
         return NULL;
     }
-    /* cPecanRealign's default steps for every alignment (job_finish: reweight, ordered chain), then the anchors job_prepare makes from the
-     * cigar it would write; no list leaves the device */
-    resident_check(cpb_batch_run(r->b, r->model, r->q, CPB_MODE_ALIGNED_PAIRS));
-    resident_check(cpb_batch_reweight_pairs(r->b, r->q->gapGamma));
-    resident_check(cpb_batch_ordered_chain(r->b, r->matchGamma));
-    resident_check(cpb_batch_anchors_from_alignments(r->b, r->q));
+    /* cPecanRealign's default steps, then the anchors job_prepare makes from the cigar it would write; no list leaves the device */
+    realign_steps(r->b, 0, r->model, r->q, r->matchGamma, NULL);
+    engine_check(cpb_batch_anchors_from_alignments(r->b, r->q));
     return NULL;
 }
 

@@ -224,6 +224,36 @@ stList **getReweightedAlignedPairsUsingAnchorsBatch(StateMachine *sM, int64_t n,
 void getAlignedPairsWithIndelsUsingAnchorsBatch(StateMachine *sM, int64_t n, const char *const *sX, const char *const *sY,
                                                 stList *const *anchorPairs, PairwiseAlignmentParameters *p, stList ***alignedPairs,
                                                 stList ***gapXPairs, stList ***gapYPairs, const bool *raggedLeft, const bool *raggedRight);
+/* What cPecanRealign does with every alignment, for n problems in one pass over the device set, with no list of tuples: an ALIGNED_PAIRS
+ * run, reweightAlignedPairs2 by p->gapGamma, filterPairwiseAlignmentToMakePairsOrdered at matchGamma (>= 0; above 1 no pair qualifies
+ * and every alignment is empty), and the cigar operations of the resulting alignment -- all on the device.  On request also one scoreBy*
+ * per problem (scoreKind one of CPECAN_SCORE_BY_*, or -1 for none), the alignments' (pInt, x, y) triples (wantAlignments) and list 0 of the
+ * run before reweighting, in the order getAlignedPairsUsingAnchorsBatch returns it (wantRawPairs).  Every result is a flat array with
+ * n + 1 offsets, at the problems' own indices; lists not asked for are NULL.  Operations are (type, length) int32 pairs, type
+ * PAIRWISE_MATCH, PAIRWISE_INDEL_X or PAIRWISE_INDEL_Y (cpecan/pairwiseAlignment.h), as cPecanRealign writes them: the gaps before each
+ * column, X before Y, adjacent columns merged into one match, the gaps after the last column.  Scores and triples are bit for bit those of
+ * the host functions (host/realign.c) on the lists getAlignedPairsUsingAnchorsBatch returns.  An invalid band aborts with
+ * PAIRWISE_ALIGNMENT_EXCEPTION, any other engine error with the engine's message.  Free the result with cpecanRealignedCigars_destruct. */
+#define CPECAN_SCORE_BY_IDENTITY 0 /* scoreByIdentity, and so on */
+#define CPECAN_SCORE_BY_IDENTITY_IGNORING_GAPS 1
+#define CPECAN_SCORE_BY_POSTERIOR_PROBABILITY 2
+#define CPECAN_SCORE_BY_POSTERIOR_PROBABILITY_IGNORING_GAPS 3
+typedef struct {
+    int64_t *offsets; /* n + 1, in entries: problem i's entries are [offsets[i], offsets[i + 1]) */
+    int32_t *values;
+} CpecanFlatList;
+typedef struct {
+    int64_t n;
+    CpecanFlatList ops;        /* 2 int32 per entry: (type, length) */
+    CpecanFlatList alignments; /* 3 int32 per entry: (pInt, x, y), x and y strictly increasing; NULL unless wantAlignments */
+    CpecanFlatList rawPairs;   /* 3 int32 per entry: (pInt, x, y); NULL unless wantRawPairs */
+    double *scores;            /* n, NULL if scoreKind is -1 */
+} CpecanRealignedCigars;
+CpecanRealignedCigars *getRealignedCigarsUsingAnchorsBatch(StateMachine *sM, int64_t n, const char *const *sX, const char *const *sY,
+                                                           stList *const *anchorPairs, PairwiseAlignmentParameters *p, const bool *raggedLeft,
+                                                           const bool *raggedRight, float matchGamma, int scoreKind, bool wantAlignments,
+                                                           bool wantRawPairs);
+void cpecanRealignedCigars_destruct(CpecanRealignedCigars *r);
 /* sums the expectations of all n problems into hmmExpectations (+=), as n calls of getExpectationsUsingAnchors would */
 void getExpectationsUsingAnchorsBatch(StateMachine *sM, Hmm *hmmExpectations, int64_t n, const char *const *sX, const char *const *sY,
                                       stList *const *anchorPairs, PairwiseAlignmentParameters *p, const bool *raggedLeft,

@@ -191,7 +191,8 @@ int cpb_batch_alignment_scores(cpb_batch *b, int64_t *scores);
  * returns, at tolerance 0 (same triples, same order, same double bits), what the host function of libcpecan.so (host/realign.c) returns on
  * the lists libcpecan.so would hand it.  Each decode call replaces the alignment list; cpb_batch_run clears it; cpb_batch_reweight_pairs
  * does not touch it.  Work arrays are processed in chunks that fit the scratch budget; a single pair that does not fit returns
- * CPB_ERR_MEMORY.  libcpecan.so and cPecanRealign still decode on the host.
+ * CPB_ERR_MEMORY.  libcpecan.so's cPecanRealign route (getRealignedCigarsUsingAnchorsBatch) decodes here: a run, reweighting, the
+ * ordered chain, scores and cigars, with only operations and scores crossing to the host.
  *
  * cpb_batch_ordered_chain: filterPairwiseAlignmentToMakePairsOrdered (impl/multipleAligner.c:945-972; realign.c:150-247) of list 0 as it
  *   stands (reweighted if cpb_batch_reweight_pairs was called, as cPecanRealign does): the heaviest chain, strictly increasing in x and y,
@@ -214,6 +215,21 @@ int cpb_batch_mea(cpb_batch *b, float gapGamma, int leftShift, double *scores);
 int64_t cpb_batch_alignments_count(const cpb_batch *b);
 int cpb_batch_fetch_alignments(const cpb_batch *b, int64_t *offsets, int32_t *triples);
 int cpb_batch_score_alignments(cpb_batch *b, int kind, double *scores);
+/*
+ * Cigar operations of the alignment list: per pair, the operations cPecanRealign writes for its alignment (pairs_to_alignment of
+ * host/cPecanRealign.c).  For columns (x_k, y_k), k < m, and (x_-1, y_-1) = (-1, -1): before every column an INDEL_X of
+ * x_k - x_{k-1} - 1 and an INDEL_Y of y_k - y_{k-1} - 1, each only if positive, then the column; adjacent columns merge into one MATCH;
+ * after the last column an INDEL_X of lX - x_{m-1} - 1 and an INDEL_Y of lY - y_{m-1} - 1, each only if positive.  An empty alignment is
+ * [INDEL_X lX][INDEL_Y lY] (each only if positive); a pair has at most 3m + 2 operations.
+ * cpb_batch_alignment_cigars builds them on the device; offsets receives n+1 entries, in operations.  cpb_batch_fetch_cigars copies them
+ * out: 2 int32 per operation, (type, length), grouped by pair in input order.  The cigar list belongs to the alignment list it was built
+ * from: every decode call and every cpb_batch_run discard it, cpb_batch_reweight_pairs and cpb_batch_anchors_from_alignments leave it.
+ * Building without an alignment list, or fetching without a cigar list, returns CPB_ERR_ARGUMENT; out of device memory returns
+ * CPB_ERR_MEMORY.  A build that returns an error leaves no cigar list (the previous one is gone too).
+ */
+enum { CPB_OP_MATCH = 0, CPB_OP_INDEL_X = 1, CPB_OP_INDEL_Y = 2 }; /* PAIRWISE_MATCH / _INDEL_X / _INDEL_Y of cpecan/pairwiseAlignment.h */
+int cpb_batch_alignment_cigars(cpb_batch *b, int64_t *offsets);
+int cpb_batch_fetch_cigars(const cpb_batch *b, int32_t *ops);
 /*
  * Re-anchoring from the alignment list, for the next run of the same batch (cPecanEm --updateTheBand): replaces every pair's anchors with
  * those its alignment gives (p->constraintDiagonalTrim, p->diagonalExpansion) -- exactly the triples cPecanRealign's job_prepare
