@@ -118,6 +118,8 @@ def _load():
                                    C.c_void_p, C.c_void_p, P(C.c_void_p)]
     L.cpb_batch_create_anchored.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                             P(CpbParams), P(C.c_void_p)]
+    L.cpb_batch_create_from_cigars.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, P(CpbParams), P(C.c_void_p)]
     L.cpb_batch_anchor_count.restype = C.c_int64
     L.cpb_batch_anchor_count.argtypes = [C.c_void_p]
     L.cpb_batch_fetch_anchors.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
@@ -140,6 +142,7 @@ def _load():
     L.cpb_batch_anchors_from_alignments.argtypes = [C.c_void_p, P(CpbParams)]
     L.cpb_batch_alignment_cigars.argtypes = [C.c_void_p, C.c_void_p]
     L.cpb_batch_fetch_cigars.argtypes = [C.c_void_p, C.c_void_p]
+    L.cpb_batch_alignments_from_cigars.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64]
     L.cpb_batch_device_triples.restype = C.c_void_p
     L.cpb_batch_device_triples.argtypes = [C.c_void_p, C.c_int]
     L.cpb_batch_fetch_expectations.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
@@ -281,6 +284,12 @@ def _ptr(a):
     return C.c_void_p(a.ctypes.data) if a is not None else None
 
 
+def _cigar_arrays(cigars):
+    """(offsets[n+1], ops[m, 2]) as Batch.alignment_cigars returns them -> contiguous int64 offsets and int32 operations"""
+    off, ops = cigars
+    return np.ascontiguousarray(off, dtype=np.int64), np.ascontiguousarray(np.asarray(ops).reshape(-1, 2), dtype=np.int32)
+
+
 class Batch:
     """n independent (seqX, seqY, anchors, ragged flags) problems resident on the device."""
 
@@ -318,6 +327,23 @@ class Batch:
         rl, rr = _ragged(raggedLeft), _ragged(raggedRight)
         h = C.c_void_p()
         _check(lib.cpb_batch_create_anchored(ctx.h, self.n, _ptr(bx), _ptr(xo), _ptr(by), _ptr(yo), _ptr(rl), _ptr(rr), C.byref(params), C.byref(h)))
+        self.h = h
+        return self
+
+    @classmethod
+    def from_cigars(cls, ctx, seqsX, seqsY, cigars, params, raggedLeft=None, raggedRight=None):
+        """A batch whose anchors the device builds from one forward-strand cigar per pair, cigars = (offsets[n+1] int64, ops[m, 2] int32
+        (type OP_*, length)) as alignment_cigars returns them: the anchors cPecanRealign's job_prepare keeps for that alignment under
+        params.constraintDiagonalTrim and params.diagonalExpansion"""
+        self = cls.__new__(cls)
+        self.ctx, self.n, self.S, self.h = ctx, len(seqsX), None, None
+        bx, xo = _pack_sequences(seqsX)
+        by, yo = _pack_sequences(seqsY)
+        oo, ops = _cigar_arrays(cigars)
+        rl, rr = _ragged(raggedLeft), _ragged(raggedRight)
+        h = C.c_void_p()
+        _check(lib.cpb_batch_create_from_cigars(ctx.h, self.n, _ptr(bx), _ptr(xo), _ptr(by), _ptr(yo), _ptr(oo), _ptr(ops) if len(ops) else None,
+                                                _ptr(rl), _ptr(rr), C.byref(params) if params is not None else None, C.byref(h)))
         self.h = h
         return self
 
@@ -407,6 +433,13 @@ class Batch:
         ops = np.zeros((max(m, 1), 2), dtype=np.int32)
         _check(lib.cpb_batch_fetch_cigars(self.h, C.c_void_p(ops.ctypes.data)))
         return off, ops[:m]
+
+    def alignments_from_cigars(self, cigars, trim=0):
+        """replaces the alignment list with every MATCH column at [trim, L - trim) of every pair's cigar (offsets[n+1], ops[m, 2] as
+        alignment_cigars returns them), x ascending, each weighed with its weight in list 0 of the last run (0 if it is not there): what
+        cPecanRealign --rescoreOriginalAlignment scores"""
+        oo, ops = _cigar_arrays(cigars)
+        _check(lib.cpb_batch_alignments_from_cigars(self.h, _ptr(oo), _ptr(ops) if len(ops) else None, int(trim)))
 
     def anchors_from_alignments(self, params):
         """replaces every pair's anchors with those its alignment gives (params.constraintDiagonalTrim, params.diagonalExpansion): the

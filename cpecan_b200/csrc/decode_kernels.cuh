@@ -12,6 +12,8 @@
  *                                                  realign.c:32-72, cPecanRealign.c:98-123)
  *   k_cigar_count / k_cigar_write                  the cigar operations cPecanRealign writes for an alignment (pairs_to_alignment,
  *                                                  cPecanRealign.c:98-123)
+ *   k_cigar_cols_count / k_cigar_cols_write<true>  the anchors job_prepare builds from an input cigar (realignJobs.h:149-173, realign.c:32-72)
+ *   k_cigar_cols_write<false> / k_cigar_weigh      an input cigar's columns weighed against list 0 (score_anchor_pairs, cPecanRealign.c:78-104)
  *
  * Pairs are processed in chunks whose work arrays fit the context's scratch budget (engine.cu); DecodePair says where a pair's inputs
  * and work arrays are.  Alignments are int32 (pInt, x, y) triples, 0-based, like the result lists.
@@ -523,6 +525,10 @@ __global__ void k_decode_scores(const int32_t *aln, const int64_t *off, int nPai
  * alignment is.  Work array of a pair of m triples: per triple the number of its run's triples before it, then its keep flag. */
 __host__ __device__ __forceinline__ int64_t reanchor_work_bytes(int64_t m) { return dec_round(4 * m); }
 
+/* columns_match of host/realignJobs.h on the kept bytes, which are already upper-cased: a column constrains the band iff its two bytes are
+ * equal and not N */
+__device__ __forceinline__ bool columns_match(uint8_t cx, uint8_t cy) { return cx == cy && cx != 'N'; }
+
 /* One warp per pair, O(1) per triple: a forward sweep finds every triple's run start (the last start at or before it: the chunk's ballot,
  * or the run carried in from the chunks before), a backward sweep its run end likewise; lens[pi] receives the number of kept columns. */
 __global__ void k_reanchor_count(const DecodePair *P, int nP, const int32_t *aln, const uint8_t *X, const uint8_t *Y, char *scratch, int32_t trim,
@@ -554,7 +560,7 @@ __global__ void k_reanchor_count(const DecodePair *P, int nP, const int32_t *aln
         if (k < m) {
             const int end = from != 0 ? k0 + __ffs(from) - 1 : carry;
             const uint8_t cx = sx[t[3 * k + 1]], cy = sy[t[3 * k + 2]];
-            keep = w[k] >= trim && end - k >= trim && cx == cy && cx != 'N';
+            keep = w[k] >= trim && end - k >= trim && columns_match(cx, cy);
             w[k] = keep;
         }
         kept += __popc(__ballot_sync(0xFFFFFFFFu, keep));
@@ -667,6 +673,115 @@ __global__ void k_cigar_write(const int32_t *aln, const int64_t *off, int nPairs
         if (start) out[w] = make_int2(CPB_OP_MATCH, (after != 0 ? k0 + __ffs(after) - 1 : next) - (k0 + lane));
         at -= __shfl_sync(0xFFFFFFFFu, s, 0);
         if (starts != 0) next = k0 + __ffs(starts) - 1;
+    }
+}
+
+/* ---- alignments given as cigar operations (cpb_batch_create_from_cigars, cpb_batch_alignments_from_cigars) ----
+ * A pair's operations, int32 (type, length) at ops[2 * opOff[pair]...], walk from (0, 0) to (lX, lY); the host has checked that they do.
+ * A MATCH of length L at (x, y) gives the columns (x + l, y + l) for l in [trim, L - trim), adjacent MATCH operations each trimmed
+ * (convertPairwiseForwardStrandAlignmentToAnchorPairs, realign.c:32-72).  One warp per pair, 32 operations per step, no work array:
+ * warp scans of the x and y advances and of the column counts give every operation its start and its first column, carried across
+ * steps; the step's columns are then dealt to the lanes 32 at a time, each lane finding its operation by a binary search over the
+ * lanes' first columns.  O(1) per operation and per column.  cigar_columns calls f(t, valid, x, y) on every lane for the columns
+ * t = t0 + lane of the step, counted from the pair's first column, and valid = false past the step's last. */
+template <class F>
+__device__ __forceinline__ void cigar_columns(const int32_t *ops, int64_t o0, int64_t o1, int32_t trim, int lane, F f) {
+    int32_t x0 = 0, y0 = 0, c0 = 0; /* where the step's first operation starts, and its first column */
+    for (int64_t k0 = o0; k0 < o1; k0 += 32) {
+        const int64_t k = k0 + lane;
+        int32_t type = CPB_OP_INDEL_X, len = 0;
+        if (k < o1) {
+            type = ops[2 * k];
+            len = ops[2 * k + 1];
+        }
+        const int32_t dx = type != CPB_OP_INDEL_Y ? len : 0, dy = type != CPB_OP_INDEL_X ? len : 0;
+        const int32_t c = type == CPB_OP_MATCH && (int64_t) len > 2 * (int64_t) trim ? len - 2 * trim : 0;
+        int32_t sx = dx, sy = dy, sc = c; /* inclusive scans */
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int32_t ux = __shfl_up_sync(0xFFFFFFFFu, sx, o), uy = __shfl_up_sync(0xFFFFFFFFu, sy, o), uc = __shfl_up_sync(0xFFFFFFFFu, sc, o);
+            if (lane >= o) {
+                sx += ux;
+                sy += uy;
+                sc += uc;
+            }
+        }
+        const int32_t x = x0 + sx - dx, y = y0 + sy - dy, first = sc - c; /* the operation's start, and its first column within the step */
+        const int32_t total = __shfl_sync(0xFFFFFFFFu, sc, 31);
+        for (int32_t t0 = 0; t0 < total; t0 += 32) {
+            const int32_t t = t0 + lane;
+            int lo = 0; /* the last operation whose first column is at or before t: one with columns when t < total */
+#pragma unroll
+            for (int s = 16; s > 0; s >>= 1) {
+                if (__shfl_sync(0xFFFFFFFFu, first, lo + s) <= t) lo += s;
+            }
+            const int32_t at = trim + (t - __shfl_sync(0xFFFFFFFFu, first, lo)); /* l of the column in its operation */
+            f(c0 + t, t < total, __shfl_sync(0xFFFFFFFFu, x, lo) + at, __shfl_sync(0xFFFFFFFFu, y, lo) + at);
+        }
+        x0 += __shfl_sync(0xFFFFFFFFu, sx, 31);
+        y0 += __shfl_sync(0xFFFFFFFFu, sy, 31);
+        c0 += total;
+    }
+}
+
+/* lens[pair] = the number of the pair's columns that columns_match keeps (the anchors job_prepare keeps) */
+__global__ void k_cigar_cols_count(const int32_t *ops, const int64_t *opOff, int nPairs, const int64_t *xOff, const int64_t *yOff, const uint8_t *X,
+                                   const uint8_t *Y, int32_t trim, int32_t *lens) {
+    const int pair = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (pair >= nPairs) return;
+    const uint8_t *sx = X + xOff[pair], *sy = Y + yOff[pair];
+    int32_t kept = 0;
+    cigar_columns(ops, opOff[pair], opOff[pair + 1], trim, lane,
+                  [&](int32_t, bool valid, int32_t x, int32_t y) { kept += __popc(__ballot_sync(0xFFFFFFFFu, valid && columns_match(sx[x], sy[y]))); });
+    if (lane == 0) lens[pair] = kept;
+}
+
+/* After the scan: ANCHORS, the kept columns as (x, y, expansion) at out[off[pair]...]; otherwise every column as (0, x, y), the
+ * alignment list before k_cigar_weigh.  x ascending. */
+template <bool ANCHORS>
+__global__ void k_cigar_cols_write(const int32_t *ops, const int64_t *opOff, int nPairs, const int64_t *xOff, const int64_t *yOff, const uint8_t *X,
+                                   const uint8_t *Y, int32_t trim, int32_t expansion, const int64_t *off, int32_t *out) {
+    const int pair = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (pair >= nPairs) return;
+    const uint8_t *sx = X + xOff[pair], *sy = Y + yOff[pair];
+    int64_t at = off[pair];
+    cigar_columns(ops, opOff[pair], opOff[pair + 1], trim, lane, [&](int32_t t, bool valid, int32_t x, int32_t y) {
+        if (ANCHORS) {
+            const bool keep = valid && columns_match(sx[x], sy[y]);
+            const unsigned keeps = __ballot_sync(0xFFFFFFFFu, keep);
+            if (keep) {
+                const int64_t o = at + __popc(keeps & ((1u << lane) - 1));
+                out[3 * o] = x;
+                out[3 * o + 1] = y;
+                out[3 * o + 2] = expansion;
+            }
+            at += __popc(keeps);
+        } else if (valid) {
+            out[3 * (at + t)] = 0;
+            out[3 * (at + t) + 1] = x;
+            out[3 * (at + t) + 2] = y;
+        }
+    });
+}
+
+/* One warp per pair, after k_cigar_cols_write<false>: every triple (w, x, y) of list 0 (l0Off: n+1 offsets) finds column x of the pair's
+ * alignment by a binary search (the columns' x are strictly increasing) and, if that column is (x, y), gives it weight w.  (x, y) is
+ * unique in list 0, so no two lanes write one column. */
+__global__ void k_cigar_weigh(const int32_t *list0, const int64_t *l0Off, int nPairs, const int64_t *alnOff, int32_t *aln) {
+    const int pair = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (pair >= nPairs) return;
+    int32_t *a = aln + 3 * alnOff[pair];
+    const int64_t m = alnOff[pair + 1] - alnOff[pair];
+    if (m == 0) return;
+    for (int64_t k = l0Off[pair] + lane; k < l0Off[pair + 1]; k += 32) {
+        const int32_t x = list0[3 * k + 1];
+        int64_t lo = 0, hi = m; /* the first column with x at or above */
+        while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (a[3 * mid + 1] < x) lo = mid + 1;
+            else hi = mid;
+        }
+        if (lo < m && a[3 * lo + 1] == x && a[3 * lo + 2] == list0[3 * k + 2]) a[3 * lo] = list0[3 * k];
     }
 }
 

@@ -407,35 +407,86 @@ struct cpb_batch {
 };
 
 static int find_anchors(cpb_batch *b, const CpbParams *p);
+static int cigar_anchors(cpb_batch *b, const int64_t *opOff, const int32_t *ops, const std::vector<int64_t> &cols, const CpbParams *p);
 
-/* cpb_batch_create and cpb_batch_create_anchored: the caller's anchors, or (anchorParams != nullptr) those find_anchors makes on the
- * device from the raw sequences before they are encoded */
+/* The checks of an input cigar list (n+1 offsets in operations, int32 (type, length) per operation) against the pairs' lengths, O(operations)
+ * and before any device work: offsets from 0 and non-decreasing, ops there if the offsets say it is not empty, every type one of CPB_OP_*
+ * and every length >= 0, and every pair's walk from (0, 0) ending at (lX, lY), as convertPairwiseForwardStrandAlignmentToAnchorPairs
+ * demands.  cols receives n+1 offsets of the pairs' MATCH columns at [trim, L - trim). */
+static int check_cigars(const char *call, int64_t n, const int64_t *xOff, const int64_t *yOff, const int64_t *opOff, const int32_t *ops, int64_t trim,
+                        std::vector<int64_t> &cols) {
+    if (opOff == nullptr || opOff[0] != 0) {
+        cpb_set_error("%s: %s", call, opOff == nullptr ? "no operation offsets" : "operation offsets must start at 0");
+        return CPB_ERR_ARGUMENT;
+    }
+    for (int64_t i = 0; i < n; i++) {
+        if (opOff[i + 1] < opOff[i]) {
+            cpb_set_error("%s: pair %lld: operation offsets decrease", call, (long long) i);
+            return CPB_ERR_ARGUMENT;
+        }
+    }
+    if (opOff[n] > 0 && ops == nullptr) {
+        cpb_set_error("%s: ops is NULL although the offsets say it is not empty", call);
+        return CPB_ERR_ARGUMENT;
+    }
+    cols.assign((size_t) n + 1, 0);
+    for (int64_t i = 0; i < n; i++) {
+        const int64_t lX = xOff[i + 1] - xOff[i], lY = yOff[i + 1] - yOff[i];
+        int64_t x = 0, y = 0, c = 0;
+        for (int64_t k = opOff[i]; k < opOff[i + 1] && x <= lX && y <= lY; k++) { /* past (lX, lY) it cannot come back: stop before a sum overflows */
+            const int32_t type = ops[2 * k], len = ops[2 * k + 1];
+            if (type < CPB_OP_MATCH || type > CPB_OP_INDEL_Y || len < 0) {
+                cpb_set_error("%s: pair %lld: operation %lld is (%d, %d); types are CPB_OP_MATCH, _INDEL_X, _INDEL_Y and lengths >= 0", call, (long long) i,
+                              (long long) (k - opOff[i]), type, len);
+                return CPB_ERR_ARGUMENT;
+            }
+            if (type != CPB_OP_INDEL_Y) x += len;
+            if (type != CPB_OP_INDEL_X) y += len;
+            if (type == CPB_OP_MATCH && len > 2 * trim) c += len - 2 * trim;
+        }
+        if (x != lX || y != lY) {
+            cpb_set_error("%s: pair %lld: the operations do not end at the ends of the sequences (%lld, %lld)", call, (long long) i, (long long) lX,
+                          (long long) lY);
+            return CPB_ERR_ARGUMENT;
+        }
+        cols[(size_t) i + 1] = cols[(size_t) i] + c;
+    }
+    return CPB_OK;
+}
+
+/* cpb_batch_create, cpb_batch_create_anchored and cpb_batch_create_from_cigars: the caller's anchors, those find_anchors makes on the
+ * device from the raw sequences before they are encoded (anchorParams != nullptr), or those cigar_anchors makes on the device from the
+ * caller's cigars after the sequences are encoded (opOff != nullptr, with anchorParams) */
 static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY, const int64_t *yOff,
-                        const int64_t *anchors, const int64_t *anchorOff, const CpbParams *anchorParams, const uint8_t *raggedLeft,
-                        const uint8_t *raggedRight, cpb_batch **out) {
+                        const int64_t *anchors, const int64_t *anchorOff, const CpbParams *anchorParams, const int64_t *opOff, const int32_t *ops,
+                        const uint8_t *raggedLeft, const uint8_t *raggedRight, cpb_batch **out) {
+    const char *call = opOff != nullptr ? "cpb_batch_create_from_cigars" : "cpb_batch_create";
     if (ctx == nullptr || out == nullptr || nPairs < 0 || xOff == nullptr || yOff == nullptr) {
-        cpb_set_error("cpb_batch_create: bad argument");
+        cpb_set_error("%s: bad argument", call);
         return CPB_ERR_ARGUMENT;
     }
     /* The kernels trust these arrays (region lengths and anchor coordinates are int32 on the device, the band builder's bisection
      * relies on x + y growing by at least 2 per anchor): everything the reference states as asserts (impl/pairwiseAligner.c:214-219)
      * is checked here, once, and reported with the index of the offending pair. */
     if (xOff[0] != 0 || yOff[0] != 0 || (anchorOff != nullptr && anchorOff[0] != 0)) {
-        cpb_set_error("cpb_batch_create: offset arrays must start at 0");
+        cpb_set_error("%s: offset arrays must start at 0", call);
         return CPB_ERR_ARGUMENT;
     }
     for (int64_t i = 0; i < nPairs; i++) {
         const int64_t lX = xOff[i + 1] - xOff[i], lY = yOff[i + 1] - yOff[i], nAi = anchorOff != nullptr ? anchorOff[i + 1] - anchorOff[i] : 0;
         if (lX < 0 || lY < 0 || nAi < 0 || lX + lY > (int64_t) 0x7FFFFF00) {
-            cpb_set_error("cpb_batch_create: pair %lld: offsets are not non-decreasing, or the sequences are too long (lengths %lld, %lld, %lld anchors)",
+            cpb_set_error("%s: pair %lld: offsets are not non-decreasing, or the sequences are too long (lengths %lld, %lld, %lld anchors)", call,
                           (long long) i, (long long) lX, (long long) lY, (long long) nAi);
             return CPB_ERR_ARGUMENT;
         }
     }
     if ((xOff[nPairs] > 0 && seqX == nullptr) || (yOff[nPairs] > 0 && seqY == nullptr) || (anchorOff != nullptr && anchorOff[nPairs] > 0 && anchors == nullptr)) {
-        cpb_set_error("cpb_batch_create: a sequence or anchor array is NULL although its offsets say it is not empty");
+        cpb_set_error("%s: a sequence or anchor array is NULL although its offsets say it is not empty", call);
         return CPB_ERR_ARGUMENT;
     }
+    std::vector<int64_t> cigarCols;
+    int rc = CPB_OK;
+    if (opOff != nullptr && (rc = check_cigars(call, nPairs, xOff, yOff, opOff, ops, anchorParams->constraintDiagonalTrim, cigarCols)) != CPB_OK) return rc;
     *out = nullptr;
     CUDA_TRY(cudaSetDevice(ctx->device));
     cpb_batch *b = new cpb_batch();
@@ -467,7 +518,6 @@ static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, cons
     memset(&b->stats, 0, sizeof(b->stats));
 
     const int64_t nx = xOff[nPairs], ny = yOff[nPairs];
-    int rc = CPB_OK;
     /* the strip kernels index symbols up to 32 positions outside a region without bounds tests: pad both ends with 'n' */
     if ((rc = b->symX.reserve(nx + 2 * kSymPad)) != CPB_OK || (rc = b->symY.reserve(ny + 2 * kSymPad)) != CPB_OK ||
         (rc = b->keptX.reserve(std::max<int64_t>(nx, 1))) != CPB_OK || (rc = b->keptY.reserve(std::max<int64_t>(ny, 1))) != CPB_OK)
@@ -477,13 +527,14 @@ static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, cons
     CUDA_TRY(cudaMemsetAsync(b->symY.p, 4, ny + 2 * kSymPad, st));
     if (nx > 0) CUDA_TRY(cudaMemcpyAsync(b->symX.as<uint8_t>() + kSymPad, seqX, nx, cudaMemcpyHostToDevice, st));
     if (ny > 0) CUDA_TRY(cudaMemcpyAsync(b->symY.as<uint8_t>() + kSymPad, seqY, ny, cudaMemcpyHostToDevice, st));
-    if (anchorParams != nullptr) {
+    if (anchorParams != nullptr && opOff == nullptr) {
         if ((rc = find_anchors(b, anchorParams)) != CPB_OK) return rc; /* reads the raw bytes: the soft mask is their case */
-    } else if ((rc = b->dAnchors.reserve(std::max<int64_t>(nA, 1) * 3 * sizeof(int32_t))) != CPB_OK) {
+    } else if (anchorParams == nullptr && (rc = b->dAnchors.reserve(std::max<int64_t>(nA, 1) * 3 * sizeof(int32_t))) != CPB_OK) {
         return rc;
     }
     if (nx > 0) k_encode<<<(unsigned) ((nx + 255) / 256), 256, 0, st>>>(b->symX.as<uint8_t>() + kSymPad, b->keptX.as<uint8_t>(), nx);
     if (ny > 0) k_encode<<<(unsigned) ((ny + 255) / 256), 256, 0, st>>>(b->symY.as<uint8_t>() + kSymPad, b->keptY.as<uint8_t>(), ny);
+    if (opOff != nullptr && (rc = cigar_anchors(b, opOff, ops, cigarCols, anchorParams)) != CPB_OK) return rc; /* reads the upper-cased bytes */
     if (anchorParams == nullptr && nA > 0) {
         /* int64 triples of the caller -> int32 triples, straight into a page-locked buffer that serves both the copy to the device
          * and the host-side region construction of every run; a few host threads share the conversion */
@@ -542,7 +593,7 @@ static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, cons
         }
         CUDA_TRY(cudaMemcpyAsync(b->dAnchors.p, b->anchors, bytes, cudaMemcpyHostToDevice, st));
     }
-    if (nPairs > 0) {
+    if (nPairs > 0 && opOff == nullptr) { /* cigar_anchors has installed its own */
         const size_t tab = (size_t) (nPairs + 1) * sizeof(int64_t);
         if ((rc = b->dPairTab.reserve(3 * tab)) != CPB_OK) return rc;
         CUDA_TRY(cudaMemcpyAsync(b->dPairTab.as<char>(), b->aOff.data(), tab, cudaMemcpyHostToDevice, st));
@@ -559,7 +610,7 @@ static int batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, cons
 extern "C" int cpb_batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY, const int64_t *yOff,
                                 const int64_t *anchors, const int64_t *anchorOff, const uint8_t *raggedLeft, const uint8_t *raggedRight,
                                 cpb_batch **out) {
-    return batch_create(ctx, nPairs, seqX, xOff, seqY, yOff, anchors, anchorOff, nullptr, raggedLeft, raggedRight, out);
+    return batch_create(ctx, nPairs, seqX, xOff, seqY, yOff, anchors, anchorOff, nullptr, nullptr, nullptr, raggedLeft, raggedRight, out);
 }
 
 extern "C" int cpb_batch_create_anchored(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY,
@@ -569,7 +620,22 @@ extern "C" int cpb_batch_create_anchored(cpb_context *ctx, int64_t nPairs, const
         cpb_set_error("cpb_batch_create_anchored: %s", p == nullptr ? "no parameters" : "constraintDiagonalTrim and diagonalExpansion must be in [0, 2^31)");
         return CPB_ERR_ARGUMENT;
     }
-    return batch_create(ctx, nPairs, seqX, xOff, seqY, yOff, nullptr, nullptr, p, raggedLeft, raggedRight, out);
+    return batch_create(ctx, nPairs, seqX, xOff, seqY, yOff, nullptr, nullptr, p, nullptr, nullptr, raggedLeft, raggedRight, out);
+}
+
+extern "C" int cpb_batch_create_from_cigars(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY,
+                                            const int64_t *yOff, const int64_t *opOff, const int32_t *ops, const uint8_t *raggedLeft,
+                                            const uint8_t *raggedRight, const CpbParams *p, cpb_batch **out) {
+    if (out != nullptr) *out = nullptr;
+    if (p == nullptr || p->constraintDiagonalTrim < 0 || p->constraintDiagonalTrim > 0x7FFFFFFF || p->diagonalExpansion < 0 || p->diagonalExpansion > 0x7FFFFFFF) {
+        cpb_set_error("cpb_batch_create_from_cigars: %s", p == nullptr ? "no parameters" : "constraintDiagonalTrim and diagonalExpansion must be in [0, 2^31)");
+        return CPB_ERR_ARGUMENT;
+    }
+    if (opOff == nullptr) {
+        cpb_set_error("cpb_batch_create_from_cigars: no operation offsets");
+        return CPB_ERR_ARGUMENT;
+    }
+    return batch_create(ctx, nPairs, seqX, xOff, seqY, yOff, nullptr, nullptr, p, opOff, ops, raggedLeft, raggedRight, out);
 }
 
 extern "C" int64_t cpb_batch_anchor_count(const cpb_batch *b) { return b != nullptr ? b->aOff[b->n] : 0; }
@@ -2428,7 +2494,7 @@ extern "C" int64_t cpb_batch_alignments_count(const cpb_batch *b) { return b != 
 
 extern "C" int cpb_batch_fetch_alignments(const cpb_batch *b, int64_t *offsets, int32_t *triples) {
     if (b == nullptr || !b->alnValid || offsets == nullptr || (triples == nullptr && b->alnOff[(size_t) b->n] > 0)) {
-        cpb_set_error("cpb_batch_fetch_alignments: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain or cpb_batch_mea after the run"
+        cpb_set_error("cpb_batch_fetch_alignments: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain, cpb_batch_mea or cpb_batch_alignments_from_cigars after the run"
                                                                                      : "bad argument");
         return CPB_ERR_ARGUMENT;
     }
@@ -2444,7 +2510,7 @@ extern "C" int cpb_batch_fetch_alignments(const cpb_batch *b, int64_t *offsets, 
 
 extern "C" int cpb_batch_score_alignments(cpb_batch *b, int kind, double *scores) {
     if (b == nullptr || !b->alnValid || kind < CPB_SCORE_IDENTITY || kind > CPB_SCORE_POSTERIOR_IGNORING_GAPS || (scores == nullptr && b->n > 0)) {
-        cpb_set_error("cpb_batch_score_alignments: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain or cpb_batch_mea after the run"
+        cpb_set_error("cpb_batch_score_alignments: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain, cpb_batch_mea or cpb_batch_alignments_from_cigars after the run"
                                                                                      : "bad argument (kind is one of CPB_SCORE_*)");
         return CPB_ERR_ARGUMENT;
     }
@@ -2469,7 +2535,7 @@ extern "C" int cpb_batch_score_alignments(cpb_batch *b, int kind, double *scores
 extern "C" int cpb_batch_alignment_cigars(cpb_batch *b, int64_t *offsets) {
     if (b != nullptr) b->cigValid = false; /* a build replaces the cigar list, also when it fails */
     if (b == nullptr || !b->alnValid || offsets == nullptr) {
-        cpb_set_error("cpb_batch_alignment_cigars: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain or cpb_batch_mea after the run"
+        cpb_set_error("cpb_batch_alignment_cigars: %s", b != nullptr && !b->alnValid ? "no alignments: call cpb_batch_ordered_chain, cpb_batch_mea or cpb_batch_alignments_from_cigars after the run"
                                                                                      : "bad argument");
         return CPB_ERR_ARGUMENT;
     }
@@ -2522,6 +2588,91 @@ extern "C" int cpb_batch_fetch_cigars(const cpb_batch *b, int32_t *ops) {
     return CPB_OK;
 }
 
+/* An alignment list from the caller's cigars: every MATCH column at [trim, L - trim) of every pair, x ascending, as (w, x, y) with w the
+ * weight of (x, y) in list 0 as it stands and 0 where list 0 has no such pair (score_anchor_pairs of cPecanRealign, in x order).  A decode
+ * call.  check_cigars gives the offsets, so there is no count pass: k_cigar_cols_write<false> writes the columns with weight 0 and
+ * k_cigar_weigh looks every triple of list 0 up among them. */
+extern "C" int cpb_batch_alignments_from_cigars(cpb_batch *b, const int64_t *opOff, const int32_t *ops, int64_t trim) {
+    if (b != nullptr) b->alnValid = b->cigValid = false; /* a decode call replaces the list, also when it is refused */
+    if (b == nullptr || (b->lastMode != CPB_MODE_ALIGNED_PAIRS && b->lastMode != CPB_MODE_ALIGNED_PAIRS_INDELS)) {
+        cpb_set_error("cpb_batch_alignments_from_cigars: no aligned-pair results in this batch");
+        return CPB_ERR_ARGUMENT;
+    }
+    if (trim < 0 || trim > 0x7FFFFFFF) {
+        cpb_set_error("cpb_batch_alignments_from_cigars: trim must be in [0, 2^31), not %lld", (long long) trim);
+        return CPB_ERR_ARGUMENT;
+    }
+    const int64_t n = b->n;
+    std::vector<int64_t> cols;
+    int rc = check_cigars("cpb_batch_alignments_from_cigars", n, b->xOff.data(), b->yOff.data(), opOff, ops, trim, cols);
+    if (rc != CPB_OK) return rc;
+    CUDA_TRY(cudaSetDevice(b->ctx->device));
+    cudaStream_t st = b->ctx->stream;
+    const int64_t nOps = opOff[n];
+    DevBuf dAlnOff, dX, dY, dL0Off, dOps, dOpOff;
+    for (DevBuf *d : { &dAlnOff, &dX, &dY, &dL0Off, &dOps, &dOpOff }) d->pool = &b->ctx->pool;
+    const size_t tabBytes = (size_t) (n + 1) * sizeof(int64_t);
+    if ((rc = upload_pair_tables(b, cols, dAlnOff, dX, dY)) != CPB_OK || (rc = dL0Off.reserve(tabBytes)) != CPB_OK || (rc = dOpOff.reserve(tabBytes)) != CPB_OK ||
+        (rc = dOps.reserve((size_t) std::max<int64_t>(nOps, 1) * 2 * sizeof(int32_t))) != CPB_OK ||
+        (rc = b->aln.reserve((size_t) std::max<int64_t>(cols[(size_t) n], 1) * 3 * sizeof(int32_t))) != CPB_OK) /* at most min(lX, lY) per pair */
+        return rc;
+    CUDA_TRY(cudaMemcpyAsync(dL0Off.p, b->pairOff[0].data(), tabBytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(dOpOff.p, opOff, tabBytes, cudaMemcpyHostToDevice, st));
+    if (nOps > 0) CUDA_TRY(cudaMemcpyAsync(dOps.p, ops, (size_t) nOps * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    int32_t *aln = b->aln.as<int32_t>();
+    k_cigar_cols_write<false><<<grid_of(n * 32, 256), 256, 0, st>>>(dOps.as<int32_t>(), dOpOff.as<int64_t>(), (int) n, dX.as<int64_t>(), dY.as<int64_t>(),
+                                                                     b->keptX.as<uint8_t>(), b->keptY.as<uint8_t>(), (int32_t) trim, 0, dAlnOff.as<int64_t>(), aln);
+    k_cigar_weigh<<<grid_of(n * 32, 256), 256, 0, st>>>(b->out[0].as<int32_t>(), dL0Off.as<int64_t>(), (int) n, dAlnOff.as<int64_t>(), aln);
+    b->stats.kernelLaunches += 2;
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    b->alnOff.swap(cols);
+    b->alnValid = true;
+    return CPB_OK;
+}
+
+/* Makes new anchors the batch's: tri, the device triples; tab, the device pair table (aOff, xOff, yOff; not taken when the batch has no
+ * pairs); aOff, their host offsets.  The triples are copied into a page-locked host buffer, which build_regions reads, and only then is
+ * anything swapped in: on an error the batch keeps its anchors.  The kept plan goes. */
+static int install_anchors(cpb_batch *b, const char *call, DevBuf &tri, DevBuf &tab, std::vector<int64_t> &aOff, int32_t expansion) {
+    cpb_context *ctx = b->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = b->n, nA = aOff[(size_t) n];
+    const size_t bytes = (size_t) (3 * nA) * sizeof(int32_t);
+    int32_t *host = nA > 0 ? static_cast<int32_t *>(ctx->pinned.take(bytes)) : nullptr;
+    std::vector<int32_t> own;
+    if (nA > 0 && host == nullptr) {
+        own.resize((size_t) (3 * nA));
+        host = own.data();
+    }
+    cudaError_t e = nA > 0 ? cudaMemcpyAsync(host, tri.p, bytes, cudaMemcpyDeviceToHost, st) : cudaSuccess;
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) {
+        if (host != nullptr && own.empty()) ctx->pinned.give(host);
+        cpb_set_error("%s: %s", call, cudaGetErrorString(e));
+        return CPB_ERR_CUDA;
+    }
+    /* everything is built: swap */
+    if (b->anchors != nullptr && b->anchorsOwn.empty()) ctx->pinned.give(b->anchors);
+    b->anchors = host;
+    b->anchorsOwn.swap(own);
+    b->aOff.swap(aOff);
+    b->dAnchors.release();
+    b->dAnchors.adopt(tri);
+    if (n > 0) {
+        b->dPairTab.release();
+        b->dPairTab.adopt(tab);
+    }
+    b->oddExpansionPair = -1;
+    if (expansion & 1) {
+        for (int64_t i = 0; i < n && b->oddExpansionPair < 0; i++)
+            if (b->aOff[(size_t) i + 1] > b->aOff[(size_t) i]) b->oddExpansionPair = i;
+    }
+    b->planValid = false;
+    return CPB_OK;
+}
+
 /* The anchors job_prepare builds from the cigar of every pair's alignment (k_reanchor_count / k_reanchor_write), built into new buffers --
  * device triples, the device pair table, the page-locked host copy that build_regions reads -- which replace the batch's only once all of
  * them are there.  Only planning reads the anchors (k_split_flags, build_regions, k_band), so the lists, the alignment list and everything
@@ -2534,7 +2685,7 @@ extern "C" int cpb_batch_anchors_from_alignments(cpb_batch *b, const CpbParams *
         return CPB_ERR_ARGUMENT;
     }
     if (!b->alnValid) {
-        cpb_set_error("cpb_batch_anchors_from_alignments: no alignments: call cpb_batch_ordered_chain or cpb_batch_mea after the run");
+        cpb_set_error("cpb_batch_anchors_from_alignments: no alignments: call cpb_batch_ordered_chain, cpb_batch_mea or cpb_batch_alignments_from_cigars after the run");
         return CPB_ERR_ARGUMENT;
     }
     const int64_t n = b->n;
@@ -2575,40 +2726,42 @@ extern "C" int cpb_batch_anchors_from_alignments(cpb_batch *b, const CpbParams *
         nullptr, tab.as<int64_t>(), aOff);
     if (rc != CPB_OK) return rc;
     if (n > 0) CUDA_TRY(cudaMemcpyAsync(tab.as<char>() + tabBytes, b->dPairTab.as<char>() + tabBytes, 2 * tabBytes, cudaMemcpyDeviceToDevice, st));
-    const int64_t nA = aOff[(size_t) n];
-    const size_t bytes = (size_t) (3 * nA) * sizeof(int32_t);
-    int32_t *host = nA > 0 ? static_cast<int32_t *>(ctx->pinned.take(bytes)) : nullptr;
-    std::vector<int32_t> own;
-    if (nA > 0 && host == nullptr) {
-        own.resize((size_t) (3 * nA));
-        host = own.data();
-    }
-    cudaError_t e = nA > 0 ? cudaMemcpyAsync(host, tri.p, bytes, cudaMemcpyDeviceToHost, st) : cudaSuccess;
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e == cudaSuccess) e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        if (host != nullptr && own.empty()) ctx->pinned.give(host);
-        cpb_set_error("cpb_batch_anchors_from_alignments: %s", cudaGetErrorString(e));
-        return CPB_ERR_CUDA;
-    }
-    /* everything is built: swap */
-    if (b->anchors != nullptr && b->anchorsOwn.empty()) ctx->pinned.give(b->anchors);
-    b->anchors = host;
-    b->anchorsOwn.swap(own);
-    b->aOff.swap(aOff);
-    b->dAnchors.release();
-    b->dAnchors.adopt(tri);
-    if (n > 0) {
-        b->dPairTab.release();
-        b->dPairTab.adopt(tab);
-    }
-    b->oddExpansionPair = -1;
-    if (expansion & 1) {
-        for (int64_t i = 0; i < n && b->oddExpansionPair < 0; i++)
-            if (b->aOff[(size_t) i + 1] > b->aOff[(size_t) i]) b->oddExpansionPair = i;
-    }
-    b->planValid = false;
-    return CPB_OK;
+    return install_anchors(b, "cpb_batch_anchors_from_alignments", tri, tab, aOff, expansion);
+}
+
+/* The anchors job_prepare builds from the caller's cigars (k_cigar_cols_count / k_cigar_cols_write<true>), after check_cigars (cols: the
+ * pairs' columns before the byte filter, which bound the kept ones) and k_encode, into a batch that has no anchors yet.  No work array:
+ * the counts are scanned over all pairs at once, into the new pair table. */
+static int cigar_anchors(cpb_batch *b, const int64_t *opOff, const int32_t *ops, const std::vector<int64_t> &cols, const CpbParams *p) {
+    cpb_context *ctx = b->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = b->n, nOps = opOff[n];
+    DevBuf dOps, dOpOff, lens, tiles, tri, tab; /* tab: the new pair table (aOff, xOff, yOff) */
+    for (DevBuf *d : { &dOps, &dOpOff, &lens, &tiles, &tri, &tab }) d->pool = &ctx->pool;
+    const size_t tabBytes = (size_t) (n + 1) * sizeof(int64_t);
+    int rc;
+    if ((rc = dOps.reserve((size_t) std::max<int64_t>(nOps, 1) * 2 * sizeof(int32_t))) != CPB_OK || (rc = dOpOff.reserve(tabBytes)) != CPB_OK ||
+        (rc = lens.reserve((size_t) std::max<int64_t>(n, 1) * sizeof(int32_t))) != CPB_OK ||
+        (rc = tiles.reserve((size_t) ((n + SCAN_TILE - 1) / SCAN_TILE + 1) * 8)) != CPB_OK ||
+        (rc = tri.reserve((size_t) std::max<int64_t>(cols[(size_t) n], 1) * 3 * sizeof(int32_t))) != CPB_OK || (rc = tab.reserve(3 * tabBytes)) != CPB_OK)
+        return rc;
+    int64_t *dA = tab.as<int64_t>(), *dX = dA + n + 1, *dY = dX + n + 1;
+    if (nOps > 0) CUDA_TRY(cudaMemcpyAsync(dOps.p, ops, (size_t) nOps * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(dOpOff.p, opOff, tabBytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(dX, b->xOff.data(), tabBytes, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(dY, b->yOff.data(), tabBytes, cudaMemcpyHostToDevice, st));
+    const uint8_t *kx = b->keptX.as<uint8_t>(), *ky = b->keptY.as<uint8_t>();
+    const int32_t trim = (int32_t) p->constraintDiagonalTrim, expansion = (int32_t) p->diagonalExpansion;
+    if (n > 0) k_cigar_cols_count<<<grid_of(n * 32, 256), 256, 0, st>>>(dOps.as<int32_t>(), dOpOff.as<int64_t>(), (int) n, dX, dY, kx, ky, trim, lens.as<int32_t>());
+    scan_counts(st, lens.as<int32_t>(), n, 0, tiles.as<int64_t>(), dA);
+    if (n > 0)
+        k_cigar_cols_write<true><<<grid_of(n * 32, 256), 256, 0, st>>>(dOps.as<int32_t>(), dOpOff.as<int64_t>(), (int) n, dX, dY, kx, ky, trim, expansion, dA,
+                                                                        tri.as<int32_t>());
+    std::vector<int64_t> aOff((size_t) n + 1);
+    CUDA_TRY(cudaMemcpyAsync(aOff.data(), dA, tabBytes, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    CUDA_TRY(cudaGetLastError());
+    return install_anchors(b, "cpb_batch_create_from_cigars", tri, tab, aOff, expansion);
 }
 
 extern "C" int cpb_batch_fetch_expectations(cpb_batch *b, double *perPair, double *total) {

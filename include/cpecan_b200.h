@@ -135,6 +135,21 @@ int cpb_batch_create(cpb_context *ctx, int64_t nPairs, const char *seqX, const i
 int cpb_batch_create_anchored(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY,
                               const int64_t *yOff, const uint8_t *raggedLeft, const uint8_t *raggedRight, const CpbParams *p,
                               cpb_batch **out);
+/* As cpb_batch_create, with every pair's anchors built on the device from a cigar: exactly the triples cPecanRealign's job_prepare
+ * (host/realignJobs.h) keeps for an input alignment.  opOff: n+1 offsets (in operations); ops: 2 int32 per operation, (CPB_OP_*, length),
+ * the format cpb_batch_fetch_cigars gives out.  Each pair's operations are a forward-strand alignment of its whole X with its whole Y,
+ * walked from (0, 0): a MATCH of length L at (x, y) gives the columns (x + l, y + l), l in [trim, L - trim), none if L <= 2 trim, with
+ * trim = p->constraintDiagonalTrim and adjacent MATCH operations trimmed separately (convertPairwiseForwardStrandAlignmentToAnchorPairs);
+ * a column is kept, as (x, y, p->diagonalExpansion), iff its two bytes are equal after toupper and not N.  Per pair x ascending.  Only the
+ * sequences, the offsets and the operations are copied to the device.  The batch then is the one cpb_batch_create makes from those
+ * anchors: cpb_batch_anchor_count / cpb_batch_fetch_anchors return them and every run gives the same outputs (an odd expansion is refused
+ * by dynamicAnchorExpansion runs, as there).  CPB_ERR_ARGUMENT, checked before any device work: p NULL, trim or expansion outside
+ * [0, 2^31), opOff NULL, not starting at 0 or decreasing, ops NULL while opOff says it is not empty, a type outside CPB_OP_* or a negative
+ * length, a pair whose operations do not end at (lX, lY), and everything cpb_batch_create checks of the sequences.  On any error *out is
+ * NULL and nothing stays allocated. */
+int cpb_batch_create_from_cigars(cpb_context *ctx, int64_t nPairs, const char *seqX, const int64_t *xOff, const char *seqY,
+                                 const int64_t *yOff, const int64_t *opOff, const int32_t *ops, const uint8_t *raggedLeft,
+                                 const uint8_t *raggedRight, const CpbParams *p, cpb_batch **out);
 /* the anchors a batch holds, whoever made them: n+1 offsets (in triples), int64 (x, y, expansion) triples */
 int64_t cpb_batch_anchor_count(const cpb_batch *b);
 int cpb_batch_fetch_anchors(const cpb_batch *b, int64_t *offsets, int64_t *triples);
@@ -205,6 +220,7 @@ int cpb_batch_alignment_scores(cpb_batch *b, int64_t *scores);
  * cpb_batch_score_alignments: per pair, scoreByIdentity, scoreByIdentityIgnoringGaps, scoreByPosteriorProbability or
  *   scoreByPosteriorProbabilityIgnoringGaps (impl/pairwiseAligner.c:1562-1597; realign.c:113-148) of its alignment; the two "ignoring
  *   gaps" forms are NaN for an empty alignment, as on the host.  Letters compare case-blind, N never matches.
+ * cpb_batch_alignments_from_cigars (below) is a decode call too.
  * Fetching or scoring before a decode call, a decode after an EXPECTATIONS or FORWARD run, and gammas or kind out of range return
  * CPB_ERR_ARGUMENT.  A decode call that returns an error, for whatever reason, leaves no alignment list (the previous one is gone too).
  * cpb_batch_alignments_count is 0 while there is no alignment list.
@@ -236,13 +252,26 @@ int cpb_batch_fetch_cigars(const cpb_batch *b, int32_t *ops);
  * (host/realignJobs.h) builds from the cigar cPecanRealign writes for that alignment.  The alignment's maximal diagonal runs are the cigar's
  * match operations; a run of length L gives its columns at positions [trim, L - trim) (convertPairwiseForwardStrandAlignmentToAnchorPairs,
  * mismatched columns counted); each becomes (x, y, diagonalExpansion) and is kept iff its two bytes are equal after toupper and not N.
- * Per pair x ascending.  Needs an alignment list (cpb_batch_ordered_chain or cpb_batch_mea); without one, with p NULL, or with a trim or
+ * Per pair x ascending.  Needs an alignment list (from a decode call); without one, with p NULL, or with a trim or
  * expansion outside [0, 2^31) it returns CPB_ERR_ARGUMENT.  All or nothing: on any error, CPB_ERR_MEMORY for a pair whose work array does
  * not fit the scratch budget included, the batch keeps its anchors.  On success cpb_batch_anchor_count / cpb_batch_fetch_anchors return the
  * new anchors and the next cpb_batch_run plans anew (planReused 0); the lists of the last run, the alignment list and its scores stay as
  * they were.  The batch then runs as one cpb_batch_create makes from the fetched anchors.
  */
 int cpb_batch_anchors_from_alignments(cpb_batch *b, const CpbParams *p);
+/*
+ * An alignment list from cigars, weighed against the posteriors: per pair every column of every MATCH operation at [trim, L - trim) of its
+ * cigar (opOff, ops as for cpb_batch_create_from_cigars, checked the same way against the batch's lengths), with no byte filter, x
+ * ascending, as (w, x, y): w is the weight of (x, y) in list 0 as it stands (reweighted if cpb_batch_reweight_pairs ran), 0 where list 0
+ * has no such pair -- score_anchor_pairs of cPecanRealign --rescoreOriginalAlignment, in x order.  A decode call: it replaces the alignment
+ * list and discards the cigar list; it needs an ALIGNED_PAIRS or ALIGNED_PAIRS_INDELS run, and returns CPB_ERR_ARGUMENT before any run,
+ * after an EXPECTATIONS or FORWARD run, for a trim outside [0, 2^31) and for operations cpb_batch_create_from_cigars would refuse.
+ * cpb_batch_score_alignments, cpb_batch_alignment_cigars, cpb_batch_fetch_alignments and cpb_batch_anchors_from_alignments then work as
+ * after any decode.  cpb_batch_create_from_cigars with cPecanRealign's parameters, an ALIGNED_PAIRS run, this call with the same
+ * operations and trim = p->constraintDiagonalTrim, then scores and cigars give what cPecanRealign --rescoreOriginalAlignment
+ * [--rescoreBy*] writes, without the posteriors leaving the device.
+ */
+int cpb_batch_alignments_from_cigars(cpb_batch *b, const int64_t *opOff, const int32_t *ops, int64_t trim);
 /* device pointers of the same (valid until the next run / destroy) */
 const int32_t *cpb_batch_device_triples(const cpb_batch *b, int list);
 /* EXPECTATIONS mode: perPair (may be NULL) receives n * CPB_HMM_LEN(S) doubles, total receives CPB_HMM_LEN(S) doubles
