@@ -5,8 +5,8 @@
  *
  *   k_chain_sort / k_chain_sweep / k_chain_write   filterPairwiseAlignmentToMakePairsOrdered   realign.c:150-247
  *   k_ref_order (k_ref_emit)                       cpb_batch_fetch_pairs_reference_order (the order libcpecan.so hands lists over in)
- *   k_mea_gaps / k_mea                             getMaximalExpectedAccuracyPairwiseAlignment realign.c:249-326
- *   k_decode_emit<SHIFT>                           its traceback, and leftShiftAlignment        realign.c:313-318, :330-356
+ *   k_mea_gaps / k_mea_summaries / k_mea           getMaximalExpectedAccuracyPairwiseAlignment realign.c:249-371
+ *   k_decode_emit<SHIFT>                           its traceback, and leftShiftAlignment        realign.c:353-358, :375-401
  *   k_decode_scores                                scoreByIdentity ... IgnoringGaps             realign.c:113-148
  *   k_reanchor_count / k_reanchor_write            the anchors job_prepare builds from the cigar of an alignment (realignJobs.h:149-173,
  *                                                  realign.c:32-72, cPecanRealign.c:98-123)
@@ -216,9 +216,14 @@ __global__ void k_chain_write(const DecodePair *P, int nP, char *scratch, const 
 
 /* ---- maximal expected accuracy ----
  * Work arrays of a pair with m triples in list 0: list 0 in the reference's order, the DP's scores, back pointers and isHigh flags
- * (m + 1 entries: the last is the virtual pair at (lX, lY)), and the cumulative gap weights of X and Y. */
+ * (m + 1 entries: the last is the virtual pair at (lX, lY)), the cumulative gap weights of X and Y, and the least (x, y) of every aligned
+ * chunk of 32 and block of 1024 reference-ordered triples (k_mea_summaries; what lets k_mea skip ranges that hold no predecessor). */
+__host__ __device__ __forceinline__ int64_t mea_chunks(int64_t m) { return (m + 31) >> 5; }
+__host__ __device__ __forceinline__ int64_t mea_blocks(int64_t m) { return (mea_chunks(m) + 31) >> 5; }
+
 __host__ __device__ __forceinline__ int64_t mea_work_bytes(int64_t m, int64_t lX, int64_t lY) {
-    return dec_round(12 * m) + dec_round(8 * (m + 1)) + dec_round(4 * (m + 1)) + dec_round(m + 1) + dec_round(8 * lX) + dec_round(8 * lY);
+    return dec_round(12 * m) + dec_round(8 * (m + 1)) + dec_round(4 * (m + 1)) + dec_round(m + 1) + dec_round(8 * lX) + dec_round(8 * lY) +
+           dec_round(8 * mea_chunks(m)) + dec_round(8 * mea_blocks(m));
 }
 
 struct MeaWork {
@@ -227,6 +232,7 @@ struct MeaWork {
     int32_t *back;
     uint8_t *high;
     long long *cumX, *cumY;
+    int2 *chunk, *block; /* least (x, y) of triples 32c ... 32c + 31, and of 1024b ... 1024b + 1023 */
 };
 
 __device__ __forceinline__ MeaWork mea_work(char *base, int64_t m, int64_t lX, int64_t lY) {
@@ -242,6 +248,10 @@ __device__ __forceinline__ MeaWork mea_work(char *base, int64_t m, int64_t lX, i
     w.cumX = reinterpret_cast<long long *>(base);
     base += dec_round(8 * lX);
     w.cumY = reinterpret_cast<long long *>(base);
+    base += dec_round(8 * lY);
+    w.chunk = reinterpret_cast<int2 *>(base);
+    base += dec_round(8 * mea_chunks(m));
+    w.block = reinterpret_cast<int2 *>(base);
     return w;
 }
 
@@ -338,6 +348,64 @@ __global__ void k_mea_gaps(const DecodePair *P, int nP, const int32_t *list1, co
     }
 }
 
+__device__ __forceinline__ int2 mea_least(int2 v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        v.x = min(v.x, __shfl_xor_sync(0xFFFFFFFFu, v.x, o));
+        v.y = min(v.y, __shfl_xor_sync(0xFFFFFFFFu, v.y, o));
+    }
+    return v;
+}
+
+/* One warp per pair, after k_ref_order: the least (x, y) of every chunk of 32 reference-ordered triples, then of every block of 32 chunks */
+__global__ void k_mea_summaries(const DecodePair *P, int nP, char *scratch) {
+    const int pi = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
+    if (pi >= nP) return;
+    const DecodePair D = P[pi];
+    MeaWork W = mea_work(scratch + D.work, D.n0, D.lX, D.lY);
+    const int m = D.n0, nChunks = (int) mea_chunks(m), nBlocks = (int) mea_blocks(m);
+    for (int c = 0; c < nChunks; c++) {
+        const int j = (c << 5) + lane;
+        const int2 v = mea_least(j < m ? make_int2(W.ref[j].y, W.ref[j].z) : make_int2(INT32_MAX, INT32_MAX));
+        if (lane == 0) W.chunk[c] = v;
+    }
+    __syncwarp();
+    for (int b = 0; b < nBlocks; b++) {
+        const int c = (b << 5) + lane;
+        const int2 v = mea_least(c < nChunks ? W.chunk[c] : make_int2(INT32_MAX, INT32_MAX));
+        if (lane == 0) W.block[b] = v;
+    }
+}
+
+/* may the triples a summary covers hold a predecessor of (x, y)? */
+__device__ __forceinline__ bool mea_may_precede(int2 least, int64_t x, int64_t y) { return least.x < x && least.y < y; }
+
+/* The highest chunk at or below c that may hold a predecessor of (x, y), or -1; the same on every lane.  A chunk whose least x or least y
+ * is not below the pair's holds none, and its triples would all be passed over by the scan.  The chunk c itself is tried first (the common
+ * case inside a block: one broadcast load).  Then the lanes test the 32 block summaries of c's group of 32 blocks (the blocks above c's
+ * excluded), and the highest block that may hold one has its 32 chunk summaries tested at once (the chunks above c excluded); a group or a
+ * block without a hit is passed whole, so the walk over the later blocks of a region costs one step per 32 768 triples. */
+__device__ __forceinline__ int mea_next_chunk(const MeaWork &W, int c, int64_t x, int64_t y, int lane) {
+    if (c < 0) return -1;
+    if (mea_may_precede(W.chunk[c], x, y)) return c;
+    c--;
+    while (c >= 0) {
+        const int b = c >> 5, g = b & ~31;
+        unsigned hit = __ballot_sync(0xFFFFFFFFu, g + lane <= b && mea_may_precede(W.block[g + lane], x, y));
+        if (hit == 0) {
+            c = (g << 5) - 1;
+            continue;
+        }
+        const int hb = g + 31 - __clz(hit);
+        if (hb < b) c = (hb << 5) + 31;
+        const int k = hb << 5;
+        hit = __ballot_sync(0xFFFFFFFFu, k + lane <= c && mea_may_precede(W.chunk[k + lane], x, y));
+        if (hit != 0) return k + 31 - __clz(hit);
+        c = k - 1;
+    }
+    return -1;
+}
+
 /* gap_weight of realign.c: the weights of positions start .. start + length - 1 */
 __device__ __forceinline__ long long mea_gap(const long long *cum, int64_t start, int64_t length) {
     return length == 0 ? 0 : cum[start + length - 1] - (start > 0 ? cum[start - 1] : 0);
@@ -348,9 +416,11 @@ __device__ __forceinline__ float mea_gap_term(long long g, float gamma) { return
 
 /* One warp per pair: the DP of getMaximalExpectedAccuracyPairwiseAlignment over the reference-ordered list, sequential in i.  For pair i
  * the host scans j = i-1, i-2, ... keeping the first strictly larger truncated candidate among the valid predecessors (x2 < x, y2 < y),
- * and stops after the first valid one with isHigh set.  Here lanes take j = j0 - lane, 32 at a time: the cutoff is the nearest valid isHigh
- * lane (included), and the maximum over valid lanes up to it by (candidate larger, then j larger) is what the strict-> scan selects; it
- * replaces the running score only if strictly larger.  scores[pi] receives maxScore, lens[pi] the length of the traceback. */
+ * and stops after the first valid one with isHigh set.  Here the warp takes the aligned chunks of 32 triples from the one holding i - 1
+ * down, lane l the triple 32c + 31 - l (those at or above i are not valid), and skips every chunk that holds no valid predecessor
+ * (mea_next_chunk): such a chunk changes nothing in the scan.  In a loaded chunk the cutoff is the nearest valid isHigh lane (included),
+ * and the maximum over valid lanes up to it by (candidate larger, then j larger) is what the strict-> scan selects; it replaces the running
+ * score only if strictly larger.  scores[pi] receives maxScore, lens[pi] the length of the traceback. */
 __global__ void k_mea(const DecodePair *P, int nP, char *scratch, float gamma, double *scores, int32_t *lens) {
     const int pi = (int) (((int64_t) blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
     if (pi >= nP) return;
@@ -371,11 +441,11 @@ __global__ void k_mea(const DecodePair *P, int nP, char *scratch, float gamma, d
         /* w + (gx + gy) * gamma: all float, then widened */
         double score = (double) __fadd_rn(__ll2float_rn(w), mea_gap_term(mea_gap(W.cumX, 0, x) + mea_gap(W.cumY, 0, y), gamma));
         int from = -1;
-        for (int j0 = i - 1; j0 >= 0; j0 -= 32) {
-            const int j = j0 - lane;
+        for (int c = mea_next_chunk(W, i > 0 ? (i - 1) >> 5 : -1, x, y, lane); c >= 0; c = mea_next_chunk(W, c - 1, x, y, lane)) {
+            const int j = (c << 5) + 31 - lane;
             bool valid = false, isHigh = false;
             double s = 0.0;
-            if (j >= 0) {
+            if (j < i) {
                 const int3 q = W.ref[j];
                 const int64_t x2 = q.y, y2 = q.z;
                 if (x2 < x && y2 < y) {

@@ -2444,10 +2444,11 @@ extern "C" int cpb_batch_mea(cpb_batch *b, float gapGamma, int leftShift, double
         b, "cpb_batch_mea", P, [](const DecodePair &D) { return mea_work_bytes(D.n0, D.lX, D.lY); },
         [&](DecodeChunk &c) {
             k_ref_order<<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, l0, T.shift, T.block0, T.blocks, T.from, c.work);
+            k_mea_summaries<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, c.work);
             k_mea_gaps<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, l1, l2, c.work);
             k_mea<<<grid_of((int64_t) c.nC * 32, 256), 256, 0, st>>>(c.desc, c.nC, c.work, gapGamma, c.scores, c.lens);
             if (leftShift) k_decode_emit<true><<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, c.work, kx, ky, c.lens, nullptr, nullptr);
-            return leftShift ? 4 : 3;
+            return leftShift ? 5 : 4;
         },
         [&](DecodeChunk &c) {
             if (leftShift) k_decode_emit<true><<<grid_of(c.nC, 128), 128, 0, st>>>(c.desc, c.nC, c.work, kx, ky, c.lens, c.off, b->aln.as<int32_t>());

@@ -432,6 +432,9 @@ typedef struct {
     /* getRealignedCigarsUsingAnchorsBatch */
     int realign, scoreKind, wantAlignments, wantRawPairs;
     float matchGamma;
+    /* getShiftedMEAAlignmentBatch: the left-shifted MEA into lists[0], each alignmentScore into alignmentScores (if not NULL) */
+    int shiftedMea;
+    double *alignmentScores;
     /* results, in the caller's indexing */
     stList **lists[3];
     double *logProbs;
@@ -533,6 +536,29 @@ static void device_realign(DeviceJob *j, cpb_batch *b, const char *const *sX, co
     }
 }
 
+/* getShiftedMEAAlignment for this device's problems after their ALIGNED_PAIRS_INDELS run: MEA with p->gapGamma and leftShiftAlignment on
+ * the device (cpb_batch_mea), the alignments' tuples cut from one slab per problem */
+static void device_shifted_mea(DeviceJob *j, cpb_batch *b) {
+    const int64_t n = j->n;
+    double *scores = cpecan_malloc((size_t) (n + 1) * sizeof(double));
+    engine_check(cpb_batch_mea(b, j->p->gapGamma, 1, scores));
+    int64_t *off = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t));
+    int32_t *tri = cpecan_malloc((size_t) (3 * cpb_batch_alignments_count(b) + 3) * sizeof(int32_t));
+    engine_check(cpb_batch_fetch_alignments(b, off, tri));
+    stList **mine = cpecan_malloc((size_t) (n + 1) * sizeof(stList *));
+    ListJob job = { mine, off, tri };
+    cpecan_parallel_for(n, off, lists_range, &job);
+    for (int64_t i = 0; i < n; i++) {
+        const int64_t g = j->idx != NULL ? j->idx[i] : i;
+        j->lists[0][g] = mine[i];
+        if (j->alignmentScores != NULL) j->alignmentScores[g] = scores[i];
+    }
+    free(mine);
+    free(tri);
+    free(off);
+    free(scores);
+}
+
 static void *device_job(void *v) {
     DeviceJob *j = v;
     const int64_t n = j->n;
@@ -565,10 +591,13 @@ static void *device_job(void *v) {
         if (cpb_batch_create(j->ctx, k.n, k.seqX, k.xOff, k.seqY, k.yOff, k.anchors, k.aOff, k.rl, k.rr, &b) != CPB_OK) st_errAbort("cpecan: %s", cpb_last_error());
         if (j->realign) device_realign(j, b, sX, sY);
     } else {
-        b = run(j->ctx, &k, j->sM, j->p, j->mode, j->reweight ? NULL : &sinks); /* (reweighting rewrites the list on the device after the run) */
+        /* (reweighting rewrites the list on the device after the run; the MEA's lists never leave it) */
+        b = run(j->ctx, &k, j->sM, j->p, j->mode, j->reweight || j->shiftedMea ? NULL : &sinks);
     }
     STAGE("device pass (create + run)");
     if (j->realign) {
+    } else if (j->shiftedMea) {
+        device_shifted_mea(j, b);
     } else if (j->mode == CPB_MODE_ALIGNED_PAIRS || j->mode == CPB_MODE_ALIGNED_PAIRS_INDELS) {
         if (j->reweight && cpb_batch_reweight_pairs(b, j->gapGamma) != CPB_OK) st_errAbort("cpecan: %s", cpb_last_error());
         const int nLists = j->mode == CPB_MODE_ALIGNED_PAIRS ? 1 : 3;
@@ -785,6 +814,20 @@ CpecanRealignedCigars *getRealignedCigarsUsingAnchorsBatch(StateMachine *sM, int
     }
     for (int d = 0; d < nDev; d++) free(idx[d]);
     return r;
+}
+
+stList **getShiftedMEAAlignmentBatch(StateMachine *sM, int64_t n, char *const *seqX, char *const *seqY, stList *const *anchorAlignments,
+                                     PairwiseAlignmentParameters *p, const bool *raggedLeft, const bool *raggedRight, double *alignmentScores) {
+    stList **out = new_list_array(n);
+    if (n == 0) return out;
+    DeviceJob proto = job_of(sM, (const char *const *) seqX, (const char *const *) seqY, anchorAlignments, p, raggedLeft, raggedRight,
+                             CPB_MODE_ALIGNED_PAIRS_INDELS),
+              jobs[CPECAN_MAX_DEVICES];
+    proto.shiftedMea = 1;
+    proto.alignmentScores = alignmentScores;
+    proto.lists[0] = out;
+    run_on_devices(&proto, n, jobs, NULL);
+    return out;
 }
 
 void cpecanRealignedCigars_destruct(CpecanRealignedCigars *r) {

@@ -267,6 +267,30 @@ static int64_t gap_weight(const int64_t *cum, int64_t start, int64_t length) {
     return length == 0 ? 0 : cum[start + length - 1] - (start > 0 ? cum[start - 1] : 0);
 }
 
+/* The walk-back from pair (x, y) acts only on entries with x2 < x and y2 < y; every other entry is passed over without effect.  So a range
+ * of list positions whose least x is not below x, or whose least y is not below y, holds no predecessor and is skipped whole: score, from,
+ * the cutoff and isHigh come out as the entry-by-entry scan leaves them, in any list order.  In the reference's order a region's
+ * traceback blocks come last to first, so the walk from a pair of block k would otherwise read every triple of the blocks after k (later
+ * diagonals, none of them a predecessor) -- quadratic in the list length.  The least x and y are kept for every aligned range of
+ * MEA_CHUNK entries and of MEA_CHUNK^2 entries (decode_kernels.cuh keeps the same two levels). */
+#define MEA_CHUNK_SHIFT 5
+#define MEA_CHUNK ((int64_t) 1 << MEA_CHUNK_SHIFT)
+#define MEA_BLOCK_SHIFT (2 * MEA_CHUNK_SHIFT)
+#define MEA_BLOCK ((int64_t) 1 << MEA_BLOCK_SHIFT)
+
+/* least[2 * r], least[2 * r + 1] = the least x and y of the entries r << shift ... ((r + 1) << shift) - 1 */
+static int64_t *least_xy(const int64_t *x, const int64_t *y, int64_t n, int shift) {
+    const int64_t ranges = (n + ((int64_t) 1 << shift) - 1) >> shift;
+    int64_t *least = cpecan_malloc((size_t) (2 * ranges + 2) * sizeof(int64_t));
+    for (int64_t r = 0; r < ranges; r++) least[2 * r] = least[2 * r + 1] = INT64_MAX;
+    for (int64_t j = 0; j < n; j++) {
+        int64_t *l = least + 2 * (j >> shift);
+        if (x[j] < l[0]) l[0] = x[j];
+        if (y[j] < l[1]) l[1] = y[j];
+    }
+    return least;
+}
+
 stList *getMaximalExpectedAccuracyPairwiseAlignment(stList *alignedPairs, stList *gapXPairs, stList *gapYPairs, int64_t seqXLength,
                                                     int64_t seqYLength, double *alignmentScore, PairwiseAlignmentParameters *p) {
     const int64_t n = stList_length(alignedPairs);
@@ -275,22 +299,38 @@ stList *getMaximalExpectedAccuracyPairwiseAlignment(stList *alignedPairs, stList
     bool *isHigh = cpecan_malloc((size_t) (n + 1) * sizeof(bool));
     memset(isHigh, 0, (size_t) (n + 1) * sizeof(bool));
     int64_t *cumY = cumulative_gap_weights(gapYPairs, seqYLength, 2), *cumX = cumulative_gap_weights(gapXPairs, seqXLength, 1);
+    int64_t *tw = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t)), *tx = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t)),
+            *ty = cpecan_malloc((size_t) (n + 1) * sizeof(int64_t));
+    for (int64_t i = 0; i < n; i++) {
+        stIntTuple *t = stList_get(alignedPairs, i);
+        tw[i] = stIntTuple_get(t, 0);
+        tx[i] = stIntTuple_get(t, 1);
+        ty[i] = stIntTuple_get(t, 2);
+    }
+    int64_t *chunk = least_xy(tx, ty, n, MEA_CHUNK_SHIFT), *block = least_xy(tx, ty, n, MEA_BLOCK_SHIFT);
     const float gamma = p->gapGamma;
     double maxScore = 0;
     /* pairs in list order (the engine's order: increasing x + y within a region); a virtual pair at (lX, lY) closes the alignment */
     for (int64_t i = 0; i <= n; i++) {
         int64_t w = 0, x = seqXLength, y = seqYLength;
         if (i < n) {
-            stIntTuple *t = stList_get(alignedPairs, i);
-            w = stIntTuple_get(t, 0);
-            x = stIntTuple_get(t, 1);
-            y = stIntTuple_get(t, 2);
+            w = tw[i];
+            x = tx[i];
+            y = ty[i];
         }
         double score = w + (gap_weight(cumX, 0, x) + gap_weight(cumY, 0, y)) * gamma;
         int64_t from = -1;
         for (int64_t j = i - 1; j >= 0; j--) {
-            stIntTuple *q = stList_get(alignedPairs, j);
-            const int64_t x2 = stIntTuple_get(q, 1), y2 = stIntTuple_get(q, 2);
+            /* at the last entry of an aligned range: skip the whole range if it holds no predecessor (a range that i - 1 ends early is scanned) */
+            if ((j & (MEA_BLOCK - 1)) == MEA_BLOCK - 1 && !(block[2 * (j >> MEA_BLOCK_SHIFT)] < x && block[2 * (j >> MEA_BLOCK_SHIFT) + 1] < y)) {
+                j -= MEA_BLOCK - 1;
+                continue;
+            }
+            if ((j & (MEA_CHUNK - 1)) == MEA_CHUNK - 1 && !(chunk[2 * (j >> MEA_CHUNK_SHIFT)] < x && chunk[2 * (j >> MEA_CHUNK_SHIFT) + 1] < y)) {
+                j -= MEA_CHUNK - 1;
+                continue;
+            }
+            const int64_t x2 = tx[j], y2 = ty[j];
             if (x2 < x && y2 < y) {
                 /* the candidate is held in an int64 in the reference (:1668), i.e. truncated before the comparison */
                 const int64_t s = (int64_t) (w + scores[j] + (gap_weight(cumX, x2 + 1, x - x2 - 1) + gap_weight(cumY, y2 + 1, y - y2 - 1)) * gamma);
@@ -319,6 +359,11 @@ stList *getMaximalExpectedAccuracyPairwiseAlignment(stList *alignedPairs, stList
     free(scores);
     free(back);
     free(isHigh);
+    free(tw);
+    free(tx);
+    free(ty);
+    free(chunk);
+    free(block);
     free(cumX);
     free(cumY);
     *alignmentScore = maxScore;

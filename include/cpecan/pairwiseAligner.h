@@ -254,6 +254,13 @@ CpecanRealignedCigars *getRealignedCigarsUsingAnchorsBatch(StateMachine *sM, int
                                                            const bool *raggedRight, float matchGamma, int scoreKind, bool wantAlignments,
                                                            bool wantRawPairs);
 void cpecanRealignedCigars_destruct(CpecanRealignedCigars *r);
+/* getShiftedMEAAlignment (:1769-1792) for n problems in one pass over the device set: an ALIGNED_PAIRS_INDELS run, MEA with p->gapGamma
+ * and leftShiftAlignment, all on the device (cpb_batch_mea).  Returns n new lists of (pInt, x, y) tuples (free each with stList_destruct,
+ * the array with free); alignmentScores (n doubles, or NULL) receives each problem's alignmentScore.  Lengths are strlen; anchorAlignments[i]
+ * and raggedLeft / raggedRight may be NULL as for getAlignedPairsUsingAnchorsBatch.  Triples and scores are bit for bit those of
+ * getShiftedMEAAlignment.  An invalid band aborts with PAIRWISE_ALIGNMENT_EXCEPTION, any other engine error with the engine's message. */
+stList **getShiftedMEAAlignmentBatch(StateMachine *sM, int64_t n, char *const *seqX, char *const *seqY, stList *const *anchorAlignments,
+                                     PairwiseAlignmentParameters *p, const bool *raggedLeft, const bool *raggedRight, double *alignmentScores);
 /* sums the expectations of all n problems into hmmExpectations (+=), as n calls of getExpectationsUsingAnchors would */
 void getExpectationsUsingAnchorsBatch(StateMachine *sM, Hmm *hmmExpectations, int64_t n, const char *const *sX, const char *const *sY,
                                       stList *const *anchorPairs, PairwiseAlignmentParameters *p, const bool *raggedLeft,

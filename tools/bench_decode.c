@@ -6,7 +6,9 @@
  *   mea:   device MEA + left shift vs host getMaximalExpectedAccuracyPairwiseAlignment + leftShiftAlignment over the lists in the
  *          reference's order (cpb_batch_fetch_pairs_reference_order, what libcpecan.so hands over).
  * Device time: median of REPS synchronised calls after a warm-up (the chain's batch is run again before each, not timed).  Host time: the
- * functions alone on THREADS threads, their input lists built beforehand.  Every pair is compared.  One JSON line on stdout.
+ * functions alone on THREADS threads, their input lists built beforehand.  Every pair is compared.  One JSON line on stdout.  THREADS 0
+ * times the device alone: no host arm and no comparison (pairs_checked 0), e.g. to time another build's libcpecan_b200.so through
+ * LD_LIBRARY_PATH.
  *
  *   bench_decode SEQS.bin chain|mea TRIM EXPANSION SPLIT GAMMA REWEIGHT THREADS REPS
  *   SEQS.bin: int64 n; int64 xOff[n+1], yOff[n+1]; char seqX[xOff[n]], seqY[yOff[n]]
@@ -134,7 +136,7 @@ int main(int argc, char **argv) {
     fprintf(stderr, "bench_decode: %" PRIi64 " pairs anchored and run\n", n);
 
     /* the host arm's inputs: the lists as libcpecan.so hands them over */
-    const int nLists = mea ? 3 : 1;
+    const int nLists = mea ? 3 : 1, hostArm = threads > 0;
     int64_t *off[3] = { NULL, NULL, NULL }, cloud = 0;
     int32_t *tri[3] = { NULL, NULL, NULL };
     for (int l = 0; l < nLists; l++) {
@@ -142,7 +144,7 @@ int main(int argc, char **argv) {
         cloud += c;
         off[l] = malloc((size_t) (n + 1) * 8);
         tri[l] = malloc((size_t) (c > 0 ? c : 1) * 12);
-        check(mea ? cpb_batch_fetch_pairs_reference_order(b, l, off[l], tri[l]) : cpb_batch_fetch_pairs(b, l, off[l], tri[l]), "fetch");
+        if (hostArm) check(mea ? cpb_batch_fetch_pairs_reference_order(b, l, off[l], tri[l]) : cpb_batch_fetch_pairs(b, l, off[l], tri[l]), "fetch");
     }
     Work w;
     memset(&w, 0, sizeof(w));
@@ -159,8 +161,8 @@ int main(int argc, char **argv) {
         memcpy(w.sY[i], seqY + yOff[i], (size_t) lY);
         w.sX[i][lX] = w.sY[i][lY] = 0;
     }
-    w.in0 = lists_of(n, off[0], tri[0]);
-    if (mea) {
+    w.in0 = hostArm ? lists_of(n, off[0], tri[0]) : calloc((size_t) (n > 0 ? n : 1), sizeof(stList *));
+    if (mea && hostArm) {
         w.in1 = lists_of(n, off[1], tri[1]);
         w.in2 = lists_of(n, off[2], tri[2]);
     }
@@ -198,7 +200,7 @@ int main(int argc, char **argv) {
     check(cpb_batch_fetch_alignments(b, aOff, aTri), "fetch alignments");
 
     int64_t differ = 0, first = -1;
-    for (int64_t i = 0; i < n; i++) {
+    for (int64_t i = 0; hostArm && i < n; i++) {
         stList *o = w.out[i];
         const int64_t len = stList_length(o);
         int same = len == aOff[i + 1] - aOff[i];
@@ -217,8 +219,8 @@ int main(int argc, char **argv) {
            ", \"alignment_bytes\": %" PRIi64 ", \"host_threads\": %d, \"host_ms\": %.1f, \"device_ms\": %.2f, \"device_ms_all\": [",
            n, cloud, cloud * 12 + (int64_t) nLists * (n + 1) * 8, alnCount, alnCount * 12 + (n + 1) * 8, threads, hostMs, dev[1 + reps / 2]);
     for (int r = 1; r <= reps; r++) printf("%s%.2f", r > 1 ? ", " : "", dev[r]);
-    printf("], \"warmup_ms\": %.2f, \"pairs_checked\": %" PRIi64 ", \"pairs_differing\": %" PRIi64 ", \"first_differing\": %" PRIi64 "}\n", dev[0], n,
-           differ, first);
+    printf("], \"warmup_ms\": %.2f, \"pairs_checked\": %" PRIi64 ", \"pairs_differing\": %" PRIi64 ", \"first_differing\": %" PRIi64 "}\n", dev[0],
+           hostArm ? n : 0, differ, first);
     cpb_batch_destroy(b);
     cpb_context_destroy(ctx);
     return differ != 0;
